@@ -2,6 +2,7 @@
 """bench.py -- self-play MCTS throughput of the B200 engine (BASELINE.json metric: MCTS simulations/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm
+    python bench.py ... --dump-outputs DIR                         # + training records of a tree sample as DIR/*.npy
     python bench.py --impl reference [--steps K] [--warmup W]      # CPU arm: the oracle port of the reference
     torchrun ... bench.py --gpus N ...                             # one rank per GPU, NCCL
 
@@ -33,6 +34,7 @@ if ROOT not in sys.path:
 
 ROUNDS_PER_STEP = 50
 SETTLE_MIN_ROUNDS, SETTLE_MAX_ROUNDS = 1500, 12000
+DUMP_TREES = 4096
 # BASELINE.json configs by index; trees = concurrent games per GPU
 CONFIGS = {
     "c4": {"index": 2, "game": "connect_four", "playouts": 800, "trees": 16384},
@@ -226,7 +228,7 @@ def build_net(args, shape, n_actions):
     return net, weights
 
 
-def settle(runner, n_trees, dev):
+def settle(runner, n_trees, dev, drain):
     """Untimed: run the pool into steady state (see the module docstring).  Returns the round trips spent."""
     import torch
     rounds = 0
@@ -234,18 +236,67 @@ def settle(runner, n_trees, dev):
         runner.round(250)
         rounds += 250
         if rounds % 1000 == 0:
-            runner.drain()
+            drain()
         c = runner.counters()
         torch.cuda.synchronize(dev)
         if rounds >= SETTLE_MIN_ROUNDS and c["moves"] >= 2 * n_trees and c["games"] > 0:
             break
         if rounds >= SETTLE_MAX_ROUNDS:
             break
-    runner.drain()
+    drain()
     return rounds
 
 
+def dump_move(args):
+    """--dump-outputs writes each sample tree's search number dump_move(args) (1-based): a lower bound on the searches every
+    tree has finished when the last timed step ends.  A search of n playouts takes at most n + 3 round trips (one evaluation
+    per playout, the root evaluation, the move and the re-rooting), and by then the run has made at least the settle
+    minimum plus the warm-up and timed steps' round trips."""
+    rounds = (0 if args.no_settle else SETTLE_MIN_ROUNDS) + (args.warmup + args.steps) * ROUNDS_PER_STEP
+    return rounds // (args.playouts + 3)
+
+
+def dump_trees(n_trees):
+    """The fixed, seeded sample of trees whose searches --dump-outputs writes (at most DUMP_TREES of them)."""
+    import numpy as np
+    return np.sort(np.random.RandomState(0).choice(n_trees, min(n_trees, DUMP_TREES), replace=False))
+
+
+def dump_outputs(path, records, trees, move, game):
+    """What the self-play path hands its caller, the training record of a search (policy target, root value, the position
+    searched and the move played), for search number `move` of every tree in `trees`, as float arrays path/<name>.npy.
+    Which move a tree is on when the last timed step ends depends on timing (the step kernel's cycle budget is a clock
+    bound); what each search computes does not, so this selection is the same from run to run for the same arguments.
+    A tree that has not finished that search (an arena overflow stops a tree) gives a row of NaN."""
+    import numpy as np
+    from alphazero_openspiel_b200.engine import game_shape, parse_game_name
+    from alphazero_openspiel_b200.examplegenerator import boards_from_bitboards, policy_targets_batch
+    gid, rows, cols = parse_game_name(game)
+    n_actions = game_shape(game)[1]
+    recs = np.concatenate(records)
+    recs = recs[np.lexsort((recs["ply"], recs["game_seq"], recs["tree"]))]
+    first = np.searchsorted(recs["tree"], recs["tree"])          # index of each tree's first search
+    recs = recs[np.arange(len(recs)) - first == move - 1]
+    slot = np.searchsorted(trees, recs["tree"])
+    n = len(trees)
+    out = {"tree": trees.astype(np.float64)}
+    for name in ("game_seq", "ply", "action", "root_q"):
+        out[name] = np.full((n,), np.nan)
+        out[name][slot] = recs[name]
+    out["policy"] = np.full((n, n_actions), np.nan)
+    out["policy"][slot] = policy_targets_batch(recs["counts"], recs["actions"], recs["n_legal"], n_actions)
+    out["board"] = np.full((n, 4, rows, cols), np.nan, dtype=np.float32)
+    out["board"][slot] = boards_from_bitboards(gid, rows, cols, recs["bb"], recs["ply"])
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    if len(recs) < n:
+        sys.stderr.write("WARNING: --dump-outputs: %d of %d sample trees had not finished search %d (rows of NaN)\n"
+                         % (n - len(recs), n, move))
+
+
 def run_ours(args):
+    import numpy as np
     import torch
     import torch.distributed as dist
     from alphazero_openspiel_b200 import _lib as L
@@ -279,21 +330,30 @@ def run_ours(args):
                             virtual_loss=args.virtual_loss, step_cycle_budget=args.cycle_budget)
     rps = ROUNDS_PER_STEP
     n_rounds = args.steps * rps
+    # --dump-outputs keeps the sample trees' training records from every drain up to the end of the timed steps
+    dump = args.dump_outputs and rank == 0
+    kept, sample = [], dump_trees(args.trees) if dump else None
+
+    def drain():
+        recs = runner.drain()
+        if dump:
+            kept.append(recs[(recs["kind"] == 0) & np.isin(recs["tree"], sample)])
+
     # ---- settle (untimed, steady state) + warm-up (untimed, W steps).  nvidia-smi needs up to a second to deliver its
     # first sample, so the clock sampler is started before the warm-up; only samples taken after mark() are reported.
-    settle_rounds = 0 if args.no_settle else settle(runner, args.trees, dev)
+    settle_rounds = 0 if args.no_settle else settle(runner, args.trees, dev, drain)
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     runner.round(args.warmup * rps)
-    runner.drain()
+    drain()
     torch.cuda.synchronize(dev)
     if rank == 0:
         t_wait = time.time()
         while not sampler.rows and time.time() - t_wait < 3.0:
             runner.round(rps)
             torch.cuda.synchronize(dev)
-        runner.drain()
+        drain()
         torch.cuda.synchronize(dev)
 
     def barrier():
@@ -323,7 +383,9 @@ def run_ours(args):
     for t in list(host_net.parameters()) + list(host_net.buffers()):
         t.data = t.data.pin_memory()
     h2d = sum(t.numel() * t.element_size() for t in list(host_net.parameters()) + list(host_net.buffers()))
-    runner.drain()
+    drain()
+    if dump:
+        dump_outputs(args.dump_outputs, kept, sample, dump_move(args), game)
     barrier()
     e0 = runner.counters()
     t0 = time.perf_counter()
@@ -504,7 +566,7 @@ def run_train(args):
     tr = Trainer(name="bench", name_game=args.game, device=dev, save=False, n_playouts_train=args.playouts,
                  array_buffer=not args.list_buffer, device_training=not args.list_buffer,
                  graph_step=not (args.list_buffer or args.eager_train or args.ddp), ddp=args.ddp)
-    gens = max(1, args.generations)
+    gens = args.steps if args.generations is None else max(1, args.generations)
 
     def sync():
         torch.cuda.synchronize(dev)
@@ -596,12 +658,17 @@ def main():
     ap.add_argument("--evaluator", default="fused", choices=["fused", "torch"])
     ap.add_argument("--node-capacity", type=int, default=0)
     ap.add_argument("--virtual-loss", type=int, default=0, help="K leaves in flight per tree (non-bit-exact mode); 0 = off")
-    ap.add_argument("--generations", type=int, default=3, help="--config train: generations timed")
+    ap.add_argument("--generations", type=int, default=None, help="--config train: generations timed (default: --steps)")
     ap.add_argument("--ddp", action="store_true", help="--config train: data-parallel optimisation steps (NCCL gradient all-reduce)")
     ap.add_argument("--eager-train", action="store_true", help="--config train: eager optimisation steps (no CUDA graph)")
     ap.add_argument("--list-buffer", action="store_true", help="--config train: the reference's Python-list replay buffer")
     ap.add_argument("--no-keep-tree", action="store_true", help="experiment: fresh tree every move (no re-root compaction)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="self-play configs: after the timed steps write the training records of a fixed sample of trees as "
+                         "DIR/<name>.npy (see dump_outputs), for comparing the outputs of two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries ONE JSON line and nothing else: whatever libraries write to file descriptor 1 (NCCL prints its version
     # banner there when NCCL_DEBUG is VERSION or higher, as on some boxes) is sent to stderr; emit() writes to the real stdout
     global _REAL_STDOUT
@@ -614,6 +681,10 @@ def main():
     args.playouts = args.playouts or cfg["playouts"]
     if args.warmup < 3:
         args.warmup = 3
+    if args.dump_outputs and (args.impl == "reference" or args.config == "train"):
+        ap.error("--dump-outputs is for the self-play configs (c4, bt6, bt8) of --impl ours")
+    if args.dump_outputs and dump_move(args) < 1:
+        ap.error("--dump-outputs: too few round trips for every tree to finish a search; raise --steps or --warmup")
     if args.impl == "reference":
         run_reference(args)
     elif args.config == "train":

@@ -2,10 +2,10 @@
 
 Exposes exactly the API subset the reference calls (SURVEY Appendix B.1), with the pre-Feb-2020
 OpenSpiel method names (`information_state_normalized_vector_shape`, ...), so that the reference's
-own mcts.py / alphazerobot.py / game_utils.py run unmodified in this container:
+own mcts.py / alphazerobot.py / game_utils.py run unmodified over it:
 
     from oracle import pyspiel_shim; pyspiel_shim.install()   # registers sys.modules['pyspiel']
-    sys.path.insert(0, '/root/reference'); import game_utils
+    sys.path.insert(0, REFERENCE_CHECKOUT); import game_utils
 
 Real pyspiel is absent (no network); game semantics follow SURVEY Appendix B.2/B.3.
 """

@@ -1,7 +1,6 @@
 """Pure-Python restatement of the reference's self-play path (CPU ORACLE -- test infrastructure only).
 
-This is the CPU baseline that travels to the GPU box (the reference is Python and /root/reference does
-not exist there).  It restates, with flat parallel lists instead of linked Node objects:
+This is the CPU baseline bench.py times (the reference itself is not part of this repository).  It restates, with flat parallel lists instead of linked Node objects:
 
     PortMCTS          <- mcts.py:92-203   (search / playout / expand_root_dirichlet / update_root)
       ._pick          <- mcts.py:38-52,68-80  Node.select + get_value (PUCT and use_puct=False branches)
@@ -15,8 +14,8 @@ not exist there).  It restates, with flat parallel lists instead of linked Node 
     PortGenerator     <- examplegenerator.py:17-22,39-175  worker pool + batching evaluator process
 
 The arithmetic (operation order, Python-float fp64, first-max tie-breaking, global numpy RNG call
-order) is kept identical so results are bit-equal to the reference; tests/test_oracle_vs_reference.py
-pins that in-container against /root/reference run over oracle.pyspiel_shim.
+order) is kept identical so results are bit-equal to the reference; tests/test_oracle_golden.py pins that against
+the reference's recorded outputs (tests/golden/).
 """
 import math
 import os

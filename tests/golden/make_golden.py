@@ -1,8 +1,8 @@
-"""Generates tests/golden/*.json|npz by running the UNMODIFIED reference (/root/reference: mcts.py, alphazerobot.py,
-game_utils.py, network.py) in this container over oracle.pyspiel_shim.  /root/reference cannot travel to the
-GPU box, so the vectors are committed; re-run this script to regenerate them:
+"""Generates tests/golden/reference_golden.json by running the UNMODIFIED reference (mcts.py, alphazerobot.py,
+game_utils.py, network.py of a checkout of danielwillemsen/alphazero-openspiel) over oracle.pyspiel_shim.  The reference
+is not part of this repository, so the vectors are committed; re-run this script to regenerate them:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py REFERENCE_CHECKOUT
 """
 import ctypes as C
 import json
@@ -18,7 +18,8 @@ sys.path.insert(0, ROOT)
 from oracle import pyspiel_shim, cbind  # noqa: E402
 
 pyspiel = pyspiel_shim.install()
-sys.path.insert(0, "/root/reference")
+REF = os.path.abspath(sys.argv[1])
+sys.path.insert(0, REF)
 import torch  # noqa: E402
 import mcts as ref_mcts  # noqa: E402
 import game_utils as ref_game_utils  # noqa: E402
@@ -134,7 +135,7 @@ def selfplay_examples():
 def encoding_pins():
     """SURVEY B.4: the shipped checkpoints pin the observation / action encodings of the game restatement."""
     res = {}
-    ck = "/root/reference/models/example_model_connect_four.pth"
+    ck = os.path.join(REF, "models", "example_model_connect_four.pth")
     shutil.copyfile(ck, os.path.join(HERE, "example_model_connect_four.pth"))  # weights are data, kept as a fixture
     g = pyspiel.load_game("connect_four")
     net = ref_network.Net([3, 6, 7], 7)
@@ -163,7 +164,7 @@ def encoding_pins():
     pp, vv = net.predict(s)
     res["c4_fixture16"] = {"p": pp, "v": vv}
     # breakthrough 6x6: policy mass on legal moves under the B.3 encoding
-    ck6 = "/root/reference/models/example_model_breakthrough(6x6).pth"
+    ck6 = os.path.join(REF, "models", "example_model_breakthrough(6x6).pth")
     g6 = pyspiel.load_game("breakthrough(rows=6,columns=6)")
     net6 = ref_network.Net([3, 6, 6], 432)
     net6.load_state_dict(torch.load(ck6, map_location="cpu", weights_only=True))

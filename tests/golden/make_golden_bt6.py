@@ -1,7 +1,7 @@
-"""Generates the Breakthrough 6x6 fixtures by running the UNMODIFIED reference network (/root/reference/network.py) with
-its shipped checkpoint in this container:
+"""Generates the Breakthrough 6x6 fixtures by running the UNMODIFIED reference network (network.py of a checkout of
+danielwillemsen/alphazero-openspiel) with its shipped checkpoint:
 
-    python tests/golden/make_golden_bt6.py
+    python tests/golden/make_golden_bt6.py REFERENCE_CHECKOUT
 
   example_model_breakthrough_6x6.pth  the reference's models/example_model_breakthrough(6x6).pth (weights are data;
                                       BASELINE config [1] runs "with the shipped model", which cannot travel otherwise)
@@ -21,12 +21,13 @@ sys.path.insert(0, ROOT)
 from oracle import pyspiel_shim  # noqa: E402
 
 pyspiel = pyspiel_shim.install()
-sys.path.insert(0, "/root/reference")
+REF = os.path.abspath(sys.argv[1])
+sys.path.insert(0, REF)
 import torch  # noqa: E402
 import network as ref_network  # noqa: E402
 
 if __name__ == "__main__":
-    ck = "/root/reference/models/example_model_breakthrough(6x6).pth"
+    ck = os.path.join(REF, "models", "example_model_breakthrough(6x6).pth")
     shutil.copyfile(ck, os.path.join(HERE, "example_model_breakthrough_6x6.pth"))
     game = "breakthrough(rows=6,columns=6)"
     g = pyspiel.load_game(game)

@@ -1,5 +1,5 @@
 """GPU parity of the drop-in Python API (MCTS / AlphaZeroBot / play_game_self / Net / ExampleGenerator)
-against the oracle's port of the reference (oracle.ref_port, pinned to /root/reference in test_oracle_vs_reference)."""
+against the oracle's port of the reference (oracle.ref_port, pinned to the reference's recorded outputs in test_oracle_golden)."""
 import ctypes as C
 
 import numpy as np

@@ -1,10 +1,9 @@
-"""CPU: the oracle (C restatement + Python port + RefNet) against the golden vectors generated from the
-UNMODIFIED reference by tests/golden/make_golden.py, and -- when /root/reference is present (this container) --
-against the reference itself run live."""
+"""CPU: the oracle (C restatement + Python port + RefNet) and the drop-in's host code against the golden vectors of the
+UNMODIFIED reference: tests/golden/reference_golden.json (tests/golden/make_golden.py) and
+tests/golden/reference_crosscheck.json (tests/golden/make_golden_crosscheck.py)."""
 import ctypes as C
 import json
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -14,6 +13,8 @@ from oracle import cbind, pyspiel_shim, ref_port
 HERE = os.path.dirname(os.path.abspath(__file__))
 with open(os.path.join(HERE, "golden", "reference_golden.json")) as f:
     GOLD = json.load(f)
+with open(os.path.join(HERE, "golden", "reference_crosscheck.json")) as f:
+    CROSS = json.load(f)
 L = cbind.lib()
 
 
@@ -220,131 +221,88 @@ def test_game_rules_properties():
     assert s.legal_actions() == [74, 76, 84, 86, 88, 96, 98, 100, 108, 110, 112, 120, 122, 124, 132, 134]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="the reference only exists in the build container")
 def test_port_and_c_oracle_vs_live_reference():
-    """Live cross-check against /root/reference (mcts.py / game_utils.py run unmodified over the shim)."""
-    pyspiel_shim.install()
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    import game_utils as ref_gu
-    import mcts as ref_mcts
+    """play_game_self and a 300-playout search as the unmodified reference returns them (mcts.py / game_utils.py run over
+    the shim; recorded in reference_crosscheck.json): the port's self-play and the C oracle's search reproduce them."""
     fn = _hash_policy(123)
-    for game in ["connect_four", "breakthrough(rows=6,columns=6)"]:
-        for backup in ["on-policy", "off-policy"]:
-            np.random.seed(11)
-            a = ref_gu.play_game_self(fn, game, n_playouts=25, backup=backup)
-            np.random.seed(11)
-            b = ref_port.selfplay_game(fn, game, pyspiel_shim.load_game, n_playouts=25, backup=backup)
-            assert len(a) == len(b)
-            for x, y in zip(a, b):
-                assert x[0] == y[0] and np.array_equal(x[1], y[1]) and x[2] == y[2] and x[3] == y[3]
-    g = pyspiel_shim.load_game("connect_four")
-    s = g.new_initial_state()
-    m = ref_mcts.MCTS(fn, 7, use_dirichlet=False, n_playouts=300)
-    m.search(s)
+    for case in CROSS["selfplay"]:
+        np.random.seed(11)
+        b = ref_port.selfplay_game(fn, case["game"], pyspiel_shim.load_game, n_playouts=25, backup=case["backup"])
+        A = pyspiel_shim.load_game(case["game"]).num_distinct_actions()
+        assert len(b) == len(case["keys"])
+        for i, y in enumerate(b):
+            dense = [0.0] * A
+            for a, p in case["policies"][i]:
+                dense[a] = p
+            assert y[0] == case["keys"][i] and y[2] == dense and y[3] == case["values"][i]
+            assert np.array_equal(y[1].ravel(), np.array(case["boards"][i]))
+    s = pyspiel_shim.load_game("connect_four").new_initial_state()
     t = L.oz_tree_new(7, 2.5, 300, 0, 0.25)
     counts = (C.c_int64 * 7)()
     L.oz_tree_search(t, C.byref(s.raw()), _eval_cb(1, 123), None, None, counts)
-    assert list(counts) == [m.root.children[a].N for a in range(7)]
-    assert L.oz_tree_root_q(t) == m.root.Q
+    assert list(counts) == CROSS["search300"]["counts"]
+    assert L.oz_tree_root_q(t) == CROSS["search300"]["root_q"]
     L.oz_tree_free(t)
 
 
 def test_random_rollout_evaluator_matches_live_reference():
-    """MCTS.random_rollout (mcts.py:205-223, SURVEY 8(f).4): the oracle port, the drop-in's host implementation and the
-    live reference draw the same playouts from the same numpy seed; a whole search driven by it matches the port."""
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("/root/reference is not mounted (GPU box)")
-    pyspiel_shim.install()
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    import mcts as ref_mcts
+    """MCTS.random_rollout (mcts.py:205-223, SURVEY 8(f).4): the oracle port and the drop-in's host implementation draw the
+    reference's playouts from the same numpy seed (same priors, value and RNG position afterwards); a whole search driven
+    by it gives the reference's visit distribution."""
     from alphazero_openspiel_b200.mcts import MCTS as OurMCTS
-    for game in ["connect_four", "breakthrough(rows=6,columns=6)"]:
-        g = pyspiel_shim.load_game(game)
+    for case in CROSS["rollouts"]:
+        g = pyspiel_shim.load_game(case["game"])
         A = g.num_distinct_actions()
-        ref = ref_mcts.MCTS(None, A, n_playouts=40, use_dirichlet=False)
         ours = OurMCTS(None, A)                      # no engine is created before a search
         port_fn = ref_port.rollout_policy(A)
         s = g.new_initial_state()
-        for ply in range(6):
-            outs = []
-            for fn in (ref.random_rollout, ours.random_rollout, port_fn):
+        for ply, want in enumerate(case["evals"]):
+            for fn in (ours.random_rollout, port_fn):
                 np.random.seed(100 + ply)
                 pri, v = fn(s)
-                outs.append((list(pri), v, np.random.random_sample()))   # same priors, value and RNG position
-            assert outs[0] == outs[1] == outs[2]
+                assert (list(pri), v, np.random.random_sample()) == (want["priors"], want["value"], want["next_draw"])
             s.apply_action(s.legal_actions()[ply % len(s.legal_actions())])
-        # a search with the rollout evaluator: port vs live reference
-        s = g.new_initial_state()
-        ref.policy_fn = ref.random_rollout
         port = ref_port.PortMCTS(port_fn, A, n_playouts=40, use_dirichlet=False)
         np.random.seed(5)
-        a = ref.search(s)
-        np.random.seed(5)
-        b = port.search(s)
-        assert list(a) == list(b)
+        assert list(port.search(g.new_initial_state())) == case["search"]
 
 
 def test_uct_mode_port_vs_live_reference():
     """use_puct=False (mcts.py:80, SURVEY 8(f).4) exactly as the reference behaves: the flag lives on the nodes, the first
     root is built without it (mcts.py:122), so only a tree whose root came from update_root on a leaf root (mcts.py:199-200)
-    scores with the UCT formula.  The port follows the unmodified live reference through both kinds of tree."""
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("/root/reference is not mounted (GPU box)")
-    pyspiel_shim.install()
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    import mcts as ref_mcts
+    scores with the UCT formula.  The port gives the reference's visit distributions and root Q through both kinds of
+    tree."""
     fn = _hash_policy(31)
-    for game in ["connect_four", "breakthrough(rows=6,columns=6)"]:
-        g = pyspiel_shim.load_game(game)
+    for case in CROSS["uct"]:
+        g = pyspiel_shim.load_game(case["game"])
         A = g.num_distinct_actions()
-        for dirichlet in (False, True):
-            for leaf_update_first in (False, True):
-                ref = ref_mcts.MCTS(fn, A, n_playouts=80, use_dirichlet=dirichlet, use_puct=False)
-                port = ref_port.PortMCTS(fn, A, n_playouts=80, use_dirichlet=dirichlet, use_puct=False)
-                s = g.new_initial_state()
-                if leaf_update_first:     # what a second player's bot does before its first search: the UCT tree
-                    first = s.legal_actions()[1]
-                    s.apply_action(first)
-                    ref.update_root(first)
-                    port.update_root(first)
-                    assert ref.root.use_puct is False and port.tree_uct
-                uct_counts = None
-                for move in range(3):
-                    np.random.seed(70 + move)
-                    a = ref.search(s)
-                    np.random.seed(70 + move)
-                    b = port.search(s)
-                    assert list(a) == list(b) and ref.root.Q == port.mean[port.root]
-                    uct_counts = uct_counts or list(a)
-                    act = int(np.argmax(a))
-                    ref.update_root(act)
-                    port.update_root(act)
-                    s.apply_action(act)
+        port = ref_port.PortMCTS(fn, A, n_playouts=80, use_dirichlet=case["dirichlet"], use_puct=False)
+        s = g.new_initial_state()
+        if case["leaf_update_first"]:     # what a second player's bot does before its first search: the UCT tree
+            first = s.legal_actions()[1]
+            s.apply_action(first)
+            port.update_root(first)
+            assert port.tree_uct
+        for move, want in enumerate(case["moves"]):
+            np.random.seed(70 + move)
+            b = port.search(s)
+            assert list(b) == want["counts"] and port.mean[port.root] == want["root_q"]
+            act = int(np.argmax(b))
+            port.update_root(act)
+            s.apply_action(act)
 
 
 def test_neuralnetbot_and_play_game_match_live_reference():
-    """The host-only pieces of the match-up harness (alphazerobot.py:96-118, game_utils.py:16-35): same policies, actions and
-    game results as the unmodified reference for the same policy function."""
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("/root/reference is not mounted (GPU box)")
-    pyspiel_shim.install()
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    import alphazerobot as ref_bot
-    import game_utils as ref_gu
+    """The host-only pieces of the match-up harness (alphazerobot.py:96-118, game_utils.py:16-35): the reference's
+    policies, actions and game results for the same policy functions."""
     from alphazero_openspiel_b200 import alphazerobot as our_bot, game_utils as our_gu
-    for game in ["connect_four", "breakthrough(rows=6,columns=6)"]:
-        g = pyspiel_shim.load_game(game)
+    for case in CROSS["netbot"]:
+        g = pyspiel_shim.load_game(case["game"])
         fa, fb = _hash_policy(3), _hash_policy(4)
         s = g.new_initial_state()
-        for _ in range(5):
-            pr, ar = ref_bot.NeuralNetBot(g, 0, fa).step(s)
+        for want in case["steps"]:
             po, ao = our_bot.NeuralNetBot(g, 0, fa).step(s)
-            assert ar == ao and [(int(a), float(p)) for a, p in pr] == [(int(a), float(p)) for a, p in po]
-            s.apply_action(int(ar))
-        want = ref_gu.play_game(g, ref_bot.NeuralNetBot(g, 0, fa), ref_bot.NeuralNetBot(g, 1, fb))
+            assert ao == want["action"] and [[int(a), float(p)] for a, p in po] == want["policy"]
+            s.apply_action(int(ao))
         got = our_gu.play_game(g, our_bot.NeuralNetBot(g, 0, fa), our_bot.NeuralNetBot(g, 1, fb))
-        assert want == got
+        assert got == case["play_game"]
