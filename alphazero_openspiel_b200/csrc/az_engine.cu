@@ -5,7 +5,7 @@
 //   Node.expand            mcts.py:54-66           -> expand_node()
 //   Node.update_recursive  mcts.py:82-89           -> backup_path()
 //   MCTS.playout/search    mcts.py:126-180         -> k_step main loop
-//   expand_root_dirichlet  mcts.py:182-190         -> consume_root_eval()
+//   expand_root_dirichlet  mcts.py:182-190         -> expand_root()
 //   MCTS.update_root       mcts.py:192-203         -> reroot_compact()
 //   AlphaZeroBot.step      alphazerobot.py:42-93   -> finish_move()
 //   play_game_self targets game_utils.py:168-204   -> emit_record()
@@ -15,6 +15,7 @@
 //   hdr   [n_trees]            64-byte tree header (root/pending positions, phase, arena cursor)
 //   nodes [n_trees][2][cap]    24-byte records {uint2 {N, link}, double Q, double P}; link = first_child << 8 | n_children
 //   path  [n_trees][MAXD]      node indices root..leaf of the in-flight simulation
+//   cache [2^log2 entries]     AZ_F_EVAL_CACHE: evaluator outputs by position (CacheHead + float priors, see cache_find)
 // The children of a node are ONE contiguous block in legal (ascending action) order, so a lane group
 // reads a node's child statistics with three coalesced loads; the winning child's {N, link} comes back by
 // shuffle, which makes one dependent load round per tree level.  Actions are never stored: child k of a
@@ -82,6 +83,9 @@ struct Params {
   long long* dbg;      // optional [n_trees][4]: cycles, phase in, sims this step, flags (az_debug_timing)
   VlPend* vl_pend;     // AZ_F_VIRTUAL_LOSS: [n_trees][vl_k] in-flight requests
   int vl_k;            // leaves in flight per tree (evaluator rows per tree); 1 in the exact mode
+  uint8_t* cache;            // AZ_F_EVAL_CACHE table, nullptr when off
+  unsigned long long cache_mask;
+  uint32_t* cache_epoch;     // [0] epoch of the current weights, [1] epoch of the rows the next k_cache_insert stores
   const double* logtab;  // AZ_F_UCT: log(n) for n < LOGTAB_N, computed on the host with the C library's log() -- the same
                          // function CPython's math.log calls, so the UCT scores are bit-equal to the reference's
   long long rec_cap;
@@ -197,6 +201,36 @@ __device__ __forceinline__ double eval_value(const Params& p, const StepIO& io, 
   return (double)((int)((ek.k >> 20) & 31) - 16) / 16.0;
 }
 
+// ---------------------------------------------------------------- evaluator output cache (AZ_F_EVAL_CACHE)
+// One direct-mapped entry per slot: CacheHead, float priors[MAXC] in legal order, and a 32-bit insertion lock in the last
+// word; the stride is a power of two (64 B for Connect Four, 256 B for Breakthrough).  tag = epoch << 1 | (ply & 1), and the
+// epoch starts at 1, so a zeroed slot never matches.  The evaluator's output is a function of (b0, b1, ply & 1) alone (the
+// observation planes are built from exactly that), so a hit gives the float values a new evaluator row would give.
+struct CacheHead {
+  uint64_t b0, b1;
+  uint32_t tag;
+  float value;
+};
+static_assert(sizeof(CacheHead) == 24, "CacheHead size");
+template <class GM>
+__host__ __device__ constexpr int cache_stride() {
+  int s = 1;
+  while (s < (int)sizeof(CacheHead) + 4 * GM::MAXC + 4) s *= 2;
+  return s;
+}
+template <class GM>
+__device__ __forceinline__ uint8_t* cache_slot(const Params& p, const St& s) {
+  return p.cache + (size_t)(eval_key(p, s).k & p.cache_mask) * cache_stride<GM>();
+}
+// The entry of position s under the current weights, or nullptr.  The full key is compared: a hash collision is a miss.
+template <class GM>
+__device__ __forceinline__ const CacheHead* cache_find(const Params& p, const St& s) {
+  const CacheHead* e = reinterpret_cast<const CacheHead*>(cache_slot<GM>(p, s));
+  const uint32_t tag = (p.cache_epoch[0] << 1) | (uint32_t)(s.ply & 1);
+  return (e->b0 == s.b0 && e->b1 == s.b1 && e->tag == tag) ? e : nullptr;
+}
+__device__ __forceinline__ const float* cache_priors(const CacheHead* e) { return reinterpret_cast<const float*>(e + 1); }
+
 // Gamma(alpha<1) by Marsaglia-Tsang on alpha+1 with the U^(1/alpha) boost; counter stream 5.
 __device__ double gamma_draw(double alpha, uint64_t seed, uint64_t tree, uint64_t gseq, uint64_t ply, int child) {
   const double d = alpha + 1.0 - 1.0 / 3.0, c = 1.0 / sqrt(9.0 * d);
@@ -281,11 +315,13 @@ __device__ __forceinline__ void backup_path(const Arena& a, const int32_t* path,
 }
 
 // Node.expand (mcts.py:54-66).  noise != nullptr: root Dirichlet mix (mcts.py:186-189), eta indexed by legal position.
+// cached != nullptr: the priors come from an AZ_F_EVAL_CACHE entry (float, legal order) instead of the evaluator row.
 // Returns false on arena overflow (nothing written).
 template <class GM, int G>
 __device__ __forceinline__ bool expand_node(const Params& p, const StepIO& io, const Arena& a, TreeHdr& h, int tree,
                                             int node, const St& s, int lane, unsigned gm, bool root_mix,
-                                            const double* eta_lane /* [SLOTS] per-lane eta values */, int* L_out) {
+                                            const double* eta_lane /* [SLOTS] per-lane eta values */, int* L_out,
+                                            const float* cached = nullptr) {
   const typename GM::Legal lg = GM::legal(s, p.geo);
   const int L = GM::count(lg);
   *L_out = L;
@@ -307,8 +343,7 @@ __device__ __forceinline__ bool expand_node(const Params& p, const StepIO& io, c
   for (int sl = 0; sl < GM::SLOTS; ++sl) {
     const int i = lane + sl * G;
     if (i < L) {
-      const int act = GM::action_of(lg, s, p.geo, i);
-      double pr = eval_prior(p, io, tree, ek, act);
+      double pr = cached ? (double)cached[i] : eval_prior(p, io, tree, ek, GM::action_of(lg, s, p.geo, i));
       if (root_mix) pr = __dadd_rn(__dmul_rn(p.keep, pr), __dmul_rn(p.noise_w, eta_lane[sl]));
       a.p(fc + i) = pr;
       if (fresh) {
@@ -694,6 +729,59 @@ __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, uns
   h.phase = PH_BEGIN;
 }
 
+// expand_root_dirichlet (mcts.py:182-190): the root expansion with the noise mix, from the evaluator row (cached == nullptr)
+// or from an AZ_F_EVAL_CACHE entry's priors.  Leaves the tree in AZ_PH_RUN.
+template <class GM, int G>
+__device__ __forceinline__ void expand_root(const Params& p, const StepIO& io, TreeHdr& h, int tree, int lane, unsigned gm,
+                                          unsigned long long* s_ctr, const float* cached) {
+  const Arena a = arena_of(p, tree, h.half);
+  St s;
+  s.b0 = h.root_b0;
+  s.b1 = h.root_b1;
+  s.ply = h.root_ply;
+  const typename GM::Legal lg = GM::legal(s, p.geo);
+  const int L = GM::count(lg);
+  double eta[GM::SLOTS];
+#pragma unroll
+  for (int sl = 0; sl < GM::SLOTS; ++sl) eta[sl] = 0.0;
+  if (p.noise_mode == AZ_NOISE_HOST) {
+#pragma unroll
+    for (int sl = 0; sl < GM::SLOTS; ++sl) {
+      const int i = lane + sl * G;
+      if (i < L) eta[sl] = io.noise[(size_t)tree * GM::MAXC + i];
+    }
+  } else if (p.noise_mode == AZ_NOISE_COUNTER) {
+    double sum = 0.0;  // sequential sum in legal order, identical on every lane (oracle: oz_selfplay_game)
+    for (int i = 0; i < L; ++i) {
+      const double u = (double)((counter(p.seed, tree, h.game_seq, s.ply, i, 1) >> 11) + 1ULL) *
+                       (1.0 / 9007199254740992.0);
+      sum = __dadd_rn(sum, u);
+      if (i % G == lane) eta[i / G] = u;
+    }
+#pragma unroll
+    for (int sl = 0; sl < GM::SLOTS; ++sl) eta[sl] = __ddiv_rn(eta[sl], sum);
+  } else if (p.noise_mode == AZ_NOISE_DIRICHLET) {
+    double sum = 0.0;
+#pragma unroll
+    for (int sl = 0; sl < GM::SLOTS; ++sl) {
+      const int i = lane + sl * G;
+      if (i < L) eta[sl] = gamma_draw(p.alpha, p.seed, tree, h.game_seq, s.ply, i);
+      sum += eta[sl];
+    }
+    sum = gsumd<G>(gm, sum);
+#pragma unroll
+    for (int sl = 0; sl < GM::SLOTS; ++sl) eta[sl] = sum > 0.0 ? eta[sl] / sum : 1.0 / (double)L;
+  }
+  int L2 = 0;
+  const bool ok = expand_node<GM, G>(p, io, a, h, tree, h.root_node, s, lane, gm, true, eta, &L2, cached);
+  if (!ok) {
+    h.err = 1;
+    if (lane == 0) ctr_add(s_ctr, AZ_CTR_OVERFLOW, 1);
+  }
+  h.phase = AZ_PH_RUN;
+  if (lane == 0) ctr_add(s_ctr, AZ_CTR_ROOT_EVALS, 1);
+}
+
 // ---------------------------------------------------------------- the step kernel
 template <class GM, bool UCT>
 __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params p, const StepIO io) {
@@ -704,6 +792,8 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
   __syncthreads();
   const int tree = (int)((blockIdx.x * (unsigned)BLOCK + threadIdx.x) / G);
   const int lane = threadIdx.x % G;
+  // the rows k_cache_insert stores next are evaluated (after this launch) with the current weights
+  if (p.cache && blockIdx.x == 0 && threadIdx.x == 0) p.cache_epoch[1] = p.cache_epoch[0];
   if (tree < p.n_trees) {
     const unsigned gm = group_mask<G>();
     int32_t* spath = s_path[threadIdx.x / G];
@@ -739,52 +829,7 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
       c_exp += 1;
       c_legal += L;
     } else if (h.phase == AZ_PH_ROOT_EVAL) {
-      const Arena a = arena_of(p, tree, h.half);
-      St s;
-      s.b0 = h.root_b0;
-      s.b1 = h.root_b1;
-      s.ply = h.root_ply;
-      const typename GM::Legal lg = GM::legal(s, p.geo);
-      const int L = GM::count(lg);
-      double eta[GM::SLOTS];
-#pragma unroll
-      for (int sl = 0; sl < GM::SLOTS; ++sl) eta[sl] = 0.0;
-      if (p.noise_mode == AZ_NOISE_HOST) {
-#pragma unroll
-        for (int sl = 0; sl < GM::SLOTS; ++sl) {
-          const int i = lane + sl * G;
-          if (i < L) eta[sl] = io.noise[(size_t)tree * GM::MAXC + i];
-        }
-      } else if (p.noise_mode == AZ_NOISE_COUNTER) {
-        double sum = 0.0;  // sequential sum in legal order, identical on every lane (oracle: oz_selfplay_game)
-        for (int i = 0; i < L; ++i) {
-          const double u = (double)((counter(p.seed, tree, h.game_seq, s.ply, i, 1) >> 11) + 1ULL) *
-                           (1.0 / 9007199254740992.0);
-          sum = __dadd_rn(sum, u);
-          if (i % G == lane) eta[i / G] = u;
-        }
-#pragma unroll
-        for (int sl = 0; sl < GM::SLOTS; ++sl) eta[sl] = __ddiv_rn(eta[sl], sum);
-      } else if (p.noise_mode == AZ_NOISE_DIRICHLET) {
-        double sum = 0.0;
-#pragma unroll
-        for (int sl = 0; sl < GM::SLOTS; ++sl) {
-          const int i = lane + sl * G;
-          if (i < L) eta[sl] = gamma_draw(p.alpha, p.seed, tree, h.game_seq, s.ply, i);
-          sum += eta[sl];
-        }
-        sum = gsumd<G>(gm, sum);
-#pragma unroll
-        for (int sl = 0; sl < GM::SLOTS; ++sl) eta[sl] = sum > 0.0 ? eta[sl] / sum : 1.0 / (double)L;
-      }
-      int L2 = 0;
-      const bool ok = expand_node<GM, G>(p, io, a, h, tree, h.root_node, s, lane, gm, true, eta, &L2);
-      if (!ok) {
-        h.err = 1;
-        if (lane == 0) ctr_add(s_ctr, AZ_CTR_OVERFLOW, 1);
-      }
-      h.phase = AZ_PH_RUN;
-      if (lane == 0) ctr_add(s_ctr, AZ_CTR_ROOT_EVALS, 1);
+      expand_root<GM, G>(p, io, h, tree, lane, gm, s_ctr, nullptr);
     }
 
     if (p.dbg) t_consume = clock64() - t_start;
@@ -799,14 +844,19 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
           s.b0 = h.root_b0;
           s.b1 = h.root_b1;
           s.ply = h.root_ply;
-          h.phase = AZ_PH_ROOT_EVAL;
-          h.pend_b0 = s.b0;
-          h.pend_b1 = s.b1;
-          h.pend_ply = s.ply;
-          h.pend_depth = 0;
-          h.pend_node = h.root_node;
-          write_obs<GM, G>(p, io, tree, lane, s);
-          break;
+          const CacheHead* hit = p.cache ? cache_find<GM>(p, s) : nullptr;
+          if (hit) {
+            expand_root<GM, G>(p, io, h, tree, lane, gm, s_ctr, cache_priors(hit));
+          } else {
+            h.phase = AZ_PH_ROOT_EVAL;
+            h.pend_b0 = s.b0;
+            h.pend_b1 = s.b1;
+            h.pend_ply = s.ply;
+            h.pend_depth = 0;
+            h.pend_node = h.root_node;
+            write_obs<GM, G>(p, io, tree, lane, s);
+            break;
+          }
         }
         h.phase = AZ_PH_RUN;
       }
@@ -868,7 +918,27 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
         c_term += 1;
         continue;
       }
-      // non-terminal leaf: request the evaluator (mcts.py:146)
+      // non-terminal leaf: its evaluation from the cache, exactly as the AZ_PH_LEAF_EVAL consume path would apply the row
+      if (p.cache) {
+        const CacheHead* hit = cache_find<GM>(p, s);
+        if (hit) {
+          int L = 0;
+          if (!expand_node<GM, G>(p, io, a, h, tree, node, s, lane, gm, false, nullptr, &L, cache_priors(hit))) {
+            h.err = 1;
+            if (lane == 0) ctr_add(s_ctr, AZ_CTR_OVERFLOW, 1);
+          }
+          backup_path<G>(a, spath, depth, -(double)hit->value, lane);
+          __syncwarp(gm);
+          h.sims_done += 1;
+          c_sims += 1;
+          c_depth += depth;
+          c_exp += 1;
+          c_legal += L;
+          if (lane == 0) ctr_add(s_ctr, AZ_CTR_CACHE_HITS, 1);
+          continue;
+        }
+      }
+      // otherwise request the evaluator (mcts.py:146)
       h.pend_b0 = s.b0;
       h.pend_b1 = s.b1;
       h.pend_ply = s.ply;
@@ -903,6 +973,52 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
     else atomicAdd(&p.ctr[threadIdx.x], s_ctr[threadIdx.x]);
   }
 }
+
+// ---------------------------------------------------------------- evaluator cache insertion (AZ_F_EVAL_CACHE)
+// Runs right before k_step: stores the evaluator rows of every pending request (leaf or root) under the epoch of the weights
+// that computed them.  Lookups happen only in the following k_step, so no reader sees a half-written entry.  Two writers of
+// one launch may map to the same slot: the first to take the slot's lock writes the whole entry, the other skips its insert.
+template <class GM>
+__global__ void __launch_bounds__(BLOCK) k_cache_insert(const Params p, const StepIO io) {
+  constexpr int G = GM::G;
+  const int tree = (int)((blockIdx.x * (unsigned)BLOCK + threadIdx.x) / G);
+  const int lane = threadIdx.x % G;
+  if (tree >= p.n_trees) return;
+  const TreeHdr& h = p.hdr[tree];
+  if (h.phase != AZ_PH_LEAF_EVAL && h.phase != AZ_PH_ROOT_EVAL) return;
+  const unsigned gm = group_mask<G>();
+  St s;
+  s.b0 = h.pend_b0;
+  s.b1 = h.pend_b1;
+  s.ply = h.pend_ply;
+  uint8_t* slot = cache_slot<GM>(p, s);
+  unsigned* lock = reinterpret_cast<unsigned*>(slot + cache_stride<GM>() - 4);
+  int got = 0;
+  if (lane == 0) got = atomicCAS(lock, 0u, 1u) == 0u;
+  if (!gshfl<G>(gm, got, 0)) return;
+  const typename GM::Legal lg = GM::legal(s, p.geo);
+  const int L = GM::count(lg);
+  float* pri = reinterpret_cast<float*>(slot + sizeof(CacheHead));
+  const float* row = (const float*)io.priors + (size_t)tree * p.geo.n_actions;
+#pragma unroll
+  for (int sl = 0; sl < GM::SLOTS; ++sl) {
+    const int i = lane + sl * G;
+    if (i < L) pri[i] = row[GM::action_of(lg, s, p.geo, i)];
+  }
+  if (lane == 0) {
+    CacheHead e;
+    e.b0 = s.b0;
+    e.b1 = s.b1;
+    e.tag = (p.cache_epoch[1] << 1) | (uint32_t)(s.ply & 1);
+    e.value = ((const float*)io.values)[tree];
+    *reinterpret_cast<CacheHead*>(slot) = e;
+  }
+  __threadfence();
+  __syncwarp(gm);
+  if (lane == 0) atomicExch(lock, 0u);
+}
+
+__global__ void k_cache_new_epoch(uint32_t* epoch) { epoch[0] += 1u; }
 
 // ---------------------------------------------------------------- virtual-loss step kernel (AZ_F_VIRTUAL_LOSS)
 // Throughput mode for SMALL pools (BASELINE configs[1]: 1,024 games cannot fill the evaluator with one row per tree): every
@@ -1612,6 +1728,22 @@ int az_create(const az_config* cfg_in, az_engine** out) {
     return fail(-1, "AZ_F_VIRTUAL_LOSS is a batched self-play mode (no AZ_F_MANUAL / AZ_F_UCT)");
   if (cfg.record_capacity <= 0) cfg.record_capacity = cfg.n_trees * 64 < (1 << 20) ? (1 << 20) : cfg.n_trees * 64;
   if (!(cfg.flags & AZ_F_RECORDS)) cfg.record_capacity = 1;
+  if (cfg.flags & AZ_F_EVAL_CACHE) {
+    if (cfg.eval_mode != AZ_EVAL_EXTERNAL || (cfg.flags & (AZ_F_PRIORS_F64 | AZ_F_MANUAL | AZ_F_VIRTUAL_LOSS)) ||
+        cfg.noise_mode == AZ_NOISE_HOST)
+      return fail(-1, "AZ_F_EVAL_CACHE needs AZ_EVAL_EXTERNAL float outputs, no AZ_F_MANUAL / AZ_F_VIRTUAL_LOSS / "
+                      "AZ_NOISE_HOST");
+    int lg = (int)AZ_EVAL_CACHE_LOG2(cfg.flags);
+    if (lg == 0) {
+      lg = AZ_EVAL_CACHE_EXTRA_LOG2;
+      while ((1LL << lg) < (long long)cfg.n_trees * cfg.n_playouts << AZ_EVAL_CACHE_EXTRA_LOG2) ++lg;
+      lg = lg < 16 ? 16 : (lg > 27 ? 27 : lg);
+    }
+    if (lg > 30) return fail(-1, "evaluator cache size 2^%d: at most 2^30 entries", lg);
+    cfg.flags = (cfg.flags & ~(31u << AZ_EVAL_CACHE_LOG2_SHIFT)) | ((uint32_t)lg << AZ_EVAL_CACHE_LOG2_SHIFT);
+  } else {
+    cfg.flags &= ~(31u << AZ_EVAL_CACHE_LOG2_SHIFT);
+  }
 
   CK(cudaSetDevice(cfg.device));
   cudaDeviceProp prop;
@@ -1672,6 +1804,20 @@ int az_create(const az_config* cfg_in, az_engine** out) {
     az_destroy(e);
     return -2;
   }
+  if (cfg.flags & AZ_F_EVAL_CACHE) {
+    const size_t n = (size_t)1 << AZ_EVAL_CACHE_LOG2(cfg.flags);
+    const size_t cbytes = n * (cfg.game_id == AZ_GAME_CONNECT_FOUR ? cache_stride<C4>() : cache_stride<BT>());
+    if ((err = alloc((void**)&p.cache, cbytes)) != cudaSuccess ||
+        (err = alloc((void**)&p.cache_epoch, 2 * sizeof(uint32_t))) != cudaSuccess) {
+      fail(-2, "cudaMalloc failed (evaluator cache, %zu bytes): %s", cbytes, cudaGetErrorString(err));
+      az_destroy(e);
+      return -2;
+    }
+    p.cache_mask = n - 1;
+    const uint32_t epoch0[2] = {1u, 1u};  // a zeroed entry (tag 0) never matches
+    CK(cudaMemset(p.cache, 0, cbytes));
+    CK(cudaMemcpy(p.cache_epoch, epoch0, sizeof(epoch0), cudaMemcpyHostToDevice));
+  }
   if (cfg.flags & AZ_F_UCT) {
     double* tab = nullptr;
     if ((err = alloc((void**)&tab, sizeof(double) * LOGTAB_N)) != cudaSuccess) {
@@ -1712,6 +1858,8 @@ int az_destroy(az_engine* e) {
   cudaFree(p.compact_count);
   if (p.dbg) cudaFree(p.dbg);
   if (p.logtab) cudaFree(const_cast<double*>(p.logtab));
+  if (p.cache) cudaFree(p.cache);
+  if (p.cache_epoch) cudaFree(p.cache_epoch);
   cudaFree(e->d_cmd);
   cudaFree(e->d_bad);
   delete e;
@@ -1818,11 +1966,21 @@ int az_step(az_engine* e, const void* priors_dev, const void* values_dev, const 
   }
   dispatch_game(e->cfg.game_id, [&](auto gm) {
     using GM = decltype(gm);
+    // k_step stays the last launch of az_step: the evaluator's first kernel waits on it with griddepcontrol.wait
+    if (p.cache && priors_dev) k_cache_insert<GM><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p, io);
     if (p.flags & AZ_F_VIRTUAL_LOSS) k_step_vl<GM><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p, io);
     else if (p.flags & AZ_F_UCT) k_step<GM, true><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p, io);
     else k_step<GM, false><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p, io);
     return 0;
   });
+  CK(cudaGetLastError());
+  return 0;
+}
+
+int az_eval_cache_invalidate(az_engine* e, void* stream) {
+  if (!e) return fail(-1, "null engine");
+  if (!e->p.cache) return 0;
+  k_cache_new_epoch<<<1, 1, 0, (cudaStream_t)stream>>>(e->p.cache_epoch);
   CK(cudaGetLastError());
   return 0;
 }

@@ -56,7 +56,8 @@ class Engine:
     def __init__(self, game_name, n_trees, n_playouts=100, c_puct=2.5, dirichlet_ratio=0.25, temperature=1.0,
                  num_probabilistic_actions=1000, noise_mode=L.NOISE_DIRICHLET, eval_mode=L.EVAL_EXTERNAL,
                  eval_shift=None, flags=L.F_KEEP_TREE, seed=0, device=0, node_capacity=0, max_sims_per_step=0,
-                 start_plies_mod=0, record_capacity=0, max_games=0, leaves_per_tree=1, step_cycle_budget=0):
+                 start_plies_mod=0, record_capacity=0, max_games=0, leaves_per_tree=1, step_cycle_budget=0,
+                 eval_cache_log2=0):
         self.lib = L.load()
         if not torch.cuda.is_available():
             raise L.EngineUnavailable("the B200 engine needs a CUDA device; there is no CPU fallback")
@@ -73,6 +74,8 @@ class Engine:
         cfg.noise_mode, cfg.eval_mode = noise_mode, eval_mode
         cfg.eval_shift = (2 if gid == L.GAME_CONNECT_FOUR else 4) if eval_shift is None else eval_shift
         cfg.max_sims_per_step, cfg.start_plies_mod = max_sims_per_step, start_plies_mod
+        if flags & L.F_EVAL_CACHE:   # table size: 2^eval_cache_log2 entries, 0 = the engine's default
+            flags |= int(eval_cache_log2) << L.EVAL_CACHE_LOG2_SHIFT
         cfg.record_capacity, cfg.device, cfg.flags, cfg.seed = record_capacity, device, flags, seed
         cfg.max_games = max_games
         cfg.leaves_per_tree = leaves_per_tree if (flags & L.F_VIRTUAL_LOSS) else 1
@@ -84,6 +87,7 @@ class Engine:
         eff = L.AzConfig()
         L.check(self.lib.az_config_get(self.h, C.byref(eff)))
         self.cfg = eff
+        self.eval_cache_log2 = (eff.flags >> L.EVAL_CACHE_LOG2_SHIFT) & 31   # F_EVAL_CACHE table in use (0 = off)
         self.n_trees = n_trees
         self.flags = flags
         self.rows_per_tree = int(eff.leaves_per_tree)        # evaluator rows per tree (1 unless AZ_F_VIRTUAL_LOSS)
@@ -138,6 +142,10 @@ class Engine:
         """Re-root compaction of the trees that just moved (only needed with F_ASYNC_COMPACT)."""
         st = self._stream() if stream is None else C.c_void_p(stream.cuda_stream)
         L.check(self.lib.az_compact(self.h, st))
+
+    def invalidate_eval_cache(self):
+        """F_EVAL_CACHE: the evaluator's weights change after the rows already computed (az_eval_cache_invalidate)."""
+        L.check(self.lib.az_eval_cache_invalidate(self.h, self._stream()))
 
     def set_positions(self, histories):
         """histories: list (len n_trees) of action lists, or None entries to leave a tree untouched."""

@@ -157,7 +157,8 @@ class SelfPlayRunner:
                  dirichlet_ratio=0.25, temperature=1.0, num_probabilistic_actions=1000, keep_search_tree=True,
                  backup="on-policy", seed=0, max_games=0, auto_restart=True, random_start_mod=0,
                  max_sims_per_step=16, records=True, use_graph=True, noise_mode=None, node_capacity=0,
-                 record_capacity=0, evaluator="fused", virtual_loss=0, step_cycle_budget=None, **_ignored):
+                 record_capacity=0, evaluator="fused", virtual_loss=0, step_cycle_budget=None, eval_cache=None,
+                 eval_cache_log2=0, **_ignored):
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise L.EngineUnavailable("SelfPlayRunner needs a CUDA device; there is no CPU fallback")
@@ -189,15 +190,7 @@ class SelfPlayRunner:
         self.backup = backup
         self.game_name = game_name
         with torch.cuda.device(self.device):
-            self.engine = Engine(game_name, n_trees, n_playouts=n_playouts, c_puct=c_puct,
-                                 dirichlet_ratio=dirichlet_ratio, temperature=temperature,
-                                 num_probabilistic_actions=num_probabilistic_actions, noise_mode=noise_mode,
-                                 eval_mode=L.EVAL_EXTERNAL, flags=flags, seed=seed, device=dev_index,
-                                 max_sims_per_step=max_sims_per_step, start_plies_mod=random_start_mod,
-                                 max_games=max_games, node_capacity=node_capacity,
-                                 record_capacity=record_capacity, leaves_per_tree=leaves,
-                                 step_cycle_budget=step_cycle_budget)
-            n_rows = self.engine.n_rows
+            n_rows = n_trees * leaves
             if evaluator == "fused":      # hand-written tcgen05 convs (csrc/az_resnet.cu)
                 from .nn_fused import FusedEvaluator
                 self.evaluator = FusedEvaluator(net, n_rows, self.device)
@@ -205,6 +198,25 @@ class SelfPlayRunner:
                 self.evaluator = BatchedEvaluator(net, n_rows, self.device, use_graph=False)
             else:
                 raise ValueError("evaluator must be 'fused' or 'torch'")
+            # eval_cache (None = on where it is exact): expand leaves whose position was already evaluated from a device
+            # table of the evaluator's outputs (F_EVAL_CACHE) instead of sending them to the evaluator again.  Results are
+            # unchanged only if an output row depends on that row's board alone: true of the fused evaluator, not promised
+            # by cuDNN / cuBLAS (torch evaluator).  Virtual-loss mode has no cache.
+            cache_ok = getattr(self.evaluator, "row_independent", False) and not (flags & L.F_VIRTUAL_LOSS)
+            if eval_cache is None:
+                eval_cache = cache_ok
+            elif eval_cache and not cache_ok:
+                raise ValueError("eval_cache needs the fused evaluator (with its own FC head) and virtual_loss=0")
+            if eval_cache:
+                flags |= L.F_EVAL_CACHE
+            self.engine = Engine(game_name, n_trees, n_playouts=n_playouts, c_puct=c_puct,
+                                 dirichlet_ratio=dirichlet_ratio, temperature=temperature,
+                                 num_probabilistic_actions=num_probabilistic_actions, noise_mode=noise_mode,
+                                 eval_mode=L.EVAL_EXTERNAL, flags=flags, seed=seed, device=dev_index,
+                                 max_sims_per_step=max_sims_per_step, start_plies_mod=random_start_mod,
+                                 max_games=max_games, node_capacity=node_capacity,
+                                 record_capacity=record_capacity, leaves_per_tree=leaves,
+                                 step_cycle_budget=step_cycle_budget, eval_cache_log2=eval_cache_log2)
         self.use_graph = use_graph
         self._graph = None
         self._first = True
@@ -216,7 +228,10 @@ class SelfPlayRunner:
 
     def load_weights(self, net):
         """New generation's weights (host or device Net) into the captured evaluator, in place."""
-        self.evaluator.load(net)
+        with torch.cuda.device(self.device):
+            self.evaluator.load(net)
+            if self.engine.flags & L.F_EVAL_CACHE:
+                self.engine.invalidate_eval_cache()
 
     @torch.no_grad()
     def _round_eager(self):

@@ -70,6 +70,9 @@ class FusedEvaluator:
         # (AZ_NN_HEAD=0: cuBLAS + torch softmax/tanh, kept only as a numerics cross-check.)
         self.small_head = self.A + 1 <= 8 and 8 * (self.h * self.w * 8 + 4) * 16 <= 100 * 1024
         self.fused_head = os.environ.get("AZ_NN_HEAD", "1") != "0"
+        # every output row is a function of that row's board alone, whatever the other rows hold or where the row sits in
+        # the batch (our kernels give each row the same reduction order); the cuBLAS head does not promise that
+        self.row_independent = self.fused_head
         self.head_scratch = None
         if self.fused_head and not self.small_head:
             n = int(self.lib.az_nn_head_large_scratch_bytes(batch, self.A))

@@ -70,6 +70,21 @@ extern "C" {
                                           leaves in flight per tree, each path carrying a virtual loss until its evaluator
                                           row arrives.  The evaluator batch is n_trees * leaves_per_tree rows, row =
                                           tree * leaves_per_tree + slot, for priors, values and observations alike */
+#define AZ_F_EVAL_CACHE     (1u << 12) /* reuse evaluator outputs of positions already evaluated: a direct-mapped device table of
+                                          2^AZ_EVAL_CACHE_LOG2(flags) entries keyed by the full position (b0, b1, ply & 1) and a
+                                          weights epoch (az_eval_cache_invalidate).  A leaf (or a root awaiting its Dirichlet
+                                          expansion) whose position is in the table is expanded from the stored float priors and
+                                          value in the same launch instead of requesting an evaluator row.  Bit-exact only if the
+                                          evaluator's output for a row depends on that row's position alone (not on its place in the
+                                          batch).  Needs AZ_EVAL_EXTERNAL with float priors; not with AZ_F_MANUAL,
+                                          AZ_F_VIRTUAL_LOSS or AZ_NOISE_HOST */
+/* AZ_F_EVAL_CACHE table size in bits 24-28 of az_config.flags (so that az_config keeps its layout): log2 of the number of
+ * entries (64 B each for Connect Four, 256 B for Breakthrough), at most 30; 0 = default: 2^AZ_EVAL_CACHE_EXTRA_LOG2 entries
+ * per simulation of one search of every tree (n_trees * n_playouts, rounded up to a power of two), within 2^16..2^27.
+ * az_config_get reports the size in use. */
+#define AZ_EVAL_CACHE_LOG2_SHIFT 24
+#define AZ_EVAL_CACHE_LOG2(flags) (((flags) >> AZ_EVAL_CACHE_LOG2_SHIFT) & 31u)
+#define AZ_EVAL_CACHE_EXTRA_LOG2 1
 
 /* root noise (mcts.py:182-190) */
 #define AZ_NOISE_NONE      0 /* use_dirichlet=False */
@@ -146,16 +161,17 @@ enum {
   AZ_CTR_SIMS = 0,        /* completed simulations (MCTS.playout calls) */
   AZ_CTR_DEPTH,           /* sum of select depth */
   AZ_CTR_CHILDREN,        /* sum of children scored during select */
-  AZ_CTR_EXPANSIONS,      /* leaf expansions (= leaf evaluator calls) */
+  AZ_CTR_EXPANSIONS,      /* leaf expansions (evaluator rows answered + AZ_CTR_CACHE_HITS) */
   AZ_CTR_LEGAL,           /* sum of legal moves at expansion */
   AZ_CTR_TERMINAL,        /* simulations that ended on a terminal leaf */
-  AZ_CTR_ROOT_EVALS,      /* root (Dirichlet) evaluator calls */
+  AZ_CTR_ROOT_EVALS,      /* root (Dirichlet) expansions, from an evaluator row or the AZ_F_EVAL_CACHE table */
   AZ_CTR_MOVES,           /* plies played */
   AZ_CTR_GAMES,           /* games finished */
   AZ_CTR_COMPACT_NODES,   /* nodes copied by re-root compaction */
   AZ_CTR_OVERFLOW,        /* arena/depth/record overflows -- must stay 0 */
   AZ_CTR_IDLE_SLOTS,      /* evaluator rows wasted (no request from that tree this step) */
   AZ_CTR_PEAK_NODES,      /* high-water mark of nodes in use in one tree's arena half (size node_capacity from it) */
+  AZ_CTR_CACHE_HITS,      /* leaf expansions served from the AZ_F_EVAL_CACHE table (no evaluator row) */
   AZ_CTR_COUNT
 };
 
@@ -198,6 +214,11 @@ int az_command(az_engine* e, const int32_t* update_root_host, const int32_t* res
  * eval_batch(obs) -> (priors, values). */
 int az_step(az_engine* e, const void* priors_dev, const void* values_dev, const double* noise_dev,
             void* obs_dev, int32_t obs_format, void* stream);
+
+/* AZ_F_EVAL_CACHE: the evaluator's weights change after this call.  Stream-ordered: evaluator rows that az_step consumes
+ * next were computed before the change and are still stored under the old weights; from that az_step on, entries of the
+ * old weights no longer match. */
+int az_eval_cache_invalidate(az_engine* e, void* stream);
 
 /* Re-root compaction (MCTS.update_root, mcts.py:192-203) of the trees that played a move in the last az_step: BFS-copies
  * the kept subtree into the other arena half, one warp per tree.  az_step runs it first by itself unless
