@@ -13,13 +13,15 @@ F_EAGER_COMPACT = 1 << 9
 F_UCT = 1 << 10
 F_VIRTUAL_LOSS = 1 << 11
 F_EVAL_CACHE = 1 << 12
+F_RESIGN = 1 << 13
 EVAL_CACHE_LOG2_SHIFT = 24   # flags bits 24-28: log2 of the F_EVAL_CACHE table's entries (0 = default)
 NOISE_NONE, NOISE_DIRICHLET, NOISE_HOST, NOISE_COUNTER = 0, 1, 2, 3
 EVAL_EXTERNAL, EVAL_UNIFORM, EVAL_HASH, EVAL_ROLLOUT = 0, 1, 2, 3
 OBS_NONE, OBS_F32_NCHW, OBS_BF16_NHWC = 0, 1, 2
 PH_IDLE, PH_ROOT_EVAL, PH_LEAF_EVAL, PH_SEARCH_DONE, PH_RUN, PH_ERROR = 0, 1, 2, 3, 4, 5
 CTR_NAMES = ["sims", "depth", "children", "expansions", "legal", "terminal", "root_evals", "moves", "games",
-             "compact_nodes", "overflow", "idle_slots", "peak_nodes", "cache_hits"]
+             "compact_nodes", "overflow", "idle_slots", "peak_nodes", "cache_hits", "resigns", "resign_samples",
+             "resign_false"]
 
 
 class AzConfig(C.Structure):
@@ -38,7 +40,7 @@ class AzConfig(C.Structure):
 class AzRecord(C.Structure):
     _fields_ = [
         ("tree", C.c_int32), ("game_seq", C.c_int32), ("ply", C.c_int32), ("action", C.c_int32),
-        ("n_legal", C.c_int32), ("kind", C.c_int32), ("root_n", C.c_int32), ("pad", C.c_int32),
+        ("n_legal", C.c_int32), ("kind", C.c_int32), ("root_n", C.c_int32), ("end", C.c_int32),
         ("bb", C.c_uint64 * 2),
         ("root_q", C.c_double), ("v_a0c", C.c_double), ("v_offpolicy", C.c_double),
     ]
@@ -68,6 +70,7 @@ SIGNATURES = {
     "az_step": (C.c_int, [C.c_void_p, _VP, _VP, _F64P, _VP, C.c_int32, _VP]),
     "az_compact": (C.c_int, [C.c_void_p, _VP]),
     "az_eval_cache_invalidate": (C.c_int, [C.c_void_p, _VP]),
+    "az_set_resign": (C.c_int, [C.c_void_p, C.c_double, C.c_int32, _VP]),
     "az_debug_timing": (C.c_int, [C.c_void_p, _VP]),
     "az_status": (C.c_int, [C.c_void_p, _I32P, _I32P, _I32P, _I32P, _VP]),
     "az_request_info": (C.c_int, [C.c_void_p, _U64P, _I32P, _I32P, _I32P, C.c_int32, _VP]),

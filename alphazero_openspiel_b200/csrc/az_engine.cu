@@ -69,6 +69,19 @@ struct __align__(16) VlPend {
   int32_t node, depth, ply, valid;
 };
 
+// AZ_F_RESIGN: the values of az_set_resign, and per tree the state of its current game.  Kept out of TreeHdr, which k_step
+// carries through its whole loop; only finish_move touches ResignTree.
+struct ResignCfg {
+  double threshold;
+  int32_t permille;
+  int32_t pad;
+};
+struct ResignTree {
+  double rmin[2];   // calibration game: minimum r of player 0 / 1 so far (2.0: not moved yet)
+  int32_t game_seq; // game this entry belongs to (-1 after az_reset: initialised at the game's first searched position)
+  int32_t calib;    // no-resign calibration game
+};
+
 struct Node;
 struct Params {
   TreeHdr* hdr;
@@ -86,6 +99,8 @@ struct Params {
   uint8_t* cache;            // AZ_F_EVAL_CACHE table, nullptr when off
   unsigned long long cache_mask;
   uint32_t* cache_epoch;     // [0] epoch of the current weights, [1] epoch of the rows the next k_cache_insert stores
+  ResignCfg* resign_cfg;     // AZ_F_RESIGN, nullptr when off
+  ResignTree* resign_tree;   // AZ_F_RESIGN: [n_trees]
   const double* logtab;  // AZ_F_UCT: log(n) for n < LOGTAB_N, computed on the host with the C library's log() -- the same
                          // function CPython's math.log calls, so the UCT scores are bit-equal to the reference's
   long long rec_cap;
@@ -535,7 +550,7 @@ __device__ St start_position(const Params& p, int tree, int gseq) {
 // training record (game_utils.py:168-194); returns through *slot_out the record slot or -1
 template <class GM, int G>
 __device__ void emit_record(const Params& p, int tree, const TreeHdr& h, const St& s, int kind, int action, int n_legal,
-                            int root_n, double root_q, double v_a0c, double v_off, const int* counts_lane,
+                            int root_n, double root_q, double v_a0c, double v_off, int end, const int* counts_lane,
                             const typename GM::Legal* lg, int lane, unsigned gm, unsigned long long* s_ctr) {
   long long slot = 0;
   if (lane == 0) slot = (long long)atomicAdd(p.rec_count, 1ULL);
@@ -554,7 +569,7 @@ __device__ void emit_record(const Params& p, int tree, const TreeHdr& h, const S
     r.n_legal = n_legal;
     r.kind = kind;
     r.root_n = root_n;
-    r.pad = 0;
+    r.end = end;
     r.bb[0] = s.b0;
     r.bb[1] = s.b1;
     r.root_q = root_q;
@@ -573,6 +588,81 @@ __device__ void emit_record(const Params& p, int tree, const TreeHdr& h, const S
       act[i] = have ? (int16_t)GM::action_of(*lg, s, p.geo, i) : (int16_t)-1;
     }
   }
+}
+
+// A game is over (terminal position or resignation): count it, then start the next game in the slot (AZ_F_AUTO_RESTART,
+// within the max_games tickets) or leave the tree idle at the final position s_end.
+template <class GM, int G>
+__device__ void end_game(const Params& p, TreeHdr& h, int tree, int lane, unsigned gm, unsigned long long* s_ctr,
+                         const St& s_end) {
+  if (lane == 0) ctr_add(s_ctr, AZ_CTR_GAMES, 1);
+  bool restart = (p.flags & AZ_F_AUTO_RESTART) != 0;
+  if (restart && p.max_games > 0) {
+    int ticket = 0;
+    if (lane == 0) ticket = atomicAdd(p.games_started, 1);
+    ticket = gshfl<G>(gm, ticket, 0);
+    restart = ticket < p.max_games;
+  }
+  if (restart) {
+    h.game_seq += 1;
+    const St s0 = start_position<GM>(p, tree, h.game_seq);
+    h.root_b0 = s0.b0;
+    h.root_b1 = s0.b1;
+    h.root_ply = s0.ply;
+    fresh_tree<G>(p, h, tree, lane, gm);
+    h.phase = PH_BEGIN;
+  } else {
+    h.root_b0 = s_end.b0;
+    h.root_b1 = s_end.b1;
+    h.root_ply = s_end.ply;
+    h.phase = AZ_PH_IDLE;
+  }
+}
+
+// AZ_F_RESIGN at a searched root of the mover m = ply & 1 (see AZ_F_RESIGN in az_b200.h): starts the tree's ResignTree entry
+// at the game's first searched position, keeps a calibration game's minimum r, and returns whether the game resigns here.
+template <int G>
+__device__ bool resign_check(const Params& p, const TreeHdr& h, int tree, int lane, unsigned gm, int ply, double root_q,
+                             double a0c) {
+  ResignTree* rp = p.resign_tree + tree;
+  ResignTree t = *rp;
+  const ResignCfg c = *p.resign_cfg;
+  if (t.game_seq != h.game_seq) {
+    t.game_seq = h.game_seq;
+    t.calib = (int)(counter(p.seed, tree, h.game_seq, 0, 0, 6) % 1000ULL) < c.permille ? 1 : 0;
+    t.rmin[0] = 2.0;
+    t.rmin[1] = 2.0;
+  }
+  const double r = a0c > -root_q ? a0c : -root_q;
+  if (t.calib) {
+    if (ply & 1) {
+      if (r < t.rmin[1]) t.rmin[1] = r;
+    } else {
+      if (r < t.rmin[0]) t.rmin[0] = r;
+    }
+  }
+  __syncwarp(gm);  // every lane has read the entry before lane 0 overwrites it
+  if (lane == 0) *rp = t;
+  return !t.calib && r < c.threshold;
+}
+
+// AZ_F_RESIGN, game over at a terminal position: for a calibration game, count it and its would-be false resignations
+// (players whose minimum r is below the current threshold and who did not lose; out = GM::outcome) and return end = 2 with
+// the two minima, else end = 0.
+template <int G>
+__device__ int resign_game_over(const Params& p, int tree, int lane, unsigned gm, int out, unsigned long long* s_ctr,
+                                double& rmin0, double& rmin1) {
+  __syncwarp(gm);  // lane 0's write of the entry in resign_check is visible
+  const ResignTree t = p.resign_tree[tree];
+  if (!t.calib) return 0;
+  rmin0 = t.rmin[0];
+  rmin1 = t.rmin[1];
+  if (lane == 0) {
+    const double thr = p.resign_cfg->threshold;
+    ctr_add(s_ctr, AZ_CTR_RESIGN_SAMPLES, 1);
+    ctr_add(s_ctr, AZ_CTR_RESIGN_FALSE, (unsigned long long)((rmin0 < thr && out != 1) + (rmin1 < thr && out != 0)));
+  }
+  return 2;
 }
 
 // AlphaZeroBot.step after the search (alphazerobot.py:72-93) + play_game_self bookkeeping (game_utils.py:156-204).
@@ -615,8 +705,19 @@ __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, uns
 
   if (p.flags & AZ_F_MANUAL) {
     if (p.flags & AZ_F_RECORDS)
-      emit_record<GM, G>(p, tree, h, s, 0, -1, L, (int)rnl.x, root_q, a0c, v_off, cnt, &lg, lane, gm, s_ctr);
+      emit_record<GM, G>(p, tree, h, s, 0, -1, L, (int)rnl.x, root_q, a0c, v_off, 0, cnt, &lg, lane, gm, s_ctr);
     h.phase = AZ_PH_SEARCH_DONE;
+    return;
+  }
+
+  if ((p.flags & AZ_F_RESIGN) && resign_check<G>(p, h, tree, lane, gm, s.ply, root_q, a0c)) {
+    if (p.flags & AZ_F_RECORDS) {
+      emit_record<GM, G>(p, tree, h, s, 0, -1, L, (int)rnl.x, root_q, a0c, v_off, 0, cnt, &lg, lane, gm, s_ctr);
+      const double ret0 = (s.ply & 1) ? 1.0 : -1.0;  // the mover loses
+      emit_record<GM, G>(p, tree, h, s, 1, -1, 0, 0, ret0, 0.0, 0.0, 1, nullptr, nullptr, lane, gm, s_ctr);
+    }
+    if (lane == 0) ctr_add(s_ctr, AZ_CTR_RESIGNS, 1);
+    end_game<GM, G>(p, h, tree, lane, gm, s_ctr, s);
     return;
   }
 
@@ -671,39 +772,21 @@ __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, uns
   }
   const int action = GM::action_of(lg, s, p.geo, k);
   if (p.flags & AZ_F_RECORDS)
-    emit_record<GM, G>(p, tree, h, s, 0, action, L, (int)rnl.x, root_q, a0c, v_off, cnt, &lg, lane, gm, s_ctr);
+    emit_record<GM, G>(p, tree, h, s, 0, action, L, (int)rnl.x, root_q, a0c, v_off, 0, cnt, &lg, lane, gm, s_ctr);
 
   // ---- apply (game_utils.py:197)
   const St s2 = GM::apply(s, p.geo, action);
   if (lane == 0) ctr_add(s_ctr, AZ_CTR_MOVES, 1);
   const int out = GM::outcome(s2, p.geo);
   if (out >= 0) {
+    double rmin0 = 0.0, rmin1 = 0.0;
+    int end = 0;
+    if (p.flags & AZ_F_RESIGN) end = resign_game_over<G>(p, tree, lane, gm, out, s_ctr, rmin0, rmin1);
     if (p.flags & AZ_F_RECORDS) {
       const double ret0 = out == 2 ? 0.0 : (out == 0 ? 1.0 : -1.0);
-      emit_record<GM, G>(p, tree, h, s2, 1, -1, 0, 0, ret0, 0.0, 0.0, nullptr, nullptr, lane, gm, s_ctr);
+      emit_record<GM, G>(p, tree, h, s2, 1, -1, 0, 0, ret0, rmin0, rmin1, end, nullptr, nullptr, lane, gm, s_ctr);
     }
-    if (lane == 0) ctr_add(s_ctr, AZ_CTR_GAMES, 1);
-    bool restart = (p.flags & AZ_F_AUTO_RESTART) != 0;
-    if (restart && p.max_games > 0) {
-      int ticket = 0;
-      if (lane == 0) ticket = atomicAdd(p.games_started, 1);
-      ticket = gshfl<G>(gm, ticket, 0);
-      restart = ticket < p.max_games;
-    }
-    if (restart) {
-      h.game_seq += 1;
-      const St s0 = start_position<GM>(p, tree, h.game_seq);
-      h.root_b0 = s0.b0;
-      h.root_b1 = s0.b1;
-      h.root_ply = s0.ply;
-      fresh_tree<G>(p, h, tree, lane, gm);
-      h.phase = PH_BEGIN;
-    } else {
-      h.root_b0 = s2.b0;
-      h.root_b1 = s2.b1;
-      h.root_ply = s2.ply;
-      h.phase = AZ_PH_IDLE;
-    }
+    end_game<GM, G>(p, h, tree, lane, gm, s_ctr, s2);
     return;
   }
   h.root_b0 = s2.b0;
@@ -1726,6 +1809,8 @@ int az_create(const az_config* cfg_in, az_engine** out) {
   if (cfg.leaves_per_tree > 64) return fail(-1, "leaves_per_tree must be <= 64");
   if ((cfg.flags & AZ_F_VIRTUAL_LOSS) && (cfg.flags & (AZ_F_MANUAL | AZ_F_UCT)))
     return fail(-1, "AZ_F_VIRTUAL_LOSS is a batched self-play mode (no AZ_F_MANUAL / AZ_F_UCT)");
+  if ((cfg.flags & AZ_F_RESIGN) && (cfg.flags & AZ_F_MANUAL))
+    return fail(-1, "AZ_F_RESIGN is a batched self-play mode: with AZ_F_MANUAL the host decides the moves");
   if (cfg.record_capacity <= 0) cfg.record_capacity = cfg.n_trees * 64 < (1 << 20) ? (1 << 20) : cfg.n_trees * 64;
   if (!(cfg.flags & AZ_F_RECORDS)) cfg.record_capacity = 1;
   if (cfg.flags & AZ_F_EVAL_CACHE) {
@@ -1818,6 +1903,16 @@ int az_create(const az_config* cfg_in, az_engine** out) {
     CK(cudaMemset(p.cache, 0, cbytes));
     CK(cudaMemcpy(p.cache_epoch, epoch0, sizeof(epoch0), cudaMemcpyHostToDevice));
   }
+  if (cfg.flags & AZ_F_RESIGN) {
+    if ((err = alloc((void**)&p.resign_cfg, sizeof(ResignCfg))) != cudaSuccess ||
+        (err = alloc((void**)&p.resign_tree, sizeof(ResignTree) * (size_t)cfg.n_trees)) != cudaSuccess) {
+      fail(-2, "cudaMalloc failed (resignation state): %s", cudaGetErrorString(err));
+      az_destroy(e);
+      return -2;
+    }
+    const ResignCfg rc0 = {-1.0, 0, 0};  // never resigns
+    CK(cudaMemcpy(p.resign_cfg, &rc0, sizeof(rc0), cudaMemcpyHostToDevice));
+  }
   if (cfg.flags & AZ_F_UCT) {
     double* tab = nullptr;
     if ((err = alloc((void**)&tab, sizeof(double) * LOGTAB_N)) != cudaSuccess) {
@@ -1860,6 +1955,8 @@ int az_destroy(az_engine* e) {
   if (p.logtab) cudaFree(const_cast<double*>(p.logtab));
   if (p.cache) cudaFree(p.cache);
   if (p.cache_epoch) cudaFree(p.cache_epoch);
+  if (p.resign_cfg) cudaFree(p.resign_cfg);
+  if (p.resign_tree) cudaFree(p.resign_tree);
   cudaFree(e->d_cmd);
   cudaFree(e->d_bad);
   delete e;
@@ -1882,6 +1979,8 @@ int az_reset(az_engine* e, void* stream) {
   const Params p = e->p;
   CK(cudaMemcpyAsync(p.games_started, &e->cfg.n_trees, sizeof(int), cudaMemcpyHostToDevice, st));
   CK(cudaMemsetAsync(p.compact_count, 0, sizeof(int) * 2, st));
+  // game_seq -1: every tree's entry is started afresh at its first searched position
+  if (p.resign_tree) CK(cudaMemsetAsync(p.resign_tree, 0xff, sizeof(ResignTree) * (size_t)p.n_trees, st));
   dispatch_game(e->cfg.game_id, [&](auto gm) {
     using GM = decltype(gm);
     k_reset<GM><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p);
@@ -1982,6 +2081,18 @@ int az_eval_cache_invalidate(az_engine* e, void* stream) {
   if (!e->p.cache) return 0;
   k_cache_new_epoch<<<1, 1, 0, (cudaStream_t)stream>>>(e->p.cache_epoch);
   CK(cudaGetLastError());
+  return 0;
+}
+
+int az_set_resign(az_engine* e, double threshold, int32_t disabled_permille, void* stream) {
+  if (!e) return fail(-1, "null engine");
+  if (!e->p.resign_cfg) return fail(-1, "az_set_resign: the engine was created without AZ_F_RESIGN");
+  if (!isfinite(threshold)) return fail(-1, "az_set_resign: the threshold must be finite");
+  if (disabled_permille < 0 || disabled_permille > 1000)
+    return fail(-1, "az_set_resign: disabled_permille %d is outside [0, 1000]", disabled_permille);
+  const ResignCfg rc = {threshold, disabled_permille, 0};
+  // pageable source: the copy has been staged when the call returns
+  CK(cudaMemcpyAsync(e->p.resign_cfg, &rc, sizeof(rc), cudaMemcpyHostToDevice, (cudaStream_t)stream));
   return 0;
 }
 

@@ -37,11 +37,11 @@ def game_shape(name):
 
 def record_dtype(max_children, stride):
     return np.dtype({
-        "names": ["tree", "game_seq", "ply", "action", "n_legal", "kind", "root_n", "bb", "root_q", "v_a0c",
+        "names": ["tree", "game_seq", "ply", "action", "n_legal", "kind", "root_n", "end", "bb", "root_q", "v_a0c",
                   "v_offpolicy", "counts", "actions"],
-        "formats": ["<i4", "<i4", "<i4", "<i4", "<i4", "<i4", "<i4", ("<u8", (2,)), "<f8", "<f8", "<f8",
+        "formats": ["<i4", "<i4", "<i4", "<i4", "<i4", "<i4", "<i4", "<i4", ("<u8", (2,)), "<f8", "<f8", "<f8",
                     ("<i4", (max_children,)), ("<i2", (max_children,))],
-        "offsets": [0, 4, 8, 12, 16, 20, 24, 32, 48, 56, 64, 72, 72 + 4 * max_children],
+        "offsets": [0, 4, 8, 12, 16, 20, 24, 28, 32, 48, 56, 64, 72, 72 + 4 * max_children],
         "itemsize": stride,
     })
 
@@ -146,6 +146,11 @@ class Engine:
     def invalidate_eval_cache(self):
         """F_EVAL_CACHE: the evaluator's weights change after the rows already computed (az_eval_cache_invalidate)."""
         L.check(self.lib.az_eval_cache_invalidate(self.h, self._stream()))
+
+    def set_resign(self, threshold, disabled_permille):
+        """F_RESIGN: resign threshold and per-mille share of no-resign calibration games (az_set_resign), stream-ordered:
+        a captured graph of step() sees the new values on its next replay."""
+        L.check(self.lib.az_set_resign(self.h, float(threshold), int(disabled_permille), self._stream()))
 
     def set_positions(self, histories):
         """histories: list (len n_trees) of action lists, or None entries to leave a tree untouched."""

@@ -143,6 +143,21 @@ def records_to_games(records, game_name, backup="on-policy"):
     return games
 
 
+def resign_threshold_for(records, target_fp, current):
+    """Resign threshold calibrated on the no-resign games (F_RESIGN records of kind 1 with end == 2): the minimum r of every
+    player of such a game who did not lose, sorted v_1 <= ... <= v_n, gives v_(k+1) with k = floor(target_fp * n), capped at
+    1.0 -- so at most a target_fp share of those players would have resigned below it.  `current` when there is no value
+    (n == 0) or k >= n.  A player who never moved (minimum 2.0) has no value."""
+    ends = records[(records["kind"] == 1) & (records["end"] == 2)]
+    ret0 = ends["root_q"]
+    v = np.concatenate([ends["v_a0c"][ret0 >= 0], ends["v_offpolicy"][ret0 <= 0]]).astype(np.float64)
+    v = np.sort(v[v <= 1.0])
+    k = int(np.floor(target_fp * len(v)))
+    if k >= len(v):
+        return current
+    return min(float(v[k]), 1.0)
+
+
 def start_key_prefix(bb, ply):
     """'' for a game from the initial position, else a tag of the position the game started from."""
     if int(ply) == 0:
@@ -158,7 +173,7 @@ class SelfPlayRunner:
                  backup="on-policy", seed=0, max_games=0, auto_restart=True, random_start_mod=0,
                  max_sims_per_step=16, records=True, use_graph=True, noise_mode=None, node_capacity=0,
                  record_capacity=0, evaluator="fused", virtual_loss=0, step_cycle_budget=None, eval_cache=None,
-                 eval_cache_log2=0, **_ignored):
+                 eval_cache_log2=0, resign_threshold=None, resign_disabled_fraction=0.1, **_ignored):
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise L.EngineUnavailable("SelfPlayRunner needs a CUDA device; there is no CPU fallback")
@@ -175,6 +190,8 @@ class SelfPlayRunner:
                 flags |= L.F_OFFPOLICY
         if random_start_mod > 0:
             flags |= L.F_RANDOM_START
+        if resign_threshold is not None:
+            flags |= L.F_RESIGN     # resignation (an extension: the reference plays every game to its end)
         if noise_mode is None:
             noise_mode = L.NOISE_DIRICHLET if use_dirichlet else L.NOISE_NONE
         # virtual_loss = K > 0: K leaves in flight per tree (AZ_F_VIRTUAL_LOSS, NOT bit-exact with the reference), for pools
@@ -217,6 +234,8 @@ class SelfPlayRunner:
                                  max_games=max_games, node_capacity=node_capacity,
                                  record_capacity=record_capacity, leaves_per_tree=leaves,
                                  step_cycle_budget=step_cycle_budget, eval_cache_log2=eval_cache_log2)
+        if resign_threshold is not None:
+            self.set_resign(resign_threshold, resign_disabled_fraction)
         self.use_graph = use_graph
         self._graph = None
         self._first = True
@@ -232,6 +251,12 @@ class SelfPlayRunner:
             self.evaluator.load(net)
             if self.engine.flags & L.F_EVAL_CACHE:
                 self.engine.invalidate_eval_cache()
+
+    def set_resign(self, threshold, disabled_fraction=0.1):
+        """Resign threshold and share of no-resign calibration games (needs resign_threshold at construction).  Takes effect
+        on the next round, also in an already captured graph."""
+        with torch.cuda.device(self.device):
+            self.engine.set_resign(threshold, int(round(float(disabled_fraction) * 1000)))
 
     @torch.no_grad()
     def _round_eager(self):
@@ -309,7 +334,15 @@ class ExampleGenerator:
         self.game_name = game_name
         self.kwargs = kwargs
         self.rank0_only = bool(self.kwargs.pop("rank0_only", False))
+        # resignation: with resign_threshold set, last_stats["resign_threshold_suggested"] is the threshold at which a
+        # resign_false_positive share of the calibration games' non-losing players would have resigned
+        self.resign_false_positive = float(self.kwargs.pop("resign_false_positive", 0.05))
         self.last_stats = {}
+
+    def _resign_suggestion(self, records, stats):
+        current = self.kwargs.get("resign_threshold")
+        stats["resign_threshold_suggested"] = None if current is None else \
+            resign_threshold_for(records, self.resign_false_positive, current)
 
     def generate_examples(self, n_games):
         """Play n_games self-play games (split over ranks when torch.distributed is initialised)."""
@@ -320,6 +353,7 @@ class ExampleGenerator:
         records, stats = self._play(share, seed_offset=rank)
         if world > 1:
             records = parallel.gather_records(records, self.device)
+        self._resign_suggestion(records, stats)     # on the gathered records: every rank derives the same value
         backup = str(self.kwargs.get("backup", "on-policy"))
         # rank0_only (Trainer: only rank 0 trains): the other ranks skip the host-side conversion and return no games
         games = [] if (self.rank0_only and rank != 0) else records_to_games(records, self.game_name, backup)
@@ -340,6 +374,7 @@ class ExampleGenerator:
         records, stats = self._play(share, seed_offset=rank)
         if world > 1:
             records = parallel.gather_records(records, self.device)
+        self._resign_suggestion(records, stats)
         if self.rank0_only and rank != 0:
             records = records[:0]
         batch = ExampleBatch.from_records(records, self.game_name, str(self.kwargs.get("backup", "on-policy")))

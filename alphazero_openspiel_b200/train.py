@@ -68,6 +68,15 @@ class Trainer:
         # static minibatch buffers -- the 5x50 network at batch 256 is launch-bound in eager mode (~60 kernels of a few
         # microseconds per step).  Same arithmetic, same sampling calls.  Needs device_training; not combined with ddp.
         self.graph_step = False
+        # Extension: resignation in self-play (AlphaGo Zero; the reference plays every game to its end).  A game resigns once
+        # its mover's root value and best child value are both below resign_threshold (-1: never, until the first
+        # calibration); a resign_disabled_fraction share of the games never resigns, and after every generation the
+        # threshold becomes the one at which a resign_false_positive share of those games' non-losing players would have
+        # resigned.
+        self.resign = False
+        self.resign_false_positive = 0.05
+        self.resign_disabled_fraction = 0.1
+        self.resign_threshold = -1.0
         for k, v in overrides.items():
             if not hasattr(self, k):
                 raise TypeError("unknown Trainer setting %r" % k)
@@ -268,6 +277,10 @@ class Trainer:
     # ------------------------------------------------------------------ generation (train.py:203-236)
     def generate_examples(self, n_games, **engine_kwargs):
         start = time.time()
+        if self.resign:
+            engine_kwargs = dict(engine_kwargs, resign_threshold=self.resign_threshold,
+                                 resign_disabled_fraction=self.resign_disabled_fraction,
+                                 resign_false_positive=self.resign_false_positive)
         generator = ExampleGenerator(self.current_net, self.name_game, self.device,
                                      n_playouts=self.n_playouts_train, temperature=self.temperature,
                                      dirichlet_ratio=self.dirichlet_ratio, c_puct=self.uct_train, backup=self.backup,
@@ -292,6 +305,13 @@ class Trainer:
                 self.buffer.append(examples)
         self.games_played += self.n_games_per_generation
         self.last_generation_stats = dict(generator.last_stats, seconds=time.time() - start, games=n_new)
+        if self.resign:
+            self.last_generation_stats["resign_threshold"] = self.resign_threshold
+            self.resign_threshold = generator.last_stats["resign_threshold_suggested"]
+            logger.info("Resignation: %d resigned, %d calibration games, %d false positives; threshold %.4f -> %.4f" % (
+                generator.last_stats.get("resigns", 0), generator.last_stats.get("resign_samples", 0),
+                generator.last_stats.get("resign_false", 0), self.last_generation_stats["resign_threshold"],
+                self.resign_threshold))
         logger.info("Finished Generating Data. Took: " + str(time.time() - start) + " seconds")
         self.update_buffer_size()
         if self.device_training:

@@ -35,7 +35,8 @@
  * Deterministic counter streams (AZ_NOISE_COUNTER / AZ_F_SAMPLE_COUNTER / az_reset_random / AZ_EVAL_HASH):
  *   mix64 = splitmix64 finaliser; counter(seed,tree,game_seq,ply,idx,stream) = 6 chained mix64
  *   (oracle/az_oracle.c:oz_counter is the CPU restatement).  stream 1 = root noise, 2 = move sampling,
- *   3 = random start plies, 4 = number of random start plies, 5 = device Dirichlet gammas.
+ *   3 = random start plies, 4 = number of random start plies, 5 = device Dirichlet gammas,
+ *   6 = no-resign calibration games (AZ_F_RESIGN: counter(seed,tree,game_seq,0,0,6) % 1000 < disabled_permille).
  */
 #ifndef AZ_B200_H
 #define AZ_B200_H
@@ -82,6 +83,15 @@ extern "C" {
  * entries (64 B each for Connect Four, 256 B for Breakthrough), at most 30; 0 = default: 2^AZ_EVAL_CACHE_EXTRA_LOG2 entries
  * per simulation of one search of every tree (n_trees * n_playouts, rounded up to a power of two), within 2^16..2^27.
  * az_config_get reports the size in use. */
+#define AZ_F_RESIGN         (1u << 13) /* resignation (AlphaGo Zero; an extension: the reference plays every game to its end).
+                                          At a searched root the mover m = ply & 1 has r = max(-root_q, v_a0c) (the values of
+                                          the ply record; v_a0c = -99 when no child was visited).  A game resigns at the first
+                                          searched position with r < threshold (strict; threshold <= -1 never fires): the ply
+                                          record is emitted with action -1, then the kind-1 record (end = 1) with the resign
+                                          position and returns()[0] = -1 if player 0 resigned, else +1; no move is counted and
+                                          the game ends like a terminal one.  A no-resign calibration game (counter stream 6,
+                                          decided at its first searched position) never resigns and keeps each player's
+                                          minimum r.  Threshold and permille: az_set_resign.  Not with AZ_F_MANUAL */
 #define AZ_EVAL_CACHE_LOG2_SHIFT 24
 #define AZ_EVAL_CACHE_LOG2(flags) (((flags) >> AZ_EVAL_CACHE_LOG2_SHIFT) & 31u)
 #define AZ_EVAL_CACHE_EXTRA_LOG2 1
@@ -147,11 +157,13 @@ typedef struct az_engine az_engine;
 typedef struct az_record {
   int32_t tree, game_seq, ply, action; /* action chosen at this ply (-1 in manual mode) */
   int32_t n_legal, kind;               /* kind 0 = ply, 1 = game end */
-  int32_t root_n, pad;
-  uint64_t bb[2];                      /* position the search ran on (kind 1: final position) */
+  int32_t root_n;
+  int32_t end;                         /* kind 1: 0 = terminal position, 1 = resigned, 2 = calibration game (AZ_F_RESIGN)
+                                          that reached a terminal position; kind 0: 0 */
+  uint64_t bb[2];                      /* position the search ran on (kind 1: final or resign position) */
   double root_q;                       /* soft-Z target is -root_q (game_utils.py:174); kind 1: returns()[0] */
-  double v_a0c;                        /* game_utils.py:178 */
-  double v_offpolicy;                  /* game_utils.py:183-194 (AZ_F_OFFPOLICY) */
+  double v_a0c;                        /* game_utils.py:178; kind 1 with end 2: player 0's minimum r (2.0: never moved) */
+  double v_offpolicy;                  /* game_utils.py:183-194 (AZ_F_OFFPOLICY); kind 1 with end 2: player 1's minimum r */
   /* followed by int32 counts[max_children]: root child visits in legal (ascending action) order,
    * then int16 actions[max_children]: the action id of each child (-1 beyond n_legal) */
 } az_record;
@@ -172,6 +184,10 @@ enum {
   AZ_CTR_IDLE_SLOTS,      /* evaluator rows wasted (no request from that tree this step) */
   AZ_CTR_PEAK_NODES,      /* high-water mark of nodes in use in one tree's arena half (size node_capacity from it) */
   AZ_CTR_CACHE_HITS,      /* leaf expansions served from the AZ_F_EVAL_CACHE table (no evaluator row) */
+  AZ_CTR_RESIGNS,         /* AZ_F_RESIGN: games that ended by resignation */
+  AZ_CTR_RESIGN_SAMPLES,  /* AZ_F_RESIGN: no-resign calibration games finished */
+  AZ_CTR_RESIGN_FALSE,    /* AZ_F_RESIGN: players of finished calibration games whose minimum r was below the threshold in
+                             force at the game's end and who did not lose (would-be false resignations) */
   AZ_CTR_COUNT
 };
 
@@ -219,6 +235,13 @@ int az_step(az_engine* e, const void* priors_dev, const void* values_dev, const 
  * next were computed before the change and are still stored under the old weights; from that az_step on, entries of the
  * old weights no longer match. */
 int az_eval_cache_invalidate(az_engine* e, void* stream);
+
+/* AZ_F_RESIGN: resign threshold and the share of no-resign calibration games, in per mille (0..1000).  A stream-ordered write
+ * to device memory that the step kernels read there, so a captured CUDA graph of az_step sees the new values on its next
+ * replay.  After az_create: threshold -1.0 (never resigns), permille 0.  A game's calibration status is drawn with the
+ * permille in force at its first searched position.  Rejects a non-finite threshold, a permille outside [0, 1000] and an
+ * engine created without AZ_F_RESIGN. */
+int az_set_resign(az_engine* e, double threshold, int32_t disabled_permille, void* stream);
 
 /* Re-root compaction (MCTS.update_root, mcts.py:192-203) of the trees that played a move in the last az_step: BFS-copies
  * the kept subtree into the other arena half, one warp per tree.  az_step runs it first by itself unless
