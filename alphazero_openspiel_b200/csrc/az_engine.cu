@@ -6,7 +6,7 @@
 //   Node.update_recursive  mcts.py:82-89           -> backup_path()
 //   MCTS.playout/search    mcts.py:126-180         -> k_step main loop
 //   expand_root_dirichlet  mcts.py:182-190         -> expand_root()
-//   MCTS.update_root       mcts.py:192-203         -> reroot_compact()
+//   MCTS.update_root       mcts.py:192-203         -> finish_move() / k_command + k_compact
 //   AlphaZeroBot.step      alphazerobot.py:42-93   -> finish_move()
 //   play_game_self targets game_utils.py:168-204   -> emit_record()
 //   state_to_board         network.py:9-18         -> write_obs()
@@ -62,6 +62,34 @@ struct __align__(16) TreeHdr {
   int32_t pad2[3];
 };
 static_assert(sizeof(TreeHdr) == 80, "TreeHdr size");
+
+__device__ __forceinline__ St root_state(const TreeHdr& h) {
+  St s;
+  s.b0 = h.root_b0;
+  s.b1 = h.root_b1;
+  s.ply = h.root_ply;
+  return s;
+}
+__device__ __forceinline__ St pend_state(const TreeHdr& h) {
+  St s;
+  s.b0 = h.pend_b0;
+  s.b1 = h.pend_b1;
+  s.ply = h.pend_ply;
+  return s;
+}
+__device__ __forceinline__ void set_root(TreeHdr& h, const St& s) {
+  h.root_b0 = s.b0;
+  h.root_b1 = s.b1;
+  h.root_ply = s.ply;
+}
+// the evaluator request of node `node` at depth `depth` of the tree, at position s
+__device__ __forceinline__ void set_pend(TreeHdr& h, const St& s, int node, int depth) {
+  h.pend_b0 = s.b0;
+  h.pend_b1 = s.b1;
+  h.pend_ply = s.ply;
+  h.pend_node = node;
+  h.pend_depth = depth;
+}
 
 // one in-flight evaluator request of a tree in virtual-loss mode (AZ_F_VIRTUAL_LOSS)
 struct __align__(16) VlPend {
@@ -171,6 +199,35 @@ __device__ __forceinline__ void gargmax(unsigned m, double& v, int& i) {
 
 __device__ __forceinline__ void ctr_add(unsigned long long* s_ctr, int which, unsigned long long v) {
   if (v) atomicAdd(&s_ctr[which], v);
+}
+
+// the counters one tree accumulates in registers during a step kernel; flush (lane 0) adds them to the block's
+struct StepCtr {
+  unsigned long long sims = 0, depth = 0, children = 0, exp = 0, legal = 0, term = 0;
+  __device__ __forceinline__ void flush(unsigned long long* s_ctr, int alloc) const {
+    atomicMax(&s_ctr[AZ_CTR_PEAK_NODES], (unsigned long long)alloc);
+    ctr_add(s_ctr, AZ_CTR_SIMS, sims);
+    ctr_add(s_ctr, AZ_CTR_DEPTH, depth);
+    ctr_add(s_ctr, AZ_CTR_CHILDREN, children);
+    ctr_add(s_ctr, AZ_CTR_EXPANSIONS, exp);
+    ctr_add(s_ctr, AZ_CTR_LEGAL, legal);
+    ctr_add(s_ctr, AZ_CTR_TERMINAL, term);
+  }
+};
+
+// the block's counters into the engine's, once every thread of the block is done with s_ctr
+__device__ __forceinline__ void flush_block_counters(const Params& p, const unsigned long long* s_ctr) {
+  __syncthreads();
+  if (threadIdx.x < AZ_CTR_COUNT && s_ctr[threadIdx.x]) {
+    if (threadIdx.x == AZ_CTR_PEAK_NODES) atomicMax(&p.ctr[threadIdx.x], s_ctr[threadIdx.x]);
+    else atomicAdd(&p.ctr[threadIdx.x], s_ctr[threadIdx.x]);
+  }
+}
+
+// expand_node found no room for the children in the arena half: flag the tree and count the overflow
+__device__ __forceinline__ void arena_overflow(TreeHdr& h, int lane, unsigned long long* s_ctr) {
+  h.err = 1;
+  if (lane == 0) ctr_add(s_ctr, AZ_CTR_OVERFLOW, 1);
 }
 
 // ---------------------------------------------------------------- evaluator inputs
@@ -468,49 +525,6 @@ __device__ double offpolicy_value(const Arena& a, int root, int lane, unsigned g
   return value * mult;
 }
 
-// MCTS.update_root (mcts.py:192-203) + compaction: BFS-copy the subtree of `child` into the other arena half.
-template <class GM, int G>
-__device__ void reroot_compact(const Params& p, TreeHdr& h, int tree, int child, int lane, unsigned gm,
-                               unsigned long long& copied) {
-  const Arena src = arena_of(p, tree, h.half);
-  const Arena dst = arena_of(p, tree, h.half ^ 1);
-  if (lane == 0) {
-    dst.nl(0) = src.nl(child);
-    dst.q(0) = src.q(child);
-    dst.p(0) = src.p(child);
-  }
-  __syncwarp(gm);
-  int head = 0, tail = 1;
-  while (head < tail) {
-    const int nb = min(G, tail - head);
-    const int idx = head + lane;
-    int mync = 0, oldfc = 0;
-    if (lane < nb) {
-      const uint2 nl = dst.nl(idx);
-      mync = (int)(nl.y & 0xffu);
-      oldfc = (int)(nl.y >> 8);
-    }
-    const int incl = gscan_incl<G>(gm, mync, lane);
-    const int total = gshfl<G>(gm, incl, G - 1);
-    if (mync > 0) {
-      const int newfc = tail + incl - mync;
-      dst.nl(idx).y = ((unsigned)newfc << 8) | (unsigned)mync;
-      for (int j = 0; j < mync; ++j) {
-        dst.nl(newfc + j) = src.nl(oldfc + j);
-        dst.q(newfc + j) = src.q(oldfc + j);
-        dst.p(newfc + j) = src.p(oldfc + j);
-      }
-    }
-    __syncwarp(gm);
-    tail += total;
-    head += nb;
-  }
-  copied += (unsigned long long)tail;
-  h.half ^= 1;
-  h.root_node = 0;
-  h.alloc = tail;
-}
-
 template <int G>
 // uct_root: the reference keeps use_puct on every Node, children inherit it from their parent (mcts.py:64), and only the root
 // that update_root creates for a leaf root (mcts.py:199-200) gets the MCTS object's flag -- the root of MCTS.__init__
@@ -605,16 +619,11 @@ __device__ void end_game(const Params& p, TreeHdr& h, int tree, int lane, unsign
   }
   if (restart) {
     h.game_seq += 1;
-    const St s0 = start_position<GM>(p, tree, h.game_seq);
-    h.root_b0 = s0.b0;
-    h.root_b1 = s0.b1;
-    h.root_ply = s0.ply;
+    set_root(h, start_position<GM>(p, tree, h.game_seq));
     fresh_tree<G>(p, h, tree, lane, gm);
     h.phase = PH_BEGIN;
   } else {
-    h.root_b0 = s_end.b0;
-    h.root_b1 = s_end.b1;
-    h.root_ply = s_end.ply;
+    set_root(h, s_end);
     h.phase = AZ_PH_IDLE;
   }
 }
@@ -670,10 +679,7 @@ __device__ int resign_game_over(const Params& p, int tree, int lane, unsigned gm
 template <class GM, int G>
 __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, unsigned gm, unsigned long long* s_ctr) {
   const Arena a = arena_of(p, tree, h.half);
-  St s;
-  s.b0 = h.root_b0;
-  s.b1 = h.root_b1;
-  s.ply = h.root_ply;
+  const St s = root_state(h);
   const typename GM::Legal lg = GM::legal(s, p.geo);
   const int L = GM::count(lg);
   const uint2 rnl = a.nl(h.root_node);
@@ -789,9 +795,7 @@ __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, uns
     end_game<GM, G>(p, h, tree, lane, gm, s_ctr, s2);
     return;
   }
-  h.root_b0 = s2.b0;
-  h.root_b1 = s2.b1;
-  h.root_ply = s2.ply;
+  set_root(h, s2);
   if ((p.flags & AZ_F_KEEP_TREE) && nc > 0) {
     // MCTS.update_root (mcts.py:192-203).  While the arena half still has room for the worst case of one more search
     // (every simulation expands one leaf), the chosen child simply becomes the root in place and the discarded siblings
@@ -812,16 +816,13 @@ __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, uns
   h.phase = PH_BEGIN;
 }
 
-// expand_root_dirichlet (mcts.py:182-190): the root expansion with the noise mix, from the evaluator row (cached == nullptr)
-// or from an AZ_F_EVAL_CACHE entry's priors.  Leaves the tree in AZ_PH_RUN.
+// expand_root_dirichlet (mcts.py:182-190): the root expansion with the noise mix, from evaluator row `row` (cached == nullptr)
+// or from an AZ_F_EVAL_CACHE entry's priors.  The noise is the tree's.  Leaves the tree in AZ_PH_RUN.
 template <class GM, int G>
-__device__ __forceinline__ void expand_root(const Params& p, const StepIO& io, TreeHdr& h, int tree, int lane, unsigned gm,
-                                          unsigned long long* s_ctr, const float* cached) {
+__device__ __forceinline__ void expand_root(const Params& p, const StepIO& io, TreeHdr& h, int tree, int row, int lane,
+                                            unsigned gm, unsigned long long* s_ctr, const float* cached) {
   const Arena a = arena_of(p, tree, h.half);
-  St s;
-  s.b0 = h.root_b0;
-  s.b1 = h.root_b1;
-  s.ply = h.root_ply;
+  const St s = root_state(h);
   const typename GM::Legal lg = GM::legal(s, p.geo);
   const int L = GM::count(lg);
   double eta[GM::SLOTS];
@@ -839,7 +840,9 @@ __device__ __forceinline__ void expand_root(const Params& p, const StepIO& io, T
       const double u = (double)((counter(p.seed, tree, h.game_seq, s.ply, i, 1) >> 11) + 1ULL) *
                        (1.0 / 9007199254740992.0);
       sum = __dadd_rn(sum, u);
-      if (i % G == lane) eta[i / G] = u;
+#pragma unroll
+      for (int sl = 0; sl < GM::SLOTS; ++sl)
+        if (i == lane + sl * G) eta[sl] = u;
     }
 #pragma unroll
     for (int sl = 0; sl < GM::SLOTS; ++sl) eta[sl] = __ddiv_rn(eta[sl], sum);
@@ -856,13 +859,64 @@ __device__ __forceinline__ void expand_root(const Params& p, const StepIO& io, T
     for (int sl = 0; sl < GM::SLOTS; ++sl) eta[sl] = sum > 0.0 ? eta[sl] / sum : 1.0 / (double)L;
   }
   int L2 = 0;
-  const bool ok = expand_node<GM, G>(p, io, a, h, tree, h.root_node, s, lane, gm, true, eta, &L2, cached);
-  if (!ok) {
-    h.err = 1;
-    if (lane == 0) ctr_add(s_ctr, AZ_CTR_OVERFLOW, 1);
-  }
+  if (!expand_node<GM, G>(p, io, a, h, row, h.root_node, s, lane, gm, true, eta, &L2, cached)) arena_overflow(h, lane, s_ctr);
   h.phase = AZ_PH_RUN;
   if (lane == 0) ctr_add(s_ctr, AZ_CTR_ROOT_EVALS, 1);
+}
+
+// ---------------------------------------------------------------- search operations of both step kernels
+// MCTS.search (mcts.py:173-176) from PH_BEGIN.  Without root noise the simulations start at once (AZ_PH_RUN).  With it the root
+// is expanded first: from an AZ_F_EVAL_CACHE hit, or through a root request to evaluator row `row` -- then the tree waits in
+// AZ_PH_ROOT_EVAL and this returns true.  CACHE: the kernel looks up the cache (k_step_vl runs without one).
+template <class GM, int G, bool CACHE>
+__device__ __forceinline__ bool begin_search(const Params& p, const StepIO& io, TreeHdr& h, int tree, int row, int lane,
+                                             unsigned gm, unsigned long long* s_ctr) {
+  h.sims_done = 0;
+  h.phase = AZ_PH_RUN;
+  if (p.noise_mode == AZ_NOISE_NONE) return false;
+  const St s = root_state(h);
+  const CacheHead* hit = CACHE && p.cache ? cache_find<GM>(p, s) : nullptr;
+  if (hit) {
+    expand_root<GM, G>(p, io, h, tree, row, lane, gm, s_ctr, cache_priors(hit));
+    return false;
+  }
+  h.phase = AZ_PH_ROOT_EVAL;
+  set_pend(h, s, h.root_node, 0);
+  write_obs<GM, G>(p, io, row, lane, s);
+  return true;
+}
+
+// Node.expand + node.update_recursive(-leaf_value) (mcts.py:146-152) of the non-terminal leaf `node` at position s, from
+// evaluator row `row` or (cached != nullptr) from the AZ_F_EVAL_CACHE entry that holds the same values.  BACKUP is backup_path,
+// or vl_backup for a path that carries a virtual loss.
+template <class GM, int G, void (*BACKUP)(const Arena&, const int32_t*, int, double, int)>
+__device__ __forceinline__ void apply_leaf(const Params& p, const StepIO& io, const Arena& a, TreeHdr& h, int row, int node,
+                                           const St& s, const int32_t* path, int depth, const CacheHead* cached, int lane,
+                                           unsigned gm, unsigned long long* s_ctr, StepCtr& c) {
+  int L = 0;
+  if (!expand_node<GM, G>(p, io, a, h, row, node, s, lane, gm, false, nullptr, &L, cached ? cache_priors(cached) : nullptr))
+    arena_overflow(h, lane, s_ctr);
+  const double v = cached ? (double)cached->value : eval_value<GM>(p, io, row, eval_key(p, s), s);
+  BACKUP(a, path, depth, -v, lane);
+  __syncwarp(gm);
+  h.sims_done += 1;
+  c.sims += 1;
+  c.depth += depth;
+  c.exp += 1;
+  c.legal += L;
+  if (cached && lane == 0) ctr_add(s_ctr, AZ_CTR_CACHE_HITS, 1);
+}
+
+// terminal leaf: leaf_value = -player_return(mover); node.update_recursive(-leaf_value)   mcts.py:148-152
+template <int G>
+__device__ __forceinline__ void terminal_leaf(const Arena& a, TreeHdr& h, const int32_t* path, int depth, int out, int ply,
+                                              int lane, unsigned gm, StepCtr& c) {
+  backup_path<G>(a, path, depth, mover_return(out, ply), lane);
+  __syncwarp(gm);
+  h.sims_done += 1;
+  c.sims += 1;
+  c.depth += depth;
+  c.term += 1;
 }
 
 // ---------------------------------------------------------------- the step kernel
@@ -886,33 +940,15 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
     TreeHdr h = p.hdr[tree];
     const int phase_in = h.phase;
     long long t_consume = 0;
-    unsigned long long c_sims = 0, c_depth = 0, c_children = 0, c_exp = 0, c_legal = 0, c_term = 0;
+    StepCtr c;
 
     // ---------------- 1. consume the evaluator outputs of the pending request
     if (h.phase == AZ_PH_LEAF_EVAL) {
-      const Arena a = arena_of(p, tree, h.half);
-      St s;
-      s.b0 = h.pend_b0;
-      s.b1 = h.pend_b1;
-      s.ply = h.pend_ply;
-      int L = 0;
-      const bool ok = expand_node<GM, G>(p, io, a, h, tree, h.pend_node, s, lane, gm, false, nullptr, &L);
-      if (!ok) {
-        h.err = 1;
-        if (lane == 0) ctr_add(s_ctr, AZ_CTR_OVERFLOW, 1);
-      }
-      const double v = eval_value<GM>(p, io, tree, eval_key(p, s), s);
-      // node.update_recursive(-leaf_value)   mcts.py:152
-      backup_path<G>(a, gpath, h.pend_depth, -v, lane);
-      __syncwarp(gm);
-      h.sims_done += 1;
+      apply_leaf<GM, G, backup_path<G>>(p, io, arena_of(p, tree, h.half), h, tree, h.pend_node, pend_state(h), gpath,
+                                        h.pend_depth, nullptr, lane, gm, s_ctr, c);
       h.phase = AZ_PH_RUN;
-      c_sims += 1;
-      c_depth += h.pend_depth;
-      c_exp += 1;
-      c_legal += L;
     } else if (h.phase == AZ_PH_ROOT_EVAL) {
-      expand_root<GM, G>(p, io, h, tree, lane, gm, s_ctr, nullptr);
+      expand_root<GM, G>(p, io, h, tree, tree, lane, gm, s_ctr, nullptr);
     }
 
     if (p.dbg) t_consume = clock64() - t_start;
@@ -920,29 +956,7 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
     int sims_this_step = 0;
     bool advanced = false;
     for (;;) {
-      if (h.phase == PH_BEGIN) {
-        h.sims_done = 0;
-        if (p.noise_mode != AZ_NOISE_NONE) {
-          St s;
-          s.b0 = h.root_b0;
-          s.b1 = h.root_b1;
-          s.ply = h.root_ply;
-          const CacheHead* hit = p.cache ? cache_find<GM>(p, s) : nullptr;
-          if (hit) {
-            expand_root<GM, G>(p, io, h, tree, lane, gm, s_ctr, cache_priors(hit));
-          } else {
-            h.phase = AZ_PH_ROOT_EVAL;
-            h.pend_b0 = s.b0;
-            h.pend_b1 = s.b1;
-            h.pend_ply = s.ply;
-            h.pend_depth = 0;
-            h.pend_node = h.root_node;
-            write_obs<GM, G>(p, io, tree, lane, s);
-            break;
-          }
-        }
-        h.phase = AZ_PH_RUN;
-      }
+      if (h.phase == PH_BEGIN && begin_search<GM, G, true>(p, io, h, tree, tree, lane, gm, s_ctr)) break;
       if (h.phase != AZ_PH_RUN) {
         if (lane == 0) ctr_add(s_ctr, AZ_CTR_IDLE_SLOTS, 1);
         break;
@@ -972,13 +986,10 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
       }
       // ---- one simulation (mcts.py:126-153)
       const Arena a = arena_of(p, tree, h.half);
-      St s;
-      s.b0 = h.root_b0;
-      s.b1 = h.root_b1;
-      s.ply = h.root_ply;
+      St s = root_state(h);
       int node, depth;
       bool dovf = false;
-      sim_select<GM, G, UCT>(p, a, h.root_node, s, node, depth, spath, lane, gm, c_children, dovf, h.uct != 0);
+      sim_select<GM, G, UCT>(p, a, h.root_node, s, node, depth, spath, lane, gm, c.children, dovf, h.uct != 0);
       if (dovf) {
         h.err = 1;
         h.phase = AZ_PH_ERROR;
@@ -988,45 +999,21 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
       const int out = depth > 0 ? GM::outcome(s, p.geo) : -1;
       ++sims_this_step;
       if (out >= 0) {
-        // terminal leaf: leaf_value = -player_return(mover); update_recursive(-leaf_value)   mcts.py:148-152
-        backup_path<G>(a, spath, depth, mover_return(out, s.ply), lane);
-        __syncwarp(gm);
+        terminal_leaf<G>(a, h, spath, depth, out, s.ply, lane, gm, c);
         if (p.flags & AZ_F_MANUAL) {  // MCTS.playout(state) leaves `state` at the leaf: keep the path for az_request_info
           for (int j = lane; j <= depth; j += G) gpath[j] = spath[j];
           h.pend_depth = depth;
         }
-        h.sims_done += 1;
-        c_sims += 1;
-        c_depth += depth;
-        c_term += 1;
         continue;
       }
       // non-terminal leaf: its evaluation from the cache, exactly as the AZ_PH_LEAF_EVAL consume path would apply the row
-      if (p.cache) {
-        const CacheHead* hit = cache_find<GM>(p, s);
-        if (hit) {
-          int L = 0;
-          if (!expand_node<GM, G>(p, io, a, h, tree, node, s, lane, gm, false, nullptr, &L, cache_priors(hit))) {
-            h.err = 1;
-            if (lane == 0) ctr_add(s_ctr, AZ_CTR_OVERFLOW, 1);
-          }
-          backup_path<G>(a, spath, depth, -(double)hit->value, lane);
-          __syncwarp(gm);
-          h.sims_done += 1;
-          c_sims += 1;
-          c_depth += depth;
-          c_exp += 1;
-          c_legal += L;
-          if (lane == 0) ctr_add(s_ctr, AZ_CTR_CACHE_HITS, 1);
-          continue;
-        }
+      const CacheHead* hit = p.cache ? cache_find<GM>(p, s) : nullptr;
+      if (hit) {
+        apply_leaf<GM, G, backup_path<G>>(p, io, a, h, tree, node, s, spath, depth, hit, lane, gm, s_ctr, c);
+        continue;
       }
       // otherwise request the evaluator (mcts.py:146)
-      h.pend_b0 = s.b0;
-      h.pend_b1 = s.b1;
-      h.pend_ply = s.ply;
-      h.pend_node = node;
-      h.pend_depth = depth;
+      set_pend(h, s, node, depth);
       h.phase = AZ_PH_LEAF_EVAL;
       for (int j = lane; j <= depth; j += G) gpath[j] = spath[j];
       write_obs<GM, G>(p, io, tree, lane, s);
@@ -1041,20 +1028,10 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
         p.dbg[4 * tree + 2] = sims_this_step;
         p.dbg[4 * tree + 3] = t_consume * 2 + (advanced ? 1 : 0);
       }
-      atomicMax(&s_ctr[AZ_CTR_PEAK_NODES], (unsigned long long)h.alloc);
-      ctr_add(s_ctr, AZ_CTR_SIMS, c_sims);
-      ctr_add(s_ctr, AZ_CTR_DEPTH, c_depth);
-      ctr_add(s_ctr, AZ_CTR_CHILDREN, c_children);
-      ctr_add(s_ctr, AZ_CTR_EXPANSIONS, c_exp);
-      ctr_add(s_ctr, AZ_CTR_LEGAL, c_legal);
-      ctr_add(s_ctr, AZ_CTR_TERMINAL, c_term);
+      c.flush(s_ctr, h.alloc);
     }
   }
-  __syncthreads();
-  if (threadIdx.x < AZ_CTR_COUNT && s_ctr[threadIdx.x]) {
-    if (threadIdx.x == AZ_CTR_PEAK_NODES) atomicMax(&p.ctr[threadIdx.x], s_ctr[threadIdx.x]);
-    else atomicAdd(&p.ctr[threadIdx.x], s_ctr[threadIdx.x]);
-  }
+  flush_block_counters(p, s_ctr);
 }
 
 // ---------------------------------------------------------------- evaluator cache insertion (AZ_F_EVAL_CACHE)
@@ -1070,10 +1047,7 @@ __global__ void __launch_bounds__(BLOCK) k_cache_insert(const Params p, const St
   const TreeHdr& h = p.hdr[tree];
   if (h.phase != AZ_PH_LEAF_EVAL && h.phase != AZ_PH_ROOT_EVAL) return;
   const unsigned gm = group_mask<G>();
-  St s;
-  s.b0 = h.pend_b0;
-  s.b1 = h.pend_b1;
-  s.ply = h.pend_ply;
+  const St s = pend_state(h);
   uint8_t* slot = cache_slot<GM>(p, s);
   unsigned* lock = reinterpret_cast<unsigned*>(slot + cache_stride<GM>() - 4);
   int got = 0;
@@ -1110,8 +1084,9 @@ __global__ void k_cache_new_epoch(uint32_t* epoch) { epoch[0] += 1u; }
 // NOT bit-exact with the reference: while a leaf is in flight every node on its path carries one extra visit with value -1
 // (Q <- (N*Q - 1)/(N + 1), N <- N + 1), which steers the following descents of the same step elsewhere; the real backup
 // replaces that visit (Q <- (N*Q + 1 + v)/N).  A leaf that is already in flight ends the collection for this step (its
-// link carries the marker 0xFFFFFF00).  Everything else -- PUCT arithmetic, expansion, terminal leaves, root noise, move
-// choice, records, re-rooting -- is the code of the exact kernel.  K = 1 through this kernel is still not the exact path.
+// link carries the marker 0xFFFFFF00).  Everything else is the exact kernel's code: sim_select, begin_search, expand_root
+// (root noise), apply_leaf (with vl_backup), terminal_leaf and finish_move (move choice, records, re-rooting).  K = 1
+// through this kernel is still not the exact path.
 constexpr unsigned VL_MARK = 0xFFFFFF00u;
 
 template <int G>
@@ -1151,7 +1126,7 @@ __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const Step
     VlPend* pend = p.vl_pend + (size_t)tree * K;
     const int row0 = tree * K;
     TreeHdr h = p.hdr[tree];
-    unsigned long long c_sims = 0, c_depth = 0, c_children = 0, c_exp = 0, c_legal = 0, c_term = 0;
+    StepCtr c;
 
     // ---------------- 1. consume the evaluator rows of the requests in flight
     if (h.phase == AZ_PH_LEAF_EVAL) {
@@ -1165,75 +1140,22 @@ __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const Step
         s.ply = pe.ply;
         if (lane == 0) a.nl(pe.node).y = 0u;   // drop the in-flight marker: expand_node sees a childless node
         __syncwarp(gm);
-        int L = 0;
-        const bool ok = expand_node<GM, G>(p, io, a, h, row0 + slot, pe.node, s, lane, gm, false, nullptr, &L);
-        if (!ok) {
-          h.err = 1;
-          if (lane == 0) ctr_add(s_ctr, AZ_CTR_OVERFLOW, 1);
-        }
-        const double v = eval_value<GM>(p, io, row0 + slot, eval_key(p, s), s);
-        vl_backup<G>(a, gpaths + (size_t)slot * GM::MAXD, pe.depth, -v, lane);
-        __syncwarp(gm);
+        apply_leaf<GM, G, vl_backup<G>>(p, io, a, h, row0 + slot, pe.node, s, gpaths + (size_t)slot * GM::MAXD, pe.depth,
+                                        nullptr, lane, gm, s_ctr, c);
         if (lane == 0) pend[slot].valid = 0;
-        h.sims_done += 1;
-        c_sims += 1;
-        c_depth += pe.depth;
-        c_exp += 1;
-        c_legal += L;
       }
       h.phase = AZ_PH_RUN;
     } else if (h.phase == AZ_PH_ROOT_EVAL) {
-      const Arena a = arena_of(p, tree, h.half);
-      St s;
-      s.b0 = h.root_b0;
-      s.b1 = h.root_b1;
-      s.ply = h.root_ply;
-      const typename GM::Legal lg = GM::legal(s, p.geo);
-      const int L = GM::count(lg);
-      double eta[GM::SLOTS];
-      double sum = 0.0;
-#pragma unroll
-      for (int sl = 0; sl < GM::SLOTS; ++sl) {
-        const int i = lane + sl * G;
-        eta[sl] = 0.0;
-        if (p.noise_mode == AZ_NOISE_DIRICHLET && i < L) eta[sl] = gamma_draw(p.alpha, p.seed, tree, h.game_seq, s.ply, i);
-        else if (p.noise_mode == AZ_NOISE_HOST && i < L) eta[sl] = io.noise[(size_t)tree * GM::MAXC + i];
-        else if (p.noise_mode == AZ_NOISE_COUNTER && i < L)
-          eta[sl] = (double)((counter(p.seed, tree, h.game_seq, s.ply, i, 1) >> 11) + 1ULL) * (1.0 / 9007199254740992.0);
-        sum += eta[sl];
-      }
-      if (p.noise_mode != AZ_NOISE_HOST) {
-        sum = gsumd<G>(gm, sum);
-#pragma unroll
-        for (int sl = 0; sl < GM::SLOTS; ++sl) eta[sl] = sum > 0.0 ? eta[sl] / sum : 1.0 / (double)L;
-      }
-      int L2 = 0;
-      const bool ok = expand_node<GM, G>(p, io, a, h, row0, h.root_node, s, lane, gm, true, eta, &L2);
-      if (!ok) {
-        h.err = 1;
-        if (lane == 0) ctr_add(s_ctr, AZ_CTR_OVERFLOW, 1);
-      }
-      h.phase = AZ_PH_RUN;
-      if (lane == 0) ctr_add(s_ctr, AZ_CTR_ROOT_EVALS, 1);
+      expand_root<GM, G>(p, io, h, tree, row0, lane, gm, s_ctr, nullptr);
     }
 
     // ---------------- 2. collect up to K new leaves
     int n_pending = 0, sims_this_step = 0;
     bool advanced = false;
     for (;;) {
-      if (h.phase == PH_BEGIN) {
-        h.sims_done = 0;
-        if (p.noise_mode != AZ_NOISE_NONE) {
-          St s;
-          s.b0 = h.root_b0;
-          s.b1 = h.root_b1;
-          s.ply = h.root_ply;
-          h.phase = AZ_PH_ROOT_EVAL;
-          write_obs<GM, G>(p, io, row0, lane, s);
-          n_pending = 1;   // (one evaluator row in use; not a leaf request)
-          break;
-        }
-        h.phase = AZ_PH_RUN;
+      if (h.phase == PH_BEGIN && begin_search<GM, G, false>(p, io, h, tree, row0, lane, gm, s_ctr)) {
+        n_pending = 1;   // (one evaluator row in use; not a leaf request)
+        break;
       }
       if (h.phase != AZ_PH_RUN) break;
       if (h.sims_done + n_pending >= p.n_playouts) {
@@ -1245,13 +1167,10 @@ __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const Step
       if (n_pending >= K) break;
       if (p.max_sims > 0 && sims_this_step >= p.max_sims + K) break;
       const Arena a = arena_of(p, tree, h.half);
-      St s;
-      s.b0 = h.root_b0;
-      s.b1 = h.root_b1;
-      s.ply = h.root_ply;
+      St s = root_state(h);
       int node, depth;
       bool dovf = false;
-      sim_select<GM, G, false>(p, a, h.root_node, s, node, depth, spath, lane, gm, c_children, dovf, false);
+      sim_select<GM, G, false>(p, a, h.root_node, s, node, depth, spath, lane, gm, c.children, dovf, false);
       if (dovf) {
         h.err = 1;
         h.phase = AZ_PH_ERROR;
@@ -1261,12 +1180,7 @@ __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const Step
       const int out = depth > 0 ? GM::outcome(s, p.geo) : -1;
       ++sims_this_step;
       if (out >= 0) {   // terminal leaf: real backup at once, no virtual loss needed
-        backup_path<G>(a, spath, depth, mover_return(out, s.ply), lane);
-        __syncwarp(gm);
-        h.sims_done += 1;
-        c_sims += 1;
-        c_depth += depth;
-        c_term += 1;
+        terminal_leaf<G>(a, h, spath, depth, out, s.ply, lane, gm, c);
         continue;
       }
       if (a.nl(node).y == VL_MARK) break;   // this leaf is already in flight: stop collecting for this step
@@ -1293,26 +1207,17 @@ __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const Step
     if (lane == 0) {
       p.hdr[tree] = h;
       ctr_add(s_ctr, AZ_CTR_IDLE_SLOTS, (unsigned long long)(K - n_pending));
-      atomicMax(&s_ctr[AZ_CTR_PEAK_NODES], (unsigned long long)h.alloc);
-      ctr_add(s_ctr, AZ_CTR_SIMS, c_sims);
-      ctr_add(s_ctr, AZ_CTR_DEPTH, c_depth);
-      ctr_add(s_ctr, AZ_CTR_CHILDREN, c_children);
-      ctr_add(s_ctr, AZ_CTR_EXPANSIONS, c_exp);
-      ctr_add(s_ctr, AZ_CTR_LEGAL, c_legal);
-      ctr_add(s_ctr, AZ_CTR_TERMINAL, c_term);
+      c.flush(s_ctr, h.alloc);
     }
   }
-  __syncthreads();
-  if (threadIdx.x < AZ_CTR_COUNT && s_ctr[threadIdx.x]) {
-    if (threadIdx.x == AZ_CTR_PEAK_NODES) atomicMax(&p.ctr[threadIdx.x], s_ctr[threadIdx.x]);
-    else atomicAdd(&p.ctr[threadIdx.x], s_ctr[threadIdx.x]);
-  }
+  flush_block_counters(p, s_ctr);
 }
 
 // ---------------------------------------------------------------- re-root compaction, one CTA per moving tree
-// MCTS.update_root (mcts.py:192-203) for the trees queued by finish_move.  Runs on its own stream next to the evaluator.
-// Same BFS copy as reroot_compact (the new arena is its own queue) but 256 queue nodes per iteration: the copy is a chain
-// of dependent global loads, so its duration is the number of iterations, not the number of nodes.
+// MCTS.update_root (mcts.py:192-203): BFS copy of the subtree of h.pend_node into the other arena half, for the trees queued
+// by finish_move (they wait in PH_COMPACT and go on to their next search) and by k_command's update_root (they keep the phase
+// k_command gave them).  The new arena is its own queue, 256 queue nodes per iteration: the copy is a chain of dependent
+// global loads, so its duration is the number of iterations, not the number of nodes.
 constexpr int COMPACT_BLOCK = 256;
 __global__ void __launch_bounds__(COMPACT_BLOCK) k_compact(const Params p) {
   __shared__ int s_warp_sum[COMPACT_BLOCK / 32];
@@ -1368,7 +1273,7 @@ __global__ void __launch_bounds__(COMPACT_BLOCK) k_compact(const Params p) {
       h.half ^= 1;
       h.root_node = 0;
       h.alloc = tail;
-      h.phase = PH_BEGIN;
+      if (h.phase == PH_COMPACT) h.phase = PH_BEGIN;
       p.hdr[tree] = h;
       s_copied += (unsigned long long)tail;
     }
@@ -1396,10 +1301,7 @@ __global__ void k_reset(const Params p) {
   const unsigned gm = group_mask<G>();
   TreeHdr h;
   memset(&h, 0, sizeof(h));
-  const St s0 = start_position<GM>(p, tree, 0);
-  h.root_b0 = s0.b0;
-  h.root_b1 = s0.b1;
-  h.root_ply = s0.ply;
+  set_root(h, start_position<GM>(p, tree, 0));
   h.game_seq = 0;
   h.half = 0;
   fresh_tree<G>(p, h, tree, lane, gm);
@@ -1424,17 +1326,12 @@ __global__ void k_set_positions(const Params p, const int32_t* hist, const int32
     }
     s = GM::apply(s, p.geo, a);
   }
-  p.hdr[tree].root_b0 = s.b0;
-  p.hdr[tree].root_b1 = s.b1;
-  p.hdr[tree].root_ply = s.ply;
+  set_root(p.hdr[tree], s);
 }
 
 template <class GM>
 __global__ void k_command(const Params p, const int32_t* upd, const int32_t* rst, const int32_t* beg, int32_t* bad) {
   constexpr int G = GM::G;
-  __shared__ unsigned long long s_ctr[AZ_CTR_COUNT];
-  if (threadIdx.x < AZ_CTR_COUNT) s_ctr[threadIdx.x] = 0ULL;
-  __syncthreads();
   const int tree = (int)((blockIdx.x * (unsigned)blockDim.x + threadIdx.x) / G);
   const int lane = threadIdx.x % G;
   if (tree < p.n_trees) {
@@ -1450,10 +1347,7 @@ __global__ void k_command(const Params p, const int32_t* upd, const int32_t* rst
     if (upd && upd[tree] >= 0) {
       const int action = upd[tree];
       const Arena a = arena_of(p, tree, h.half);
-      St s;
-      s.b0 = h.root_b0;
-      s.b1 = h.root_b1;
-      s.ply = h.root_ply;
+      const St s = root_state(h);
       const typename GM::Legal lg = GM::legal(s, p.geo);
       const int k = GM::outcome(s, p.geo) >= 0 ? -1 : GM::rank_of(lg, s, p.geo, action);
       const uint2 rnl = a.nl(h.root_node);
@@ -1462,17 +1356,11 @@ __global__ void k_command(const Params p, const int32_t* upd, const int32_t* rst
         fresh_tree<G>(p, h, tree, lane, gm, (p.flags & AZ_F_UCT) != 0);
       } else if (k < 0) {
         if (lane == 0) atomicAdd(bad, 1);     // KeyError in the reference (mcts.py:202)
-      } else {
-        unsigned long long copied = 0;
-        reroot_compact<GM, G>(p, h, tree, (int)(rnl.y >> 8) + k, lane, gm, copied);
-        if (lane == 0) ctr_add(s_ctr, AZ_CTR_COMPACT_NODES, copied);
+      } else {  // the chosen child becomes the root: k_compact, launched right after this kernel, copies its subtree
+        h.pend_node = (int)(rnl.y >> 8) + k;
+        if (lane == 0) p.compact_list[atomicAdd(p.compact_count, 1)] = tree;
       }
-      if (k >= 0) {
-        const St s2 = GM::apply(s, p.geo, action);
-        h.root_b0 = s2.b0;
-        h.root_b1 = s2.b1;
-        h.root_ply = s2.ply;
-      }
+      if (k >= 0) set_root(h, GM::apply(s, p.geo, action));
       h.phase = AZ_PH_IDLE;
       dirty = true;
     }
@@ -1489,8 +1377,6 @@ __global__ void k_command(const Params p, const int32_t* upd, const int32_t* rst
     }
     if (dirty && lane == 0) p.hdr[tree] = h;
   }
-  __syncthreads();
-  if (threadIdx.x < AZ_CTR_COUNT && s_ctr[threadIdx.x]) atomicAdd(&p.ctr[threadIdx.x], s_ctr[threadIdx.x]);
 }
 
 template <class GM>
@@ -1504,11 +1390,7 @@ __global__ void k_status(const Params p, int32_t* phase, int32_t* sims, int32_t*
   if (req_legal) {
     int L = 0;
     if (h.phase == AZ_PH_LEAF_EVAL || h.phase == AZ_PH_ROOT_EVAL) {
-      St s;
-      s.b0 = h.pend_b0;
-      s.b1 = h.pend_b1;
-      s.ply = h.pend_ply;
-      L = GM::count(GM::legal(s, p.geo));
+      L = GM::count(GM::legal(pend_state(h), p.geo));
     }
     req_legal[tree] = L;
   }
@@ -1532,10 +1414,7 @@ __global__ void k_request_info(const Params p, uint64_t* bb, int32_t* ply, int32
   if (path_actions && depth > 0) {
     const Arena a = arena_of(p, tree, h.half);
     const int32_t* gpath = p.path + (size_t)tree * GM::MAXD;
-    St s;
-    s.b0 = h.root_b0;
-    s.b1 = h.root_b1;
-    s.ply = h.root_ply;
+    St s = root_state(h);
     for (int j = 0; j < depth && j < max_depth; ++j) {
       const int fc = (int)(a.nl(gpath[j]).y >> 8);
       const int k = gpath[j + 1] - fc;
@@ -1559,10 +1438,7 @@ __global__ void k_root_stats(const Params p, int32_t* root_n, double* root_q, in
   const Arena a = arena_of(p, tree, h.half);
   const uint2 rnl = a.nl(h.root_node);
   const int nc = (int)(rnl.y & 0xffu), fc = (int)(rnl.y >> 8);
-  St s;
-  s.b0 = h.root_b0;
-  s.b1 = h.root_b1;
-  s.ply = h.root_ply;
+  const St s = root_state(h);
   const typename GM::Legal lg = GM::legal(s, p.geo);
   if (lane == 0) {
     if (root_n) root_n[tree] = (int)rnl.x;
@@ -1602,10 +1478,7 @@ __global__ void k_positions(const Params p, uint64_t* bb, int32_t* ply, int32_t*
   const int tree = blockIdx.x * blockDim.x + threadIdx.x;
   if (tree >= p.n_trees) return;
   const TreeHdr h = p.hdr[tree];
-  St s;
-  s.b0 = h.root_b0;
-  s.b1 = h.root_b1;
-  s.ply = h.root_ply;
+  const St s = root_state(h);
   const int out = GM::outcome(s, p.geo);
   if (bb) {
     bb[2 * tree] = s.b0;
@@ -2042,6 +1915,7 @@ int az_command(az_engine* e, const int32_t* update_root_host, const int32_t* res
     k_command<GM><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p, d_upd, d_rst, d_beg, e->d_bad);
     return 0;
   });
+  if (d_upd) k_compact<<<compact_grid(p.n_trees), 256, 0, st>>>(p);  // re-root the trees k_command queued
   CK(cudaGetLastError());
   return check_bad(e, st, "az_command(update_root)");
 }
