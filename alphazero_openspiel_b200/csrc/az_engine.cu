@@ -59,7 +59,9 @@ struct __align__(16) TreeHdr {
   int32_t root_ply;
   int32_t game_seq;
   uint8_t phase, half, err, uct;  // uct: this tree scores with the use_puct=False formula (see fresh_tree)
-  int32_t pad2[3];
+  int32_t fast_sims;  // AZ_F_PLAYOUT_CAP: simulations of the current search if it is a fast one; 0 = a full search (a zeroed
+                      // header never looks like a finished search)
+  int32_t pad2[2];
 };
 static_assert(sizeof(TreeHdr) == 80, "TreeHdr size");
 
@@ -110,6 +112,12 @@ struct ResignTree {
   int32_t calib;    // no-resign calibration game
 };
 
+// AZ_F_PLAYOUT_CAP: the values of az_set_playout_cap
+struct PlayoutCapCfg {
+  int32_t fast_playouts;
+  int32_t full_permille;
+};
+
 struct Node;
 struct Params {
   TreeHdr* hdr;
@@ -129,6 +137,7 @@ struct Params {
   uint32_t* cache_epoch;     // [0] epoch of the current weights, [1] epoch of the rows the next k_cache_insert stores
   ResignCfg* resign_cfg;     // AZ_F_RESIGN, nullptr when off
   ResignTree* resign_tree;   // AZ_F_RESIGN: [n_trees]
+  PlayoutCapCfg* pcap_cfg;   // AZ_F_PLAYOUT_CAP, nullptr when off
   const double* logtab;  // AZ_F_UCT: log(n) for n < LOGTAB_N, computed on the host with the C library's log() -- the same
                          // function CPython's math.log calls, so the UCT scores are bit-equal to the reference's
   long long rec_cap;
@@ -142,6 +151,11 @@ struct Params {
   double c_puct, keep, noise_w, alpha, temperature;
   Geo geo;
 };
+
+// the simulations of the current search, fixed when it begins (begin_search; k_command for MCTS.playout)
+__device__ __forceinline__ int search_target(const Params& p, const TreeHdr& h) {
+  return h.fast_sims ? h.fast_sims : p.n_playouts;
+}
 
 struct StepIO {
   const void* priors;
@@ -716,9 +730,10 @@ __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, uns
     return;
   }
 
+  const int ply_end = h.fast_sims ? 3 : 0;  // the ply record's end: 3 marks a fast search (AZ_F_PLAYOUT_CAP)
   if ((p.flags & AZ_F_RESIGN) && resign_check<G>(p, h, tree, lane, gm, s.ply, root_q, a0c)) {
     if (p.flags & AZ_F_RECORDS) {
-      emit_record<GM, G>(p, tree, h, s, 0, -1, L, (int)rnl.x, root_q, a0c, v_off, 0, cnt, &lg, lane, gm, s_ctr);
+      emit_record<GM, G>(p, tree, h, s, 0, -1, L, (int)rnl.x, root_q, a0c, v_off, ply_end, cnt, &lg, lane, gm, s_ctr);
       const double ret0 = (s.ply & 1) ? 1.0 : -1.0;  // the mover loses
       emit_record<GM, G>(p, tree, h, s, 1, -1, 0, 0, ret0, 0.0, 0.0, 1, nullptr, nullptr, lane, gm, s_ctr);
     }
@@ -778,7 +793,7 @@ __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, uns
   }
   const int action = GM::action_of(lg, s, p.geo, k);
   if (p.flags & AZ_F_RECORDS)
-    emit_record<GM, G>(p, tree, h, s, 0, action, L, (int)rnl.x, root_q, a0c, v_off, 0, cnt, &lg, lane, gm, s_ctr);
+    emit_record<GM, G>(p, tree, h, s, 0, action, L, (int)rnl.x, root_q, a0c, v_off, ply_end, cnt, &lg, lane, gm, s_ctr);
 
   // ---- apply (game_utils.py:197)
   const St s2 = GM::apply(s, p.geo, action);
@@ -868,11 +883,20 @@ __device__ __forceinline__ void expand_root(const Params& p, const StepIO& io, T
 // MCTS.search (mcts.py:173-176) from PH_BEGIN.  Without root noise the simulations start at once (AZ_PH_RUN).  With it the root
 // is expanded first: from an AZ_F_EVAL_CACHE hit, or through a root request to evaluator row `row` -- then the tree waits in
 // AZ_PH_ROOT_EVAL and this returns true.  CACHE: the kernel looks up the cache (k_step_vl runs without one).
+// AZ_F_PLAYOUT_CAP: a fast search (counter stream 7) runs fast_playouts simulations and starts like one without root noise.
 template <class GM, int G, bool CACHE>
 __device__ __forceinline__ bool begin_search(const Params& p, const StepIO& io, TreeHdr& h, int tree, int row, int lane,
                                              unsigned gm, unsigned long long* s_ctr) {
   h.sims_done = 0;
   h.phase = AZ_PH_RUN;
+  h.fast_sims = 0;
+  if (p.flags & AZ_F_PLAYOUT_CAP) {
+    const PlayoutCapCfg c = *p.pcap_cfg;
+    if ((int)(counter(p.seed, tree, h.game_seq, h.root_ply, 0, 7) % 1000ULL) >= c.full_permille) {
+      h.fast_sims = c.fast_playouts;
+      return false;
+    }
+  }
   if (p.noise_mode == AZ_NOISE_NONE) return false;
   const St s = root_state(h);
   const CacheHead* hit = CACHE && p.cache ? cache_find<GM>(p, s) : nullptr;
@@ -961,7 +985,7 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
         if (lane == 0) ctr_add(s_ctr, AZ_CTR_IDLE_SLOTS, 1);
         break;
       }
-      if (h.sims_done >= p.n_playouts) {
+      if (h.sims_done >= search_target(p, h)) {
         if (advanced) {
           if (lane == 0) ctr_add(s_ctr, AZ_CTR_IDLE_SLOTS, 1);
           break;
@@ -1158,7 +1182,7 @@ __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const Step
         break;
       }
       if (h.phase != AZ_PH_RUN) break;
-      if (h.sims_done + n_pending >= p.n_playouts) {
+      if (h.sims_done + n_pending >= search_target(p, h)) {
         if (n_pending > 0 || advanced) break;
         finish_move<GM, G>(p, h, tree, lane, gm, s_ctr);
         advanced = true;
@@ -1368,6 +1392,7 @@ __global__ void k_command(const Params p, const int32_t* upd, const int32_t* rst
       if (beg[tree] == 2) {  // MCTS.playout (mcts.py:126-153): ONE simulation, no root Dirichlet expansion
         h.phase = AZ_PH_RUN;
         h.sims_done = p.n_playouts - 1;
+        h.fast_sims = 0;
         h.pend_depth = 0;
       } else {
         h.phase = PH_BEGIN;
@@ -1684,6 +1709,8 @@ int az_create(const az_config* cfg_in, az_engine** out) {
     return fail(-1, "AZ_F_VIRTUAL_LOSS is a batched self-play mode (no AZ_F_MANUAL / AZ_F_UCT)");
   if ((cfg.flags & AZ_F_RESIGN) && (cfg.flags & AZ_F_MANUAL))
     return fail(-1, "AZ_F_RESIGN is a batched self-play mode: with AZ_F_MANUAL the host decides the moves");
+  if ((cfg.flags & AZ_F_PLAYOUT_CAP) && (cfg.flags & AZ_F_MANUAL))
+    return fail(-1, "AZ_F_PLAYOUT_CAP is a batched self-play mode: with AZ_F_MANUAL the host starts the searches");
   if (cfg.record_capacity <= 0) cfg.record_capacity = cfg.n_trees * 64 < (1 << 20) ? (1 << 20) : cfg.n_trees * 64;
   if (!(cfg.flags & AZ_F_RECORDS)) cfg.record_capacity = 1;
   if (cfg.flags & AZ_F_EVAL_CACHE) {
@@ -1786,6 +1813,15 @@ int az_create(const az_config* cfg_in, az_engine** out) {
     const ResignCfg rc0 = {-1.0, 0, 0};  // never resigns
     CK(cudaMemcpy(p.resign_cfg, &rc0, sizeof(rc0), cudaMemcpyHostToDevice));
   }
+  if (cfg.flags & AZ_F_PLAYOUT_CAP) {
+    if ((err = alloc((void**)&p.pcap_cfg, sizeof(PlayoutCapCfg))) != cudaSuccess) {
+      fail(-2, "cudaMalloc failed (playout cap): %s", cudaGetErrorString(err));
+      az_destroy(e);
+      return -2;
+    }
+    const PlayoutCapCfg pc0 = {cfg.n_playouts, 1000};  // every search is full
+    CK(cudaMemcpy(p.pcap_cfg, &pc0, sizeof(pc0), cudaMemcpyHostToDevice));
+  }
   if (cfg.flags & AZ_F_UCT) {
     double* tab = nullptr;
     if ((err = alloc((void**)&tab, sizeof(double) * LOGTAB_N)) != cudaSuccess) {
@@ -1830,6 +1866,7 @@ int az_destroy(az_engine* e) {
   if (p.cache_epoch) cudaFree(p.cache_epoch);
   if (p.resign_cfg) cudaFree(p.resign_cfg);
   if (p.resign_tree) cudaFree(p.resign_tree);
+  if (p.pcap_cfg) cudaFree(p.pcap_cfg);
   cudaFree(e->d_cmd);
   cudaFree(e->d_bad);
   delete e;
@@ -1967,6 +2004,19 @@ int az_set_resign(az_engine* e, double threshold, int32_t disabled_permille, voi
   const ResignCfg rc = {threshold, disabled_permille, 0};
   // pageable source: the copy has been staged when the call returns
   CK(cudaMemcpyAsync(e->p.resign_cfg, &rc, sizeof(rc), cudaMemcpyHostToDevice, (cudaStream_t)stream));
+  return 0;
+}
+
+int az_set_playout_cap(az_engine* e, int32_t fast_playouts, int32_t full_permille, void* stream) {
+  if (!e) return fail(-1, "null engine");
+  if (!e->p.pcap_cfg) return fail(-1, "az_set_playout_cap: the engine was created without AZ_F_PLAYOUT_CAP");
+  if (fast_playouts < 1 || fast_playouts > e->p.n_playouts)
+    return fail(-1, "az_set_playout_cap: fast_playouts %d is outside [1, n_playouts = %d]", fast_playouts, e->p.n_playouts);
+  if (full_permille < 0 || full_permille > 1000)
+    return fail(-1, "az_set_playout_cap: full_permille %d is outside [0, 1000]", full_permille);
+  const PlayoutCapCfg pc = {fast_playouts, full_permille};
+  // pageable source: the copy has been staged when the call returns
+  CK(cudaMemcpyAsync(e->p.pcap_cfg, &pc, sizeof(pc), cudaMemcpyHostToDevice, (cudaStream_t)stream));
   return 0;
 }
 

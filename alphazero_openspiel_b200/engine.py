@@ -152,6 +152,11 @@ class Engine:
         a captured graph of step() sees the new values on its next replay."""
         L.check(self.lib.az_set_resign(self.h, float(threshold), int(disabled_permille), self._stream()))
 
+    def set_playout_cap(self, fast_playouts, full_permille):
+        """F_PLAYOUT_CAP: simulations of a fast search and per-mille share of full searches (az_set_playout_cap),
+        stream-ordered: a captured graph of step() sees the new values on its next replay."""
+        L.check(self.lib.az_set_playout_cap(self.h, int(fast_playouts), int(full_permille), self._stream()))
+
     def set_positions(self, histories):
         """histories: list (len n_trees) of action lists, or None entries to leave a tree untouched."""
         n = self.n_trees

@@ -97,7 +97,8 @@ def policy_targets_batch(counts, actions, n_legal, num_actions):
 
 def records_to_games(records, game_name, backup="on-policy"):
     """Device training records -> list of games in the reference's example format (game_utils.py:168-204).
-    Only games that have their closing (kind 1) record are returned."""
+    Only games that have their closing (kind 1) record are returned.  A fast search's ply record (F_PLAYOUT_CAP, end 3) is
+    no example, but its action stays in the history (the key) of the examples after it."""
     gid, rows, cols = parse_game_name(game_name)
     num_actions = 7 if gid == L.GAME_CONNECT_FOUR else rows * cols * 12
     if len(records) == 0:
@@ -126,6 +127,9 @@ def records_to_games(records, game_name, backup="on-policy"):
         reward = float(recs["root_q"][e - 1])  # kind-1 record carries returns()[0]
         for i in range(s, e - 1):
             r = recs[i]
+            if r["end"] == 3:
+                history.append(int(r["action"]))
+                continue
             pol = pols[pol_rows[i]].tolist()
             if backup == "soft-Z":
                 value = -float(r["root_q"])
@@ -173,7 +177,8 @@ class SelfPlayRunner:
                  backup="on-policy", seed=0, max_games=0, auto_restart=True, random_start_mod=0,
                  max_sims_per_step=16, records=True, use_graph=True, noise_mode=None, node_capacity=0,
                  record_capacity=0, evaluator="fused", virtual_loss=0, step_cycle_budget=None, eval_cache=None,
-                 eval_cache_log2=0, resign_threshold=None, resign_disabled_fraction=0.1, **_ignored):
+                 eval_cache_log2=0, resign_threshold=None, resign_disabled_fraction=0.1, fast_playouts=None,
+                 full_search_fraction=0.25, **_ignored):
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise L.EngineUnavailable("SelfPlayRunner needs a CUDA device; there is no CPU fallback")
@@ -192,6 +197,11 @@ class SelfPlayRunner:
             flags |= L.F_RANDOM_START
         if resign_threshold is not None:
             flags |= L.F_RESIGN     # resignation (an extension: the reference plays every game to its end)
+        if fast_playouts is not None:
+            # playout cap randomization (an extension: the reference runs every search with n_playouts): a
+            # full_search_fraction share of the searches is full, the others run fast_playouts simulations without root
+            # noise, and their positions are no training examples
+            flags |= L.F_PLAYOUT_CAP
         if noise_mode is None:
             noise_mode = L.NOISE_DIRICHLET if use_dirichlet else L.NOISE_NONE
         # virtual_loss = K > 0: K leaves in flight per tree (AZ_F_VIRTUAL_LOSS, NOT bit-exact with the reference), for pools
@@ -236,6 +246,8 @@ class SelfPlayRunner:
                                  step_cycle_budget=step_cycle_budget, eval_cache_log2=eval_cache_log2)
         if resign_threshold is not None:
             self.set_resign(resign_threshold, resign_disabled_fraction)
+        if fast_playouts is not None:
+            self.set_playout_cap(fast_playouts, full_search_fraction)
         self.use_graph = use_graph
         self._graph = None
         self._first = True
@@ -257,6 +269,12 @@ class SelfPlayRunner:
         on the next round, also in an already captured graph."""
         with torch.cuda.device(self.device):
             self.engine.set_resign(threshold, int(round(float(disabled_fraction) * 1000)))
+
+    def set_playout_cap(self, fast_playouts, full_search_fraction=0.25):
+        """Simulations of a fast search and share of full searches (needs fast_playouts at construction).  Takes effect for
+        the searches that begin from the next round on, also in an already captured graph."""
+        with torch.cuda.device(self.device):
+            self.engine.set_playout_cap(fast_playouts, int(round(float(full_search_fraction) * 1000)))
 
     @torch.no_grad()
     def _round_eager(self):
@@ -434,12 +452,14 @@ class ExampleGenerator:
         chunks = []
         # Drain the device record buffer before it can fill.  A tree emits one record per move (two when the game ends) and
         # runs at most max(1, max_sims_per_step) simulations per round, so at most 2 * n_trees * sims_per_round / n_playouts
-        # records arrive per round; drain when half the capacity could be used.
+        # records arrive per round; drain when half the capacity could be used.  With fast searches (fast_playouts) moves come
+        # up to n_playouts / fast_playouts times faster: the bound takes the smallest playout count.
         n_playouts = max(1, int(kw.get("n_playouts", 100)))
+        min_playouts = n_playouts if kw.get("fast_playouts") is None else max(1, min(n_playouts, int(kw["fast_playouts"])))
         cap = int(kw.get("max_sims_per_step", 16))
         sims_per_round = cap if cap > 0 else 64    # no count cap: the cycle budget / tree depth bound it far below this
         capacity = int(runner.engine.cfg.record_capacity)
-        drain_every = max(64, int(capacity * n_playouts / (4.0 * sims_per_round * n_trees)) // 64 * 64)
+        drain_every = max(64, int(capacity * min_playouts / (4.0 * sims_per_round * n_trees)) // 64 * 64)
         # upper bound on the round trips a generation can need: every game <= max plies, every ply <= n_playouts + 2 rounds
         max_plies = 42 if runner.engine.game_id == L.GAME_CONNECT_FOUR else 8 * runner.engine.rows * runner.engine.cols
         max_rounds = (n_games // n_trees + 2) * max_plies * (n_playouts + 3) + 1024
@@ -460,6 +480,7 @@ class ExampleGenerator:
             chunks.append(runner.drain())
             stats = runner.counters()
             stats["rounds"] = runner.rounds
+            stats["fast_searches"] = int(sum(((c["kind"] == 0) & (c["end"] == 3)).sum() for c in chunks))
             if stats["overflow"]:
                 raise RuntimeError("search arena / record buffer overflow (%d); raise node_capacity" %
                                    stats["overflow"])

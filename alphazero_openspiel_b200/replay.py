@@ -53,7 +53,8 @@ class ExampleBatch:
     @staticmethod
     def from_records(records, game_name, backup="on-policy"):
         """Device training records (engine.record_dtype) -> examples of the finished games, in (tree, game_seq) order.
-        Same selection, ordering and value targets as examplegenerator.records_to_games (game_utils.py:168-204)."""
+        Same selection, ordering and value targets as examplegenerator.records_to_games (game_utils.py:168-204): a fast
+        search's ply record (F_PLAYOUT_CAP, end 3) is no example, but its action is in the history of the examples after it."""
         gid, rows, cols = parse_game_name(game_name)
         num_actions = 7 if gid == L.GAME_CONNECT_FOUR else rows * cols * 12
         if len(records) == 0:
@@ -65,13 +66,15 @@ class ExampleBatch:
         ends = np.r_[starts[1:], len(recs)]
         finished = recs["kind"][ends - 1] == 1                       # the closing record carries returns()[0]
         starts, ends = starts[finished], ends[finished]
-        n_ply = ends - 1 - starts                                    # examples per game
-        game_ptr = np.r_[0, np.cumsum(n_ply)]
-        n = int(game_ptr[-1])
-        if n == 0:
+        if len(starts) == 0:
             return ExampleBatch.empty(game_name, num_actions)
-        g_of = np.repeat(np.arange(len(starts)), n_ply)              # game of every example
-        k_of = np.arange(n) - game_ptr[g_of]                         # ply index inside its game
+        n_ply = ends - 1 - starts                                    # ply records per game
+        g_rec = np.repeat(np.arange(len(starts)), n_ply)             # game of every ply record
+        k_rec = np.arange(int(n_ply.sum())) - np.r_[0, np.cumsum(n_ply)][g_rec]   # its index inside its game
+        full = recs["end"][starts[g_rec] + k_rec] != 3               # the examples: ply records of full searches
+        g_of, k_of = g_rec[full], k_rec[full]                        # game of every example, its ply index in the game
+        game_ptr = np.r_[0, np.cumsum(np.bincount(g_of, minlength=len(starts)))]
+        n = int(game_ptr[-1])
         src = starts[g_of] + k_of                                    # row in recs
         ex = recs[src]
         policy = policy_targets_batch(ex["counts"], ex["actions"], ex["n_legal"], num_actions)

@@ -77,6 +77,11 @@ class Trainer:
         self.resign_false_positive = 0.05
         self.resign_disabled_fraction = 0.1
         self.resign_threshold = -1.0
+        # Extension: playout cap randomization in self-play (KataGo; the reference runs every search with n_playouts_train).
+        # With fast_playouts set, a full_search_fraction share of the searches is full; the others run fast_playouts
+        # simulations without root noise, still choose the move, and their positions are no training examples.
+        self.fast_playouts = None
+        self.full_search_fraction = 0.25
         for k, v in overrides.items():
             if not hasattr(self, k):
                 raise TypeError("unknown Trainer setting %r" % k)
@@ -281,6 +286,9 @@ class Trainer:
             engine_kwargs = dict(engine_kwargs, resign_threshold=self.resign_threshold,
                                  resign_disabled_fraction=self.resign_disabled_fraction,
                                  resign_false_positive=self.resign_false_positive)
+        if self.fast_playouts is not None:
+            engine_kwargs = dict(engine_kwargs, fast_playouts=self.fast_playouts,
+                                 full_search_fraction=self.full_search_fraction)
         generator = ExampleGenerator(self.current_net, self.name_game, self.device,
                                      n_playouts=self.n_playouts_train, temperature=self.temperature,
                                      dirichlet_ratio=self.dirichlet_ratio, c_puct=self.uct_train, backup=self.backup,

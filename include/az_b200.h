@@ -36,7 +36,9 @@
  *   mix64 = splitmix64 finaliser; counter(seed,tree,game_seq,ply,idx,stream) = 6 chained mix64
  *   (oracle/az_oracle.c:oz_counter is the CPU restatement).  stream 1 = root noise, 2 = move sampling,
  *   3 = random start plies, 4 = number of random start plies, 5 = device Dirichlet gammas,
- *   6 = no-resign calibration games (AZ_F_RESIGN: counter(seed,tree,game_seq,0,0,6) % 1000 < disabled_permille).
+ *   6 = no-resign calibration games (AZ_F_RESIGN: counter(seed,tree,game_seq,0,0,6) % 1000 < disabled_permille),
+ *   7 = fast searches (AZ_F_PLAYOUT_CAP: the search at root ply `ply` is fast iff
+ *       counter(seed,tree,game_seq,ply,0,7) % 1000 >= full_permille).
  */
 #ifndef AZ_B200_H
 #define AZ_B200_H
@@ -92,6 +94,14 @@ extern "C" {
                                           the game ends like a terminal one.  A no-resign calibration game (counter stream 6,
                                           decided at its first searched position) never resigns and keeps each player's
                                           minimum r.  Threshold and permille: az_set_resign.  Not with AZ_F_MANUAL */
+#define AZ_F_PLAYOUT_CAP    (1u << 14) /* playout cap randomization (KataGo; an extension: the reference runs every search with
+                                          n_playouts).  A search is decided when it begins: fast with counter stream 7 (see
+                                          above), else full.  A full search is the usual one.  A fast search runs fast_playouts
+                                          simulations instead of n_playouts and has no root noise (it starts like AZ_NOISE_NONE:
+                                          no root request, no AZ_CTR_ROOT_EVALS); the move choice and tree reuse are unchanged.
+                                          Its ply record carries end = 3 so that it can be left out of the training examples
+                                          (it stays in the record stream: later positions' action histories need its action).
+                                          fast_playouts and full_permille: az_set_playout_cap.  Not with AZ_F_MANUAL */
 #define AZ_EVAL_CACHE_LOG2_SHIFT 24
 #define AZ_EVAL_CACHE_LOG2(flags) (((flags) >> AZ_EVAL_CACHE_LOG2_SHIFT) & 31u)
 #define AZ_EVAL_CACHE_EXTRA_LOG2 1
@@ -159,7 +169,8 @@ typedef struct az_record {
   int32_t n_legal, kind;               /* kind 0 = ply, 1 = game end */
   int32_t root_n;
   int32_t end;                         /* kind 1: 0 = terminal position, 1 = resigned, 2 = calibration game (AZ_F_RESIGN)
-                                          that reached a terminal position; kind 0: 0 */
+                                          that reached a terminal position; kind 0: 3 = a fast search (AZ_F_PLAYOUT_CAP),
+                                          else 0 */
   uint64_t bb[2];                      /* position the search ran on (kind 1: final or resign position) */
   double root_q;                       /* soft-Z target is -root_q (game_utils.py:174); kind 1: returns()[0] */
   double v_a0c;                        /* game_utils.py:178; kind 1 with end 2: player 0's minimum r (2.0: never moved) */
@@ -242,6 +253,13 @@ int az_eval_cache_invalidate(az_engine* e, void* stream);
  * permille in force at its first searched position.  Rejects a non-finite threshold, a permille outside [0, 1000] and an
  * engine created without AZ_F_RESIGN. */
 int az_set_resign(az_engine* e, double threshold, int32_t disabled_permille, void* stream);
+
+/* AZ_F_PLAYOUT_CAP: simulations of a fast search and the share of full searches, in per mille (0..1000).  A stream-ordered
+ * write to device memory like az_set_resign: a captured CUDA graph of az_step uses the new values on its next replay.  A
+ * search is decided with the values in force when it begins.  After az_create: fast_playouts = n_playouts, permille 1000
+ * (every search is full).  Rejects fast_playouts outside [1, n_playouts], a permille outside [0, 1000] and an engine
+ * created without AZ_F_PLAYOUT_CAP. */
+int az_set_playout_cap(az_engine* e, int32_t fast_playouts, int32_t full_permille, void* stream);
 
 /* Re-root compaction (MCTS.update_root, mcts.py:192-203) of the trees that played a move in the last az_step: BFS-copies
  * the kept subtree into the other arena half, one warp per tree.  az_step runs it first by itself unless
