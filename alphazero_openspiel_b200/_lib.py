@@ -15,6 +15,7 @@ F_VIRTUAL_LOSS = 1 << 11
 F_EVAL_CACHE = 1 << 12
 F_RESIGN = 1 << 13
 F_PLAYOUT_CAP = 1 << 14
+F_FORCED_PLAYOUTS = 1 << 15
 EVAL_CACHE_LOG2_SHIFT = 24   # flags bits 24-28: log2 of the F_EVAL_CACHE table's entries (0 = default)
 NOISE_NONE, NOISE_DIRICHLET, NOISE_HOST, NOISE_COUNTER = 0, 1, 2, 3
 EVAL_EXTERNAL, EVAL_UNIFORM, EVAL_HASH, EVAL_ROLLOUT = 0, 1, 2, 3
@@ -73,6 +74,7 @@ SIGNATURES = {
     "az_eval_cache_invalidate": (C.c_int, [C.c_void_p, _VP]),
     "az_set_resign": (C.c_int, [C.c_void_p, C.c_double, C.c_int32, _VP]),
     "az_set_playout_cap": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, _VP]),
+    "az_set_forced_playouts": (C.c_int, [C.c_void_p, C.c_double, _VP]),
     "az_debug_timing": (C.c_int, [C.c_void_p, _VP]),
     "az_status": (C.c_int, [C.c_void_p, _I32P, _I32P, _I32P, _I32P, _VP]),
     "az_request_info": (C.c_int, [C.c_void_p, _U64P, _I32P, _I32P, _I32P, C.c_int32, _VP]),

@@ -61,9 +61,17 @@ struct __align__(16) TreeHdr {
   uint8_t phase, half, err, uct;  // uct: this tree scores with the use_puct=False formula (see fresh_tree)
   int32_t fast_sims;  // AZ_F_PLAYOUT_CAP: simulations of the current search if it is a fast one; 0 = a full search (a zeroed
                       // header never looks like a finished search)
-  int32_t pad2[2];
+  int32_t forced_lo, forced_hi;  // AZ_F_FORCED_PLAYOUTS: k of the current search if it is a forced one, 0 = not forced; the
+                                 // halves of a double (forced_k / set_forced_k): a double member changes the register
+                                 // allocation of the step kernels that never read it
 };
 static_assert(sizeof(TreeHdr) == 80, "TreeHdr size");
+
+__device__ __forceinline__ double forced_k(const TreeHdr& h) { return __hiloint2double(h.forced_hi, h.forced_lo); }
+__device__ __forceinline__ void set_forced_k(TreeHdr& h, double k) {
+  h.forced_lo = __double2loint(k);
+  h.forced_hi = __double2hiint(k);
+}
 
 __device__ __forceinline__ St root_state(const TreeHdr& h) {
   St s;
@@ -150,6 +158,7 @@ struct Params {
   uint64_t seed;
   double c_puct, keep, noise_w, alpha, temperature;
   Geo geo;
+  double* forced_cfg;  // AZ_F_FORCED_PLAYOUTS: k of az_set_forced_playouts, nullptr when off
 };
 
 // the simulations of the current search, fixed when it begins (begin_search; k_command for MCTS.playout)
@@ -444,12 +453,18 @@ __device__ __forceinline__ bool expand_node(const Params& p, const StepIO& io, c
 
 constexpr int LOGTAB_N = 1 << 20;  // parent visit counts covered by the AZ_F_UCT log table (a game has < 1e5 simulations)
 
+// AZ_F_FORCED_PLAYOUTS: the forced-playout floor nf(c) = sqrt((k * P(c)) * N_root) of a root child
+__device__ __forceinline__ double forced_floor(double k, double prior, unsigned n_root) {
+  return __dsqrt_rn(__dmul_rn(__dmul_rn(k, prior), (double)n_root));
+}
+
 // One PUCT (or, UCT = true, use_puct=False) descent (mcts.py:139-142).  On return: node/depth/state of the childless node
-// reached; path in spath.
-template <class GM, int G, bool UCT>
+// reached; path in spath.  FORCED (AZ_F_FORCED_PLAYOUTS) with forced_k > 0: at the root, a visited child below its floor
+// (1 <= N(c) < nf(c)) scores +inf, so the first such child in legal order is taken.
+template <class GM, int G, bool UCT, bool FORCED = false>
 __device__ __forceinline__ void sim_select(const Params& p, const Arena& a, int root, St& s, int& node, int& depth,
                                            int32_t* spath, int lane, unsigned gm, unsigned long long& n_children,
-                                           bool& depth_overflow, bool tree_uct) {
+                                           bool& depth_overflow, bool tree_uct, double forced_k = 0.0) {
   node = root;
   depth = 0;
   if (lane == 0) spath[0] = root;
@@ -463,6 +478,7 @@ __device__ __forceinline__ void sim_select(const Params& p, const Arena& a, int 
     // UCT: log(N_parent); a parent beyond the table (never in practice) is treated like the last entry and flagged
     const double lg_np = (UCT && tree_uct) ? p.logtab[cur.x < (unsigned)LOGTAB_N ? cur.x : (unsigned)(LOGTAB_N - 1)] : 0.0;
     if (UCT && tree_uct && cur.x >= (unsigned)LOGTAB_N) depth_overflow = true;
+    const bool forced = FORCED && depth == 0 && forced_k > 0.0;
     double best = 0.0;
     int bi = 0x7fffffff;
     uint2 bnl = make_uint2(0u, 0u);
@@ -482,6 +498,8 @@ __device__ __forceinline__ void sim_select(const Params& p, const Arena& a, int 
           // Q + (((c_puct * P) * sqrt(N_parent)) / (N + 1))      mcts.py:78
           const double u = __ddiv_rn(__dmul_rn(__dmul_rn(p.c_puct, pp), sq), (double)(nl.x + 1u));
           sc = __dadd_rn(q, u);
+          if (forced && nl.x >= 1u && (double)nl.x < forced_floor(forced_k, pp, cur.x))
+            sc = __longlong_as_double(0x7ff0000000000000LL);
         }
         if (bi == 0x7fffffff || sc > best) { best = sc; bi = i; bnl = nl; }
       }
@@ -688,9 +706,46 @@ __device__ int resign_game_over(const Params& p, int tree, int lane, unsigned gm
   return 2;
 }
 
-// AlphaZeroBot.step after the search (alphazerobot.py:72-93) + play_game_self bookkeeping (game_utils.py:156-204).
-// Sets h.phase to PH_BEGIN / AZ_PH_IDLE / AZ_PH_SEARCH_DONE.
+// AZ_F_FORCED_PLAYOUTS policy target pruning (see az_b200.h) of the root child counts cnt (per lane, legal order; qv their
+// Q) after a forced search with k = forced_k.  c* (the first maximal count) keeps its count; every other visited child drops
+// to the smallest n >= N - nf whose PUCT score stays below c*'s (sim_select's expression), and a remainder of 1 to 0.  Changes
+// no node.  Returns the new total.
 template <class GM, int G>
+__device__ int prune_counts(const Params& p, const Arena& a, int fc, int nc, unsigned n_root, double forced_k, int* cnt,
+                            const double* qv, int lane, unsigned gm) {
+  double bv = -1.0;
+  int bi = 0x7fffffff;
+#pragma unroll
+  for (int sl = 0; sl < GM::SLOTS; ++sl) {
+    const int i = lane + sl * G;
+    if (i < nc && (bi == 0x7fffffff || (double)cnt[sl] > bv)) { bv = (double)cnt[sl]; bi = i; }
+  }
+  gargmax<G>(gm, bv, bi);
+  const double sq = __dsqrt_rn((double)n_root);
+  const double s_star =
+      __dadd_rn(a.q(fc + bi), __ddiv_rn(__dmul_rn(__dmul_rn(p.c_puct, a.p(fc + bi)), sq), (double)((unsigned)bv + 1u)));
+  int total = 0;
+#pragma unroll
+  for (int sl = 0; sl < GM::SLOTS; ++sl) {
+    const int i = lane + sl * G;
+    if (i < nc && i != bi && cnt[sl] > 0) {
+      const double pp = a.p(fc + i);
+      const double cps = __dmul_rn(__dmul_rn(p.c_puct, pp), sq);
+      const double lo = __dsub_rn((double)cnt[sl], forced_floor(forced_k, pp, n_root));
+      int n = cnt[sl];
+      // score(n - 1) = Q + cps / n is non-increasing in n: step down while n - 1 is still allowed
+      while (n > 0 && (double)(n - 1) >= lo && __dadd_rn(qv[sl], __ddiv_rn(cps, (double)n)) < s_star) --n;
+      cnt[sl] = n == 1 ? 0 : n;
+    }
+    total += cnt[sl];
+  }
+  return gsum<G>(gm, total);
+}
+
+// AlphaZeroBot.step after the search (alphazerobot.py:72-93) + play_game_self bookkeeping (game_utils.py:156-204).
+// Sets h.phase to PH_BEGIN / AZ_PH_IDLE / AZ_PH_SEARCH_DONE.  FORCED: after a forced search (AZ_F_FORCED_PLAYOUTS) the
+// move choice and the ply record use the pruned counts (prune_counts); everything else uses the tree as it is.
+template <class GM, int G, bool FORCED = false>
 __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, unsigned gm, unsigned long long* s_ctr) {
   const Arena a = arena_of(p, tree, h.half);
   const St s = root_state(h);
@@ -730,6 +785,8 @@ __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, uns
     return;
   }
 
+  if (FORCED && forced_k(h) > 0.0 && nc > 0)
+    total = prune_counts<GM, G>(p, a, fc, nc, rnl.x, forced_k(h), cnt, qv, lane, gm);
   const int ply_end = h.fast_sims ? 3 : 0;  // the ply record's end: 3 marks a fast search (AZ_F_PLAYOUT_CAP)
   if ((p.flags & AZ_F_RESIGN) && resign_check<G>(p, h, tree, lane, gm, s.ply, root_q, a0c)) {
     if (p.flags & AZ_F_RECORDS) {
@@ -884,12 +941,14 @@ __device__ __forceinline__ void expand_root(const Params& p, const StepIO& io, T
 // is expanded first: from an AZ_F_EVAL_CACHE hit, or through a root request to evaluator row `row` -- then the tree waits in
 // AZ_PH_ROOT_EVAL and this returns true.  CACHE: the kernel looks up the cache (k_step_vl runs without one).
 // AZ_F_PLAYOUT_CAP: a fast search (counter stream 7) runs fast_playouts simulations and starts like one without root noise.
-template <class GM, int G, bool CACHE>
+// FORCED (AZ_F_FORCED_PLAYOUTS): a search with root noise takes the k of az_set_forced_playouts in force now (0: not forced).
+template <class GM, int G, bool CACHE, bool FORCED = false>
 __device__ __forceinline__ bool begin_search(const Params& p, const StepIO& io, TreeHdr& h, int tree, int row, int lane,
                                              unsigned gm, unsigned long long* s_ctr) {
   h.sims_done = 0;
   h.phase = AZ_PH_RUN;
   h.fast_sims = 0;
+  if (FORCED) set_forced_k(h, 0.0);
   if (p.flags & AZ_F_PLAYOUT_CAP) {
     const PlayoutCapCfg c = *p.pcap_cfg;
     if ((int)(counter(p.seed, tree, h.game_seq, h.root_ply, 0, 7) % 1000ULL) >= c.full_permille) {
@@ -898,6 +957,7 @@ __device__ __forceinline__ bool begin_search(const Params& p, const StepIO& io, 
     }
   }
   if (p.noise_mode == AZ_NOISE_NONE) return false;
+  if (FORCED) set_forced_k(h, *p.forced_cfg);
   const St s = root_state(h);
   const CacheHead* hit = CACHE && p.cache ? cache_find<GM>(p, s) : nullptr;
   if (hit) {
@@ -944,7 +1004,8 @@ __device__ __forceinline__ void terminal_leaf(const Arena& a, TreeHdr& h, const 
 }
 
 // ---------------------------------------------------------------- the step kernel
-template <class GM, bool UCT>
+// FORCED: the instantiation of AZ_F_FORCED_PLAYOUTS engines (forced playouts in sim_select, pruning in finish_move)
+template <class GM, bool UCT, bool FORCED = false>
 __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params p, const StepIO io) {
   constexpr int G = GM::G;
   __shared__ int32_t s_path[BLOCK / G][GM::MAXD];
@@ -980,7 +1041,7 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
     int sims_this_step = 0;
     bool advanced = false;
     for (;;) {
-      if (h.phase == PH_BEGIN && begin_search<GM, G, true>(p, io, h, tree, tree, lane, gm, s_ctr)) break;
+      if (h.phase == PH_BEGIN && begin_search<GM, G, true, FORCED>(p, io, h, tree, tree, lane, gm, s_ctr)) break;
       if (h.phase != AZ_PH_RUN) {
         if (lane == 0) ctr_add(s_ctr, AZ_CTR_IDLE_SLOTS, 1);
         break;
@@ -990,7 +1051,7 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
           if (lane == 0) ctr_add(s_ctr, AZ_CTR_IDLE_SLOTS, 1);
           break;
         }
-        finish_move<GM, G>(p, h, tree, lane, gm, s_ctr);
+        finish_move<GM, G, FORCED>(p, h, tree, lane, gm, s_ctr);
         advanced = true;
         continue;
       }
@@ -1013,7 +1074,8 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
       St s = root_state(h);
       int node, depth;
       bool dovf = false;
-      sim_select<GM, G, UCT>(p, a, h.root_node, s, node, depth, spath, lane, gm, c.children, dovf, h.uct != 0);
+      sim_select<GM, G, UCT, FORCED>(p, a, h.root_node, s, node, depth, spath, lane, gm, c.children, dovf, h.uct != 0,
+                                     FORCED ? forced_k(h) : 0.0);
       if (dovf) {
         h.err = 1;
         h.phase = AZ_PH_ERROR;
@@ -1133,7 +1195,7 @@ __device__ __forceinline__ void vl_backup(const Arena& a, const int32_t* path, i
   }
 }
 
-template <class GM>
+template <class GM, bool FORCED = false>
 __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const StepIO io) {
   constexpr int G = GM::G;
   __shared__ int32_t s_path[BLOCK / G][GM::MAXD];
@@ -1177,14 +1239,14 @@ __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const Step
     int n_pending = 0, sims_this_step = 0;
     bool advanced = false;
     for (;;) {
-      if (h.phase == PH_BEGIN && begin_search<GM, G, false>(p, io, h, tree, row0, lane, gm, s_ctr)) {
+      if (h.phase == PH_BEGIN && begin_search<GM, G, false, FORCED>(p, io, h, tree, row0, lane, gm, s_ctr)) {
         n_pending = 1;   // (one evaluator row in use; not a leaf request)
         break;
       }
       if (h.phase != AZ_PH_RUN) break;
       if (h.sims_done + n_pending >= search_target(p, h)) {
         if (n_pending > 0 || advanced) break;
-        finish_move<GM, G>(p, h, tree, lane, gm, s_ctr);
+        finish_move<GM, G, FORCED>(p, h, tree, lane, gm, s_ctr);
         advanced = true;
         continue;
       }
@@ -1194,7 +1256,8 @@ __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const Step
       St s = root_state(h);
       int node, depth;
       bool dovf = false;
-      sim_select<GM, G, false>(p, a, h.root_node, s, node, depth, spath, lane, gm, c.children, dovf, false);
+      sim_select<GM, G, false, FORCED>(p, a, h.root_node, s, node, depth, spath, lane, gm, c.children, dovf, false,
+                                       FORCED ? forced_k(h) : 0.0);
       if (dovf) {
         h.err = 1;
         h.phase = AZ_PH_ERROR;
@@ -1393,6 +1456,7 @@ __global__ void k_command(const Params p, const int32_t* upd, const int32_t* rst
         h.phase = AZ_PH_RUN;
         h.sims_done = p.n_playouts - 1;
         h.fast_sims = 0;
+        set_forced_k(h, 0.0);
         h.pend_depth = 0;
       } else {
         h.phase = PH_BEGIN;
@@ -1711,6 +1775,12 @@ int az_create(const az_config* cfg_in, az_engine** out) {
     return fail(-1, "AZ_F_RESIGN is a batched self-play mode: with AZ_F_MANUAL the host decides the moves");
   if ((cfg.flags & AZ_F_PLAYOUT_CAP) && (cfg.flags & AZ_F_MANUAL))
     return fail(-1, "AZ_F_PLAYOUT_CAP is a batched self-play mode: with AZ_F_MANUAL the host starts the searches");
+  if ((cfg.flags & AZ_F_FORCED_PLAYOUTS) && (cfg.flags & AZ_F_MANUAL))
+    return fail(-1, "AZ_F_FORCED_PLAYOUTS is a batched self-play mode: with AZ_F_MANUAL the host decides the moves");
+  if ((cfg.flags & AZ_F_FORCED_PLAYOUTS) && (cfg.flags & AZ_F_UCT))
+    return fail(-1, "AZ_F_FORCED_PLAYOUTS is a PUCT rule: AZ_F_UCT scores with the use_puct=False formula");
+  if ((cfg.flags & AZ_F_FORCED_PLAYOUTS) && cfg.noise_mode == AZ_NOISE_NONE)
+    return fail(-1, "AZ_F_FORCED_PLAYOUTS forces only searches with root noise: AZ_NOISE_NONE has none");
   if (cfg.record_capacity <= 0) cfg.record_capacity = cfg.n_trees * 64 < (1 << 20) ? (1 << 20) : cfg.n_trees * 64;
   if (!(cfg.flags & AZ_F_RECORDS)) cfg.record_capacity = 1;
   if (cfg.flags & AZ_F_EVAL_CACHE) {
@@ -1822,6 +1892,15 @@ int az_create(const az_config* cfg_in, az_engine** out) {
     const PlayoutCapCfg pc0 = {cfg.n_playouts, 1000};  // every search is full
     CK(cudaMemcpy(p.pcap_cfg, &pc0, sizeof(pc0), cudaMemcpyHostToDevice));
   }
+  if (cfg.flags & AZ_F_FORCED_PLAYOUTS) {
+    if ((err = alloc((void**)&p.forced_cfg, sizeof(double))) != cudaSuccess) {
+      fail(-2, "cudaMalloc failed (forced playouts): %s", cudaGetErrorString(err));
+      az_destroy(e);
+      return -2;
+    }
+    const double k0 = 0.0;  // no search is forced
+    CK(cudaMemcpy(p.forced_cfg, &k0, sizeof(k0), cudaMemcpyHostToDevice));
+  }
   if (cfg.flags & AZ_F_UCT) {
     double* tab = nullptr;
     if ((err = alloc((void**)&tab, sizeof(double) * LOGTAB_N)) != cudaSuccess) {
@@ -1867,6 +1946,7 @@ int az_destroy(az_engine* e) {
   if (p.resign_cfg) cudaFree(p.resign_cfg);
   if (p.resign_tree) cudaFree(p.resign_tree);
   if (p.pcap_cfg) cudaFree(p.pcap_cfg);
+  if (p.forced_cfg) cudaFree(p.forced_cfg);
   cudaFree(e->d_cmd);
   cudaFree(e->d_bad);
   delete e;
@@ -1978,9 +2058,18 @@ int az_step(az_engine* e, const void* priors_dev, const void* values_dev, const 
     using GM = decltype(gm);
     // k_step stays the last launch of az_step: the evaluator's first kernel waits on it with griddepcontrol.wait
     if (p.cache && priors_dev) k_cache_insert<GM><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p, io);
-    if (p.flags & AZ_F_VIRTUAL_LOSS) k_step_vl<GM><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p, io);
-    else if (p.flags & AZ_F_UCT) k_step<GM, true><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p, io);
-    else k_step<GM, false><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p, io);
+    const dim3 grid = groups_grid(p.n_trees, GM::G, BLOCK);
+    const bool forced = (p.flags & AZ_F_FORCED_PLAYOUTS) != 0;
+    if (p.flags & AZ_F_VIRTUAL_LOSS) {
+      if (forced) k_step_vl<GM, true><<<grid, BLOCK, 0, st>>>(p, io);
+      else k_step_vl<GM><<<grid, BLOCK, 0, st>>>(p, io);
+    } else if (p.flags & AZ_F_UCT) {
+      k_step<GM, true><<<grid, BLOCK, 0, st>>>(p, io);
+    } else if (forced) {
+      k_step<GM, false, true><<<grid, BLOCK, 0, st>>>(p, io);
+    } else {
+      k_step<GM, false><<<grid, BLOCK, 0, st>>>(p, io);
+    }
     return 0;
   });
   CK(cudaGetLastError());
@@ -2017,6 +2106,15 @@ int az_set_playout_cap(az_engine* e, int32_t fast_playouts, int32_t full_permill
   const PlayoutCapCfg pc = {fast_playouts, full_permille};
   // pageable source: the copy has been staged when the call returns
   CK(cudaMemcpyAsync(e->p.pcap_cfg, &pc, sizeof(pc), cudaMemcpyHostToDevice, (cudaStream_t)stream));
+  return 0;
+}
+
+int az_set_forced_playouts(az_engine* e, double k, void* stream) {
+  if (!e) return fail(-1, "null engine");
+  if (!e->p.forced_cfg) return fail(-1, "az_set_forced_playouts: the engine was created without AZ_F_FORCED_PLAYOUTS");
+  if (!isfinite(k) || k < 0.0) return fail(-1, "az_set_forced_playouts: k must be finite and >= 0 (got %g)", k);
+  // pageable source: the copy has been staged when the call returns
+  CK(cudaMemcpyAsync(e->p.forced_cfg, &k, sizeof(k), cudaMemcpyHostToDevice, (cudaStream_t)stream));
   return 0;
 }
 

@@ -157,6 +157,11 @@ class Engine:
         stream-ordered: a captured graph of step() sees the new values on its next replay."""
         L.check(self.lib.az_set_playout_cap(self.h, int(fast_playouts), int(full_permille), self._stream()))
 
+    def set_forced_playouts(self, k):
+        """F_FORCED_PLAYOUTS: k of the forced-playout floor sqrt(k * P * N) (az_set_forced_playouts; 0 forces nothing),
+        stream-ordered: a captured graph of step() sees the new value on its next replay."""
+        L.check(self.lib.az_set_forced_playouts(self.h, float(k), self._stream()))
+
     def set_positions(self, histories):
         """histories: list (len n_trees) of action lists, or None entries to leave a tree untouched."""
         n = self.n_trees

@@ -178,7 +178,7 @@ class SelfPlayRunner:
                  max_sims_per_step=16, records=True, use_graph=True, noise_mode=None, node_capacity=0,
                  record_capacity=0, evaluator="fused", virtual_loss=0, step_cycle_budget=None, eval_cache=None,
                  eval_cache_log2=0, resign_threshold=None, resign_disabled_fraction=0.1, fast_playouts=None,
-                 full_search_fraction=0.25, **_ignored):
+                 full_search_fraction=0.25, forced_playouts=None, **_ignored):
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise L.EngineUnavailable("SelfPlayRunner needs a CUDA device; there is no CPU fallback")
@@ -202,6 +202,11 @@ class SelfPlayRunner:
             # full_search_fraction share of the searches is full, the others run fast_playouts simulations without root
             # noise, and their positions are no training examples
             flags |= L.F_PLAYOUT_CAP
+        if forced_playouts is not None:
+            # forced playouts and policy target pruning (an extension the reference does not have): every visited root
+            # child of a search with root noise gets at least sqrt(k * P * N) visits, and the visits it got only from that
+            # floor are taken out of the policy target and the move choice
+            flags |= L.F_FORCED_PLAYOUTS
         if noise_mode is None:
             noise_mode = L.NOISE_DIRICHLET if use_dirichlet else L.NOISE_NONE
         # virtual_loss = K > 0: K leaves in flight per tree (AZ_F_VIRTUAL_LOSS, NOT bit-exact with the reference), for pools
@@ -248,6 +253,8 @@ class SelfPlayRunner:
             self.set_resign(resign_threshold, resign_disabled_fraction)
         if fast_playouts is not None:
             self.set_playout_cap(fast_playouts, full_search_fraction)
+        if forced_playouts is not None:
+            self.set_forced_playouts(forced_playouts)
         self.use_graph = use_graph
         self._graph = None
         self._first = True
@@ -275,6 +282,12 @@ class SelfPlayRunner:
         the searches that begin from the next round on, also in an already captured graph."""
         with torch.cuda.device(self.device):
             self.engine.set_playout_cap(fast_playouts, int(round(float(full_search_fraction) * 1000)))
+
+    def set_forced_playouts(self, k):
+        """k of the forced playouts (needs forced_playouts at construction; 0 forces nothing, 2.0 is KataGo's value).  Takes
+        effect for the searches that begin from the next round on, also in an already captured graph."""
+        with torch.cuda.device(self.device):
+            self.engine.set_forced_playouts(k)
 
     @torch.no_grad()
     def _round_eager(self):

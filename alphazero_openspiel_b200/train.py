@@ -82,6 +82,10 @@ class Trainer:
         # simulations without root noise, still choose the move, and their positions are no training examples.
         self.fast_playouts = None
         self.full_search_fraction = 0.25
+        # Extension: forced playouts and policy target pruning in self-play (KataGo; the reference has neither).  With
+        # forced_playouts = k (2.0 in the paper), every visited root child of a search with root noise gets at least
+        # sqrt(k * P * N) visits, and the visits it got only from that floor are pruned from its policy target.
+        self.forced_playouts = None
         for k, v in overrides.items():
             if not hasattr(self, k):
                 raise TypeError("unknown Trainer setting %r" % k)
@@ -289,6 +293,8 @@ class Trainer:
         if self.fast_playouts is not None:
             engine_kwargs = dict(engine_kwargs, fast_playouts=self.fast_playouts,
                                  full_search_fraction=self.full_search_fraction)
+        if self.forced_playouts is not None:
+            engine_kwargs = dict(engine_kwargs, forced_playouts=self.forced_playouts)
         generator = ExampleGenerator(self.current_net, self.name_game, self.device,
                                      n_playouts=self.n_playouts_train, temperature=self.temperature,
                                      dirichlet_ratio=self.dirichlet_ratio, c_puct=self.uct_train, backup=self.backup,

@@ -102,6 +102,21 @@ extern "C" {
                                           Its ply record carries end = 3 so that it can be left out of the training examples
                                           (it stays in the record stream: later positions' action histories need its action).
                                           fast_playouts and full_permille: az_set_playout_cap.  Not with AZ_F_MANUAL */
+#define AZ_F_FORCED_PLAYOUTS (1u << 15) /* forced playouts and policy target pruning (KataGo; an extension: the reference has
+                                          neither).  A search is forced iff, when it begins, k (az_set_forced_playouts) is > 0
+                                          and it has root noise (not an AZ_F_PLAYOUT_CAP fast search); it keeps that k.  All
+                                          fp64, rounded to nearest; N_root = the root's visit count (the sqrt of the PUCT
+                                          score), which differs from the paper's sum of child visits by at most 1.
+                                          Selection, root only: nf(c) = sqrt((k * P(c)) * N_root) with P the noise-mixed
+                                          prior; a child with 1 <= N(c) < nf(c) scores +inf, so the first one in legal order is
+                                          taken; unvisited children are never forced.  Pruning, after the search: c* = the
+                                          first child with the maximal count keeps it; every other child with N > 0 gets the
+                                          smallest n with N - nf <= n <= N and (n == N or Q + ((c_puct * P) * sqrt(N_root)) /
+                                          (n + 1) < the same score of c* at N(c*)); a pruned count of 1 becomes 0.  The
+                                          pruned counts are the ones the move is sampled from (argmax cannot change) and the
+                                          ply record's counts (root_n stays the raw visit count); root_q, v_a0c, v_offpolicy,
+                                          resignation and tree reuse see the tree as it is.  k: az_set_forced_playouts (0 after
+                                          az_create).  Not with AZ_F_MANUAL, AZ_F_UCT or AZ_NOISE_NONE */
 #define AZ_EVAL_CACHE_LOG2_SHIFT 24
 #define AZ_EVAL_CACHE_LOG2(flags) (((flags) >> AZ_EVAL_CACHE_LOG2_SHIFT) & 31u)
 #define AZ_EVAL_CACHE_EXTRA_LOG2 1
@@ -260,6 +275,12 @@ int az_set_resign(az_engine* e, double threshold, int32_t disabled_permille, voi
  * (every search is full).  Rejects fast_playouts outside [1, n_playouts], a permille outside [0, 1000] and an engine
  * created without AZ_F_PLAYOUT_CAP. */
 int az_set_playout_cap(az_engine* e, int32_t fast_playouts, int32_t full_permille, void* stream);
+
+/* AZ_F_FORCED_PLAYOUTS: the k of the forced-playout floor (the paper's value is 2; 0 forces no search).  A stream-ordered
+ * write to device memory like az_set_playout_cap: a captured CUDA graph of az_step uses the new value on its next replay.
+ * A search keeps the k in force when it begins.  After az_create: k = 0.  Rejects a non-finite or negative k and an engine
+ * created without AZ_F_FORCED_PLAYOUTS. */
+int az_set_forced_playouts(az_engine* e, double k, void* stream);
 
 /* Re-root compaction (MCTS.update_root, mcts.py:192-203) of the trees that played a move in the last az_step: BFS-copies
  * the kept subtree into the other arena half, one warp per tree.  az_step runs it first by itself unless
