@@ -16,6 +16,7 @@ F_EVAL_CACHE = 1 << 12
 F_RESIGN = 1 << 13
 F_PLAYOUT_CAP = 1 << 14
 F_FORCED_PLAYOUTS = 1 << 15
+F_REFLECT = 1 << 16
 EVAL_CACHE_LOG2_SHIFT = 24   # flags bits 24-28: log2 of the F_EVAL_CACHE table's entries (0 = default)
 NOISE_NONE, NOISE_DIRICHLET, NOISE_HOST, NOISE_COUNTER = 0, 1, 2, 3
 EVAL_EXTERNAL, EVAL_UNIFORM, EVAL_HASH, EVAL_ROLLOUT = 0, 1, 2, 3
@@ -85,6 +86,9 @@ SIGNATURES = {
     "az_game_replay": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, _I32P, _I32P, C.c_int32, _U64P, _I32P,
                                  _F64P, _I32P, _I32P, _VP, C.c_int32, _VP]),
     "az_observations": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, _U64P, _I32P, _VP, _VP, C.c_int32, _VP]),
+    "az_observations_reflected": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, _U64P, _I32P, _VP, _VP, _VP,
+                                            C.c_int32, _VP]),
+    "az_reflect_actions": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _I32P]),
     "az_game_random_playouts": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_uint64, C.c_int32, _I32P,
                                           _I32P, _VP]),
     "az_nn_last_error": (C.c_char_p, []),

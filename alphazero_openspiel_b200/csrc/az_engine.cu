@@ -262,6 +262,16 @@ __device__ __forceinline__ EvalKey eval_key(const Params& p, const St& s) {
   e.k = mix64(s.b0 ^ mix64(s.b1 ^ mix64(p.seed + (uint64_t)(s.ply & 1))));
   return e;
 }
+// AZ_F_REFLECT: m(s), whether the evaluator sees position s reflected (counter stream 8).  A function of the seed and the
+// position alone, so every evaluation of s -- a new evaluator row or an AZ_F_EVAL_CACHE entry -- is the same.
+__device__ __forceinline__ bool eval_reflected(const Params& p, const St& s) {
+  return (counter(p.seed, s.b0, s.b1, (uint64_t)(s.ply & 1), 0, 8) & 1ULL) != 0;
+}
+// the evaluator column of action a: R(a) for a position the evaluator saw reflected
+template <class GM>
+__device__ __forceinline__ int eval_action(const Params& p, int a, bool refl) {
+  return refl ? GM::reflect_action(a, p.geo) : a;
+}
 __device__ __forceinline__ double eval_prior(const Params& p, const StepIO& io, int tree, const EvalKey& ek, int a) {
   if (p.eval_mode == AZ_EVAL_EXTERNAL) {
     const size_t idx = (size_t)tree * p.geo.n_actions + a;
@@ -350,9 +360,11 @@ __device__ double gamma_draw(double alpha, uint64_t seed, uint64_t tree, uint64_
 }
 
 // ---------------------------------------------------------------- observation (network.py:9-18)
-template <class GM, int G>
-__device__ __forceinline__ void write_obs(const Params& p, const StepIO& io, int tree, int lane, const St& s) {
+// The planes of position s_in, or (REFLECT, AZ_F_REFLECT) those of R(s_in) when m(s_in).
+template <class GM, int G, bool REFLECT = false>
+__device__ __forceinline__ void write_obs(const Params& p, const StepIO& io, int tree, int lane, const St& s_in) {
   if (io.obs_format == AZ_OBS_NONE || io.obs == nullptr) return;
+  const St s = REFLECT && eval_reflected(p, s_in) ? GM::reflect(s_in, p.geo) : s_in;
   const int n = p.geo.cells;
   const uint64_t pl0 = GM::plane(s, p.geo, 0), pl1 = GM::plane(s, p.geo, 1), pl2 = GM::plane(s, p.geo, 2);
   const int cur = s.ply & 1;
@@ -411,12 +423,13 @@ __device__ __forceinline__ void backup_path(const Arena& a, const int32_t* path,
 
 // Node.expand (mcts.py:54-66).  noise != nullptr: root Dirichlet mix (mcts.py:186-189), eta indexed by legal position.
 // cached != nullptr: the priors come from an AZ_F_EVAL_CACHE entry (float, legal order) instead of the evaluator row.
+// refl (AZ_F_REFLECT, m(s)): the evaluator saw R(s), so the prior of action a is its output for R(a).
 // Returns false on arena overflow (nothing written).
 template <class GM, int G>
 __device__ __forceinline__ bool expand_node(const Params& p, const StepIO& io, const Arena& a, TreeHdr& h, int tree,
                                             int node, const St& s, int lane, unsigned gm, bool root_mix,
                                             const double* eta_lane /* [SLOTS] per-lane eta values */, int* L_out,
-                                            const float* cached = nullptr) {
+                                            const float* cached = nullptr, bool refl = false) {
   const typename GM::Legal lg = GM::legal(s, p.geo);
   const int L = GM::count(lg);
   *L_out = L;
@@ -433,12 +446,13 @@ __device__ __forceinline__ bool expand_node(const Params& p, const StepIO& io, c
     fresh = true;
     if (lane == 0) a.nl(node).y = ((unsigned)fc << 8) | (unsigned)L;
   }
-  const EvalKey ek = eval_key(p, s);
+  const EvalKey ek = eval_key(p, refl ? GM::reflect(s, p.geo) : s);
 #pragma unroll
   for (int sl = 0; sl < GM::SLOTS; ++sl) {
     const int i = lane + sl * G;
     if (i < L) {
-      double pr = cached ? (double)cached[i] : eval_prior(p, io, tree, ek, GM::action_of(lg, s, p.geo, i));
+      double pr = cached ? (double)cached[i]
+                         : eval_prior(p, io, tree, ek, eval_action<GM>(p, GM::action_of(lg, s, p.geo, i), refl));
       if (root_mix) pr = __dadd_rn(__dmul_rn(p.keep, pr), __dmul_rn(p.noise_w, eta_lane[sl]));
       a.p(fc + i) = pr;
       if (fresh) {
@@ -889,8 +903,8 @@ __device__ void finish_move(const Params& p, TreeHdr& h, int tree, int lane, uns
 }
 
 // expand_root_dirichlet (mcts.py:182-190): the root expansion with the noise mix, from evaluator row `row` (cached == nullptr)
-// or from an AZ_F_EVAL_CACHE entry's priors.  The noise is the tree's.  Leaves the tree in AZ_PH_RUN.
-template <class GM, int G>
+// or from an AZ_F_EVAL_CACHE entry's priors.  The noise is the tree's.  Leaves the tree in AZ_PH_RUN.  REFLECT: AZ_F_REFLECT.
+template <class GM, int G, bool REFLECT = false>
 __device__ __forceinline__ void expand_root(const Params& p, const StepIO& io, TreeHdr& h, int tree, int row, int lane,
                                             unsigned gm, unsigned long long* s_ctr, const float* cached) {
   const Arena a = arena_of(p, tree, h.half);
@@ -931,7 +945,9 @@ __device__ __forceinline__ void expand_root(const Params& p, const StepIO& io, T
     for (int sl = 0; sl < GM::SLOTS; ++sl) eta[sl] = sum > 0.0 ? eta[sl] / sum : 1.0 / (double)L;
   }
   int L2 = 0;
-  if (!expand_node<GM, G>(p, io, a, h, row, h.root_node, s, lane, gm, true, eta, &L2, cached)) arena_overflow(h, lane, s_ctr);
+  const bool refl = REFLECT && !cached && eval_reflected(p, s);
+  if (!expand_node<GM, G>(p, io, a, h, row, h.root_node, s, lane, gm, true, eta, &L2, cached, refl))
+    arena_overflow(h, lane, s_ctr);
   h.phase = AZ_PH_RUN;
   if (lane == 0) ctr_add(s_ctr, AZ_CTR_ROOT_EVALS, 1);
 }
@@ -942,7 +958,8 @@ __device__ __forceinline__ void expand_root(const Params& p, const StepIO& io, T
 // AZ_PH_ROOT_EVAL and this returns true.  CACHE: the kernel looks up the cache (k_step_vl runs without one).
 // AZ_F_PLAYOUT_CAP: a fast search (counter stream 7) runs fast_playouts simulations and starts like one without root noise.
 // FORCED (AZ_F_FORCED_PLAYOUTS): a search with root noise takes the k of az_set_forced_playouts in force now (0: not forced).
-template <class GM, int G, bool CACHE, bool FORCED = false>
+// REFLECT (AZ_F_REFLECT): the root request's planes and the root priors follow m(root).
+template <class GM, int G, bool CACHE, bool FORCED = false, bool REFLECT = false>
 __device__ __forceinline__ bool begin_search(const Params& p, const StepIO& io, TreeHdr& h, int tree, int row, int lane,
                                              unsigned gm, unsigned long long* s_ctr) {
   h.sims_done = 0;
@@ -961,26 +978,30 @@ __device__ __forceinline__ bool begin_search(const Params& p, const StepIO& io, 
   const St s = root_state(h);
   const CacheHead* hit = CACHE && p.cache ? cache_find<GM>(p, s) : nullptr;
   if (hit) {
-    expand_root<GM, G>(p, io, h, tree, row, lane, gm, s_ctr, cache_priors(hit));
+    expand_root<GM, G, REFLECT>(p, io, h, tree, row, lane, gm, s_ctr, cache_priors(hit));
     return false;
   }
   h.phase = AZ_PH_ROOT_EVAL;
   set_pend(h, s, h.root_node, 0);
-  write_obs<GM, G>(p, io, row, lane, s);
+  write_obs<GM, G, REFLECT>(p, io, row, lane, s);
   return true;
 }
 
 // Node.expand + node.update_recursive(-leaf_value) (mcts.py:146-152) of the non-terminal leaf `node` at position s, from
 // evaluator row `row` or (cached != nullptr) from the AZ_F_EVAL_CACHE entry that holds the same values.  BACKUP is backup_path,
-// or vl_backup for a path that carries a virtual loss.
-template <class GM, int G, void (*BACKUP)(const Arena&, const int32_t*, int, double, int)>
+// or vl_backup for a path that carries a virtual loss.  REFLECT (AZ_F_REFLECT): the row evaluated R(s) when m(s); its value
+// is the value of s.
+template <class GM, int G, void (*BACKUP)(const Arena&, const int32_t*, int, double, int), bool REFLECT = false>
 __device__ __forceinline__ void apply_leaf(const Params& p, const StepIO& io, const Arena& a, TreeHdr& h, int row, int node,
                                            const St& s, const int32_t* path, int depth, const CacheHead* cached, int lane,
                                            unsigned gm, unsigned long long* s_ctr, StepCtr& c) {
   int L = 0;
-  if (!expand_node<GM, G>(p, io, a, h, row, node, s, lane, gm, false, nullptr, &L, cached ? cache_priors(cached) : nullptr))
+  const bool refl = REFLECT && !cached && eval_reflected(p, s);
+  if (!expand_node<GM, G>(p, io, a, h, row, node, s, lane, gm, false, nullptr, &L, cached ? cache_priors(cached) : nullptr,
+                          refl))
     arena_overflow(h, lane, s_ctr);
-  const double v = cached ? (double)cached->value : eval_value<GM>(p, io, row, eval_key(p, s), s);
+  const double v =
+      cached ? (double)cached->value : eval_value<GM>(p, io, row, eval_key(p, refl ? GM::reflect(s, p.geo) : s), s);
   BACKUP(a, path, depth, -v, lane);
   __syncwarp(gm);
   h.sims_done += 1;
@@ -1004,8 +1025,9 @@ __device__ __forceinline__ void terminal_leaf(const Arena& a, TreeHdr& h, const 
 }
 
 // ---------------------------------------------------------------- the step kernel
-// FORCED: the instantiation of AZ_F_FORCED_PLAYOUTS engines (forced playouts in sim_select, pruning in finish_move)
-template <class GM, bool UCT, bool FORCED = false>
+// FORCED: the instantiation of AZ_F_FORCED_PLAYOUTS engines (forced playouts in sim_select, pruning in finish_move).
+// REFLECT: the instantiation of AZ_F_REFLECT engines (reflected requests and evaluator rows: write_obs, expand_node).
+template <class GM, bool UCT, bool FORCED = false, bool REFLECT = false>
 __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params p, const StepIO io) {
   constexpr int G = GM::G;
   __shared__ int32_t s_path[BLOCK / G][GM::MAXD];
@@ -1029,11 +1051,11 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
 
     // ---------------- 1. consume the evaluator outputs of the pending request
     if (h.phase == AZ_PH_LEAF_EVAL) {
-      apply_leaf<GM, G, backup_path<G>>(p, io, arena_of(p, tree, h.half), h, tree, h.pend_node, pend_state(h), gpath,
-                                        h.pend_depth, nullptr, lane, gm, s_ctr, c);
+      apply_leaf<GM, G, backup_path<G>, REFLECT>(p, io, arena_of(p, tree, h.half), h, tree, h.pend_node, pend_state(h),
+                                                 gpath, h.pend_depth, nullptr, lane, gm, s_ctr, c);
       h.phase = AZ_PH_RUN;
     } else if (h.phase == AZ_PH_ROOT_EVAL) {
-      expand_root<GM, G>(p, io, h, tree, tree, lane, gm, s_ctr, nullptr);
+      expand_root<GM, G, REFLECT>(p, io, h, tree, tree, lane, gm, s_ctr, nullptr);
     }
 
     if (p.dbg) t_consume = clock64() - t_start;
@@ -1041,7 +1063,7 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
     int sims_this_step = 0;
     bool advanced = false;
     for (;;) {
-      if (h.phase == PH_BEGIN && begin_search<GM, G, true, FORCED>(p, io, h, tree, tree, lane, gm, s_ctr)) break;
+      if (h.phase == PH_BEGIN && begin_search<GM, G, true, FORCED, REFLECT>(p, io, h, tree, tree, lane, gm, s_ctr)) break;
       if (h.phase != AZ_PH_RUN) {
         if (lane == 0) ctr_add(s_ctr, AZ_CTR_IDLE_SLOTS, 1);
         break;
@@ -1102,7 +1124,7 @@ __global__ void __launch_bounds__(BLOCK, K_STEP_MIN_BLOCKS) k_step(const Params 
       set_pend(h, s, node, depth);
       h.phase = AZ_PH_LEAF_EVAL;
       for (int j = lane; j <= depth; j += G) gpath[j] = spath[j];
-      write_obs<GM, G>(p, io, tree, lane, s);
+      write_obs<GM, G, REFLECT>(p, io, tree, lane, s);
       break;
     }
 
@@ -1143,10 +1165,11 @@ __global__ void __launch_bounds__(BLOCK) k_cache_insert(const Params p, const St
   const int L = GM::count(lg);
   float* pri = reinterpret_cast<float*>(slot + sizeof(CacheHead));
   const float* row = (const float*)io.priors + (size_t)tree * p.geo.n_actions;
+  const bool refl = (p.flags & AZ_F_REFLECT) && eval_reflected(p, s);  // the row holds the outputs of R(s): un-reflect it
 #pragma unroll
   for (int sl = 0; sl < GM::SLOTS; ++sl) {
     const int i = lane + sl * G;
-    if (i < L) pri[i] = row[GM::action_of(lg, s, p.geo, i)];
+    if (i < L) pri[i] = row[eval_action<GM>(p, GM::action_of(lg, s, p.geo, i), refl)];
   }
   if (lane == 0) {
     CacheHead e;
@@ -1195,7 +1218,7 @@ __device__ __forceinline__ void vl_backup(const Arena& a, const int32_t* path, i
   }
 }
 
-template <class GM, bool FORCED = false>
+template <class GM, bool FORCED = false, bool REFLECT = false>
 __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const StepIO io) {
   constexpr int G = GM::G;
   __shared__ int32_t s_path[BLOCK / G][GM::MAXD];
@@ -1226,20 +1249,20 @@ __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const Step
         s.ply = pe.ply;
         if (lane == 0) a.nl(pe.node).y = 0u;   // drop the in-flight marker: expand_node sees a childless node
         __syncwarp(gm);
-        apply_leaf<GM, G, vl_backup<G>>(p, io, a, h, row0 + slot, pe.node, s, gpaths + (size_t)slot * GM::MAXD, pe.depth,
-                                        nullptr, lane, gm, s_ctr, c);
+        apply_leaf<GM, G, vl_backup<G>, REFLECT>(p, io, a, h, row0 + slot, pe.node, s, gpaths + (size_t)slot * GM::MAXD,
+                                                 pe.depth, nullptr, lane, gm, s_ctr, c);
         if (lane == 0) pend[slot].valid = 0;
       }
       h.phase = AZ_PH_RUN;
     } else if (h.phase == AZ_PH_ROOT_EVAL) {
-      expand_root<GM, G>(p, io, h, tree, row0, lane, gm, s_ctr, nullptr);
+      expand_root<GM, G, REFLECT>(p, io, h, tree, row0, lane, gm, s_ctr, nullptr);
     }
 
     // ---------------- 2. collect up to K new leaves
     int n_pending = 0, sims_this_step = 0;
     bool advanced = false;
     for (;;) {
-      if (h.phase == PH_BEGIN && begin_search<GM, G, false, FORCED>(p, io, h, tree, row0, lane, gm, s_ctr)) {
+      if (h.phase == PH_BEGIN && begin_search<GM, G, false, FORCED, REFLECT>(p, io, h, tree, row0, lane, gm, s_ctr)) {
         n_pending = 1;   // (one evaluator row in use; not a leaf request)
         break;
       }
@@ -1288,7 +1311,7 @@ __global__ void __launch_bounds__(BLOCK, 4) k_step_vl(const Params p, const Step
       __syncwarp(gm);
       vl_apply<G>(a, spath, depth, lane);
       __syncwarp(gm);
-      write_obs<GM, G>(p, io, row0 + slot, lane, s);
+      write_obs<GM, G, REFLECT>(p, io, row0 + slot, lane, s);
     }
     if (h.phase == AZ_PH_RUN && n_pending > 0) h.phase = AZ_PH_LEAF_EVAL;
     if (lane == 0) {
@@ -1621,10 +1644,10 @@ __global__ void k_game_replay(const Geo geo, int n, const int32_t* hist, const i
 
 // state_to_board (network.py:9-18) for a gathered minibatch: example idx[i] (or i) of a replay buffer held as canonical
 // bitboards + ply -> observation planes in obs_format.  The trainer's minibatch builder (train.py:108-112 builds the same
-// planes from Python lists of numpy boards).
+// planes from Python lists of numpy boards).  reflect (nullable): row i holds the planes of R(example) where reflect[i] != 0.
 template <class GM>
-__global__ void k_observations(const Geo geo, int n, const uint64_t* bb, const int32_t* ply, const int64_t* idx, void* obs,
-                               int obs_format) {
+__global__ void k_observations(const Geo geo, int n, const uint64_t* bb, const int32_t* ply, const int64_t* idx,
+                               const uint8_t* reflect, void* obs, int obs_format) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const long long src = idx ? idx[i] : (long long)i;
@@ -1632,6 +1655,7 @@ __global__ void k_observations(const Geo geo, int n, const uint64_t* bb, const i
   s.b0 = bb[2 * src];
   s.b1 = bb[2 * src + 1];
   s.ply = ply[src];
+  if (reflect && reflect[i]) s = GM::reflect(s, geo);
   Params p;
   p.geo = geo;
   StepIO io;
@@ -1781,6 +1805,12 @@ int az_create(const az_config* cfg_in, az_engine** out) {
     return fail(-1, "AZ_F_FORCED_PLAYOUTS is a PUCT rule: AZ_F_UCT scores with the use_puct=False formula");
   if ((cfg.flags & AZ_F_FORCED_PLAYOUTS) && cfg.noise_mode == AZ_NOISE_NONE)
     return fail(-1, "AZ_F_FORCED_PLAYOUTS forces only searches with root noise: AZ_NOISE_NONE has none");
+  if ((cfg.flags & AZ_F_REFLECT) && (cfg.flags & AZ_F_MANUAL))
+    return fail(-1, "AZ_F_REFLECT is a batched self-play mode: with AZ_F_MANUAL a host policy_fn evaluates states, not planes");
+  if ((cfg.flags & AZ_F_REFLECT) && (cfg.flags & AZ_F_UCT))
+    return fail(-1, "AZ_F_REFLECT is a PUCT self-play mode: AZ_F_UCT is the search of the reference's MCTS bot");
+  if ((cfg.flags & AZ_F_REFLECT) && cfg.eval_mode == AZ_EVAL_ROLLOUT)
+    return fail(-1, "AZ_F_REFLECT reflects network evaluations: AZ_EVAL_ROLLOUT is no network");
   if (cfg.record_capacity <= 0) cfg.record_capacity = cfg.n_trees * 64 < (1 << 20) ? (1 << 20) : cfg.n_trees * 64;
   if (!(cfg.flags & AZ_F_RECORDS)) cfg.record_capacity = 1;
   if (cfg.flags & AZ_F_EVAL_CACHE) {
@@ -2060,7 +2090,16 @@ int az_step(az_engine* e, const void* priors_dev, const void* values_dev, const 
     if (p.cache && priors_dev) k_cache_insert<GM><<<groups_grid(p.n_trees, GM::G, BLOCK), BLOCK, 0, st>>>(p, io);
     const dim3 grid = groups_grid(p.n_trees, GM::G, BLOCK);
     const bool forced = (p.flags & AZ_F_FORCED_PLAYOUTS) != 0;
-    if (p.flags & AZ_F_VIRTUAL_LOSS) {
+    if (p.flags & AZ_F_REFLECT) {  // (not with AZ_F_UCT: az_create)
+      if (p.flags & AZ_F_VIRTUAL_LOSS) {
+        if (forced) k_step_vl<GM, true, true><<<grid, BLOCK, 0, st>>>(p, io);
+        else k_step_vl<GM, false, true><<<grid, BLOCK, 0, st>>>(p, io);
+      } else if (forced) {
+        k_step<GM, false, true, true><<<grid, BLOCK, 0, st>>>(p, io);
+      } else {
+        k_step<GM, false, false, true><<<grid, BLOCK, 0, st>>>(p, io);
+      }
+    } else if (p.flags & AZ_F_VIRTUAL_LOSS) {
       if (forced) k_step_vl<GM, true><<<grid, BLOCK, 0, st>>>(p, io);
       else k_step_vl<GM><<<grid, BLOCK, 0, st>>>(p, io);
     } else if (p.flags & AZ_F_UCT) {
@@ -2233,19 +2272,37 @@ int az_game_replay(int32_t game_id, int32_t rows, int32_t cols, int32_t n, const
   return 0;
 }
 
-int az_observations(int32_t game_id, int32_t rows, int32_t cols, int32_t n, const uint64_t* bb_dev, const int32_t* ply_dev,
-                    const int64_t* idx_dev, void* obs_dev, int32_t obs_format, void* stream) {
+int az_observations_reflected(int32_t game_id, int32_t rows, int32_t cols, int32_t n, const uint64_t* bb_dev,
+                              const int32_t* ply_dev, const int64_t* idx_dev, const uint8_t* reflect_dev, void* obs_dev,
+                              int32_t obs_format, void* stream) {
   if (check_game(game_id, rows, cols)) return -1;
   if (n <= 0) return 0;
   if (!bb_dev || !ply_dev || !obs_dev || obs_format < 1 || obs_format > 2) return fail(-1, "az_observations: bad argument");
   const Geo geo = make_geo(game_id, rows, cols);
   dispatch_game(game_id, [&](auto gm) {
     using GM = decltype(gm);
-    k_observations<GM><<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(geo, n, bb_dev, ply_dev, idx_dev, obs_dev, obs_format);
+    k_observations<GM><<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(geo, n, bb_dev, ply_dev, idx_dev, reflect_dev,
+                                                                         obs_dev, obs_format);
     return 0;
   });
   CK(cudaGetLastError());
   return 0;
+}
+
+int az_observations(int32_t game_id, int32_t rows, int32_t cols, int32_t n, const uint64_t* bb_dev, const int32_t* ply_dev,
+                    const int64_t* idx_dev, void* obs_dev, int32_t obs_format, void* stream) {
+  return az_observations_reflected(game_id, rows, cols, n, bb_dev, ply_dev, idx_dev, nullptr, obs_dev, obs_format, stream);
+}
+
+int az_reflect_actions(int32_t game_id, int32_t rows, int32_t cols, int32_t* perm_host) {
+  if (check_game(game_id, rows, cols)) return -1;
+  if (!perm_host) return fail(-1, "az_reflect_actions: null perm_host");
+  const Geo geo = make_geo(game_id, rows, cols);
+  return dispatch_game(game_id, [&](auto gm) {
+    using GM = decltype(gm);
+    for (int a = 0; a < geo.n_actions; ++a) perm_host[a] = GM::reflect_action(a, geo);
+    return 0;
+  });
 }
 
 int az_game_random_playouts(int32_t game_id, int32_t rows, int32_t cols, int32_t n, uint64_t seed, int32_t max_plies,

@@ -43,6 +43,20 @@ __device__ __forceinline__ uint64_t counter(uint64_t seed, uint64_t tree, uint64
   return x;
 }
 
+// Left-right reflection of a cell mask: column c <-> column cols-1-c, rows unchanged.  Both games are symmetric under it
+// (AZ_F_REFLECT); the host uses the same code (az_reflect_actions, tests).
+__host__ __device__ __forceinline__ uint64_t mirror_columns(uint64_t x, const Geo& g) {
+  const uint64_t col0 = g.all & ~g.notcol0;
+  uint64_t y = 0;
+  for (int c = 0; c < g.cols; ++c) y |= ((x >> c) & col0) << (g.cols - 1 - c);
+  return y;
+}
+__host__ __device__ __forceinline__ St mirror_state(St s, const Geo& g) {
+  s.b0 = mirror_columns(s.b0, g);
+  s.b1 = mirror_columns(s.b1, g);
+  return s;
+}
+
 // ------------------------------------------------------------------------------------------------
 // Connect Four: 6 rows x 7 columns, action = column, row 0 = bottom (SURVEY B.2).
 // ------------------------------------------------------------------------------------------------
@@ -104,6 +118,9 @@ struct C4 {
   static __device__ __forceinline__ uint64_t plane(const St& s, const Geo& g, int ch) {
     return ch == 0 ? (~(s.b0 | s.b1) & g.all) : (ch == 1 ? s.b1 : s.b0);
   }
+  // left-right reflection R(s) and the action map R(a): column a <-> 6 - a
+  static __host__ __device__ __forceinline__ St reflect(const St& s, const Geo& g) { return mirror_state(s, g); }
+  static __host__ __device__ __forceinline__ int reflect_action(int a, const Geo& g) { return g.cols - 1 - a; }
   static __device__ __forceinline__ St initial(const Geo&) {
     St s;
     s.b0 = s.b1 = 0;
@@ -206,6 +223,15 @@ struct BT {
   // planes: black (player 0), white (player 1), empty
   static __device__ __forceinline__ uint64_t plane(const St& s, const Geo& g, int ch) {
     return ch == 0 ? s.b0 : (ch == 1 ? s.b1 : (~(s.b0 | s.b1) & g.all));
+  }
+  // left-right reflection R(s) and the action map R(a): the move from (r, c) with column step dcol <-> the move from
+  // (r, cols-1-c) with step -dcol (d3 <-> 2 - d3), same player, same capture bit
+  static __host__ __device__ __forceinline__ St reflect(const St& s, const Geo& g) { return mirror_state(s, g); }
+  static __host__ __device__ __forceinline__ int reflect_action(int a, const Geo& g) {
+    const int dir = (a >> 1) % 6, cell = (a >> 1) / 6;
+    const int r = cell / g.cols, c = cell - r * g.cols;
+    const int d3 = dir % 3, pl = dir / 3;
+    return ((r * g.cols + g.cols - 1 - c) * 6 + (2 - d3) + 3 * pl) * 2 + (a & 1);
   }
   static __device__ __forceinline__ St initial(const Geo& g) {
     St s;

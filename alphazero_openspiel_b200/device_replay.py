@@ -16,7 +16,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from .engine import parse_game_name
+from .engine import parse_game_name, reflect_actions
 
 
 def key_hash(batch):
@@ -46,6 +46,7 @@ class DeviceReplay:
         self.lib = L.load()
         self.game_ptr = np.zeros(1, np.int64)        # host: examples of game g are rows game_ptr[g] : game_ptr[g+1]
         self.bb = self.ply = self.key = self.policy = self.value = None
+        self._reflect_perm = None
 
     def __len__(self):
         return 0 if self.bb is None else int(self.bb.shape[0])
@@ -114,15 +115,27 @@ class DeviceReplay:
         self.value[first] = val
         return first, pol, val
 
+    @property
+    def reflect_perm(self):
+        """The action reflection (engine.reflect_actions) as a device index tensor: a reflected policy row is p[:, perm]."""
+        if self._reflect_perm is None:
+            self._reflect_perm = torch.from_numpy(reflect_actions(self.game_name)).to(self.device)
+        return self._reflect_perm
+
     @torch.no_grad()
-    def boards(self, ids):
+    def boards(self, ids, reflect=None):
         """state_to_board planes (network.py:9-18) of examples `ids` (int64 device tensor): float32 [n, 4, rows, cols],
-        gathered and encoded by the az_observations kernel."""
+        gathered and encoded by the az_observations kernel.  reflect (uint8 / bool device tensor [n], optional): rows where
+        it is set hold the planes of the left-right reflected position (columns flipped)."""
         ids = ids.to(self.device, torch.int64).contiguous()
         n = int(ids.numel())
+        if reflect is not None:
+            reflect = reflect.to(self.device, torch.uint8).contiguous()
+            assert reflect.numel() == n
         out = torch.empty((n, 4, self.rows, self.cols), dtype=torch.float32, device=self.device)
         st = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        L.check(self.lib.az_observations(self.game_id, self.rows, self.cols, n, C.c_void_p(self.bb.data_ptr()),
-                                         C.c_void_p(self.ply.data_ptr()), C.c_void_p(ids.data_ptr()),
-                                         C.c_void_p(out.data_ptr()), L.OBS_F32_NCHW, st))
+        L.check(self.lib.az_observations_reflected(self.game_id, self.rows, self.cols, n, C.c_void_p(self.bb.data_ptr()),
+                                                   C.c_void_p(self.ply.data_ptr()), C.c_void_p(ids.data_ptr()),
+                                                   None if reflect is None else C.c_void_p(reflect.data_ptr()),
+                                                   C.c_void_p(out.data_ptr()), L.OBS_F32_NCHW, st))
         return out

@@ -253,6 +253,16 @@ class Engine:
         return {k: int(v) for k, v in zip(L.CTR_NAMES, out)}
 
 
+def reflect_actions(game_name):
+    """The left-right reflection of the game's actions (az_reflect_actions, F_REFLECT's R): int64 [num_distinct_actions],
+    perm[a] = R(a).  A reflected policy target is p[perm]; an involution.  Host only."""
+    lib = L.load()
+    gid, rows, cols = parse_game_name(game_name)
+    perm = np.zeros(game_shape(game_name)[1], dtype=np.int32)
+    L.check(lib.az_reflect_actions(gid, rows, cols, perm.ctypes.data))
+    return perm.astype(np.int64)
+
+
 def game_replay(game_name, histories, obs_format=L.OBS_F32_NCHW, device=0):
     """Stateless batched game ops (parity tests): replay histories on the device."""
     lib = L.load()

@@ -178,7 +178,7 @@ class SelfPlayRunner:
                  max_sims_per_step=16, records=True, use_graph=True, noise_mode=None, node_capacity=0,
                  record_capacity=0, evaluator="fused", virtual_loss=0, step_cycle_budget=None, eval_cache=None,
                  eval_cache_log2=0, resign_threshold=None, resign_disabled_fraction=0.1, fast_playouts=None,
-                 full_search_fraction=0.25, forced_playouts=None, **_ignored):
+                 full_search_fraction=0.25, forced_playouts=None, reflect_evaluations=False, **_ignored):
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise L.EngineUnavailable("SelfPlayRunner needs a CUDA device; there is no CPU fallback")
@@ -207,6 +207,10 @@ class SelfPlayRunner:
             # child of a search with root noise gets at least sqrt(k * P * N) visits, and the visits it got only from that
             # floor are taken out of the policy target and the move choice
             flags |= L.F_FORCED_PLAYOUTS
+        if reflect_evaluations:
+            # left-right reflection of the evaluations (an extension the reference does not have): the network sees the
+            # mirrored board of a position chosen by a hash of the seed and the position, and its policy is mapped back
+            flags |= L.F_REFLECT
         if noise_mode is None:
             noise_mode = L.NOISE_DIRICHLET if use_dirichlet else L.NOISE_NONE
         # virtual_loss = K > 0: K leaves in flight per tree (AZ_F_VIRTUAL_LOSS, NOT bit-exact with the reference), for pools

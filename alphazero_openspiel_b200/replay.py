@@ -16,6 +16,23 @@ from .engine import parse_game_name
 from .examplegenerator import boards_from_bitboards, policy_targets_batch
 
 
+def _mix64(x):
+    """splitmix64 finaliser (csrc/az_games.cuh mix64) on uint64 arrays."""
+    x = x + np.uint64(0x9E3779B97F4A7C15)
+    x = (x ^ (x >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+    x = (x ^ (x >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+    return x ^ (x >> np.uint64(31))
+
+
+def reflect_bits(step, n):
+    """Trainer(reflect_minibatches=True): example j of optimisation step `step` is reflected iff the top bit of
+    mix64(mix64(step) + j) is set -> bool [n].  Stateless, so it draws nothing from numpy's global RNG and the sample ids
+    stay those of the reference."""
+    with np.errstate(over="ignore"):
+        h = _mix64(_mix64(np.full(1, step, dtype=np.uint64)) + np.arange(n, dtype=np.uint64))
+    return (h >> np.uint64(63)).astype(bool)
+
+
 class ExampleBatch:
     """Examples of whole games, game after game, ply after ply.
 

@@ -18,9 +18,10 @@ import torch
 import torch.nn as nn
 
 from . import parallel
-from .engine import game_shape
+from .engine import game_shape, reflect_actions
 from .examplegenerator import ExampleGenerator
 from .network import Net
+from .replay import reflect_bits
 
 logger = logging.getLogger("alphazero")
 
@@ -86,6 +87,12 @@ class Trainer:
         # forced_playouts = k (2.0 in the paper), every visited root child of a search with root noise gets at least
         # sqrt(k * P * N) visits, and the visits it got only from that floor are pruned from its policy target.
         self.forced_playouts = None
+        # Extension: left-right reflection, the one symmetry of both games (AlphaGo Zero; the reference uses every position
+        # as it is).  With reflect_evaluations, self-play evaluates a position mirrored (column c <-> cols-1-c) when a hash of
+        # the engine seed and the position says so, and maps the policy back.  With reflect_minibatches, every sampled
+        # training example is mirrored, board planes and policy target, when a hash of (optimisation step, row) says so.
+        self.reflect_evaluations = False
+        self.reflect_minibatches = False
         for k, v in overrides.items():
             if not hasattr(self, k):
                 raise TypeError("unknown Trainer setting %r" % k)
@@ -111,19 +118,35 @@ class Trainer:
                                           capturable=bool(self.graph_step and self.device.type == "cuda"))
         self._step_graph = None
         self._gids = None
+        self._perm = None
         self.criterion_value = nn.MSELoss()
         self.current_net.eval()
         self.last_generation_stats = {}
 
     # ------------------------------------------------------------------ optimisation (train.py:95-154)
+    def _reflect_rows(self):
+        """reflect_minibatches: the minibatch rows of this optimisation step (self.it) to mirror, bool [batch_size] (for
+        the whole minibatch: ddp slices it like the sample ids); None when off."""
+        return reflect_bits(self.it, self.batch_size) if self.reflect_minibatches else None
+
+    def _host_perm(self):
+        if self._perm is None:
+            self._perm = reflect_actions(self.name_game)
+        return self._perm
+
     def net_step_arrays(self, batch, first, pol, val):
         """net_step on the array form of the buffer (replay.ExampleBatch after remove_duplicates): same sampling call,
         same losses; the board planes are rebuilt for the sampled minibatch only."""
         self.current_net.zero_grad()
         sample_ids = np.random.randint(len(first), size=self.batch_size)
-        x = torch.from_numpy(batch.boards(first[sample_ids])).float().to(self.device)
+        boards, p = batch.boards(first[sample_ids]), pol[sample_ids]
+        refl = self._reflect_rows()
+        if refl is not None:
+            boards[refl] = boards[refl][..., ::-1]
+            p[refl] = p[refl][:, self._host_perm()]
+        x = torch.from_numpy(boards).float().to(self.device)
         p_t, v_t = self.current_net(x)
-        p_r = torch.tensor(pol[sample_ids]).float().to(self.device)
+        p_r = torch.tensor(p).float().to(self.device)
         v_r = torch.tensor(val[sample_ids]).float().to(self.device)
         loss_v = self.criterion_value(v_t, v_r.unsqueeze(1))
         loss_p = -torch.sum(p_r * torch.log(p_t)) / p_r.size()[0]
@@ -137,16 +160,21 @@ class Trainer:
         of the sampled examples come from the az_observations gather kernel, targets are gathered on the device; with
         `ddp` every rank trains on its slice of the minibatch and the gradients are averaged over NCCL."""
         sample_ids = np.random.randint(int(first.numel()), size=self.batch_size)
+        refl = self._reflect_rows()
         rank, world = parallel.rank_world()
         if self.graph_step and not (self.ddp and world > 1):
-            return self._net_step_graphed(replay, first, pol, val, sample_ids)
+            return self._net_step_graphed(replay, first, pol, val, sample_ids, refl)
         self.current_net.zero_grad()
         if self.ddp and world > 1:
             sample_ids = sample_ids[rank::world]
+            refl = None if refl is None else refl[rank::world]
         ids = torch.from_numpy(sample_ids).to(self.device)
-        x = replay.boards(first[ids])
+        refl = None if refl is None else torch.from_numpy(refl).to(self.device)
+        x = replay.boards(first[ids], refl)
         p_t, v_t = self.current_net(x)
         p_r = pol[ids].float()
+        if refl is not None:
+            p_r = torch.where(refl[:, None], p_r[:, replay.reflect_perm], p_r)
         v_r = val[ids].float()
         loss_v = self.criterion_value(v_t, v_r.unsqueeze(1))
         loss_p = -torch.sum(p_r * torch.log(p_t)) / p_r.size()[0]
@@ -157,23 +185,35 @@ class Trainer:
         self.it += 1
         return loss_p, loss_v
 
-    def _net_step_graphed(self, replay, first, pol, val, sample_ids):
+    def _net_step_graphed(self, replay, first, pol, val, sample_ids, refl=None):
         """The device step as ONE CUDA-graph replay: minibatch gather (az_observations kernel + two index_selects from the
         de-duplicated targets), forward, MSE + cross-entropy, backward, Adam.  Per step the host only draws the sample ids
         (the reference's np.random.randint call) and copies 2 KB of indices to the device; the graph is re-captured
-        when a new generation brings new target tensors."""
+        when a new generation brings new target tensors.  refl (reflect_minibatches): the rows to mirror travel as bit 32
+        of the same indices (the ids are below 2^31)."""
         dev = self.device
         if getattr(self, "_gids", None) is None:
             self._gids = torch.zeros(self.batch_size, dtype=torch.int64, device=dev)
             self._graph_key = None
             self._graph_warm = False
+        gids = np.ascontiguousarray(sample_ids, dtype=np.int64)
+        perm = None
+        if refl is not None:
+            gids = gids | (refl.astype(np.int64) << 32)
+            perm = replay.reflect_perm         # (built here: no host-to-device copy inside the capture)
         # (pageable source: the driver stages the 2 KB before returning, so the next step may overwrite sample_ids)
-        self._gids.copy_(torch.from_numpy(np.ascontiguousarray(sample_ids, dtype=np.int64)))
+        self._gids.copy_(torch.from_numpy(gids))
 
         def step():
             ids = self._gids
-            x = replay.boards(first[ids])
+            rows = None
+            if perm is not None:
+                rows = (ids >> 32).to(torch.uint8)
+                ids = ids & 0xFFFFFFFF
+            x = replay.boards(first[ids], rows)
             p_r = pol[ids].float()
+            if perm is not None:
+                p_r = torch.where(rows[:, None].bool(), p_r[:, perm], p_r)
             v_r = val[ids].float().unsqueeze(1)
             self.optimizer.zero_grad(set_to_none=False)
             p_t, v_t = self.current_net(x)
@@ -195,7 +235,8 @@ class Trainer:
             self._graph_warm = True
             self.it += 1
             return out[0].clone(), out[1].clone()
-        key = (first.data_ptr(), pol.data_ptr(), val.data_ptr(), int(first.numel()), replay.bb.data_ptr())
+        key = (first.data_ptr(), pol.data_ptr(), val.data_ptr(), int(first.numel()), replay.bb.data_ptr(),
+               perm is not None)
         if key != self._graph_key:
             torch.cuda.current_stream(dev).synchronize()
             self._step_graph = torch.cuda.CUDAGraph()
@@ -212,6 +253,12 @@ class Trainer:
         boards = [flattened_buffer[i][1] for i in sample_ids]
         pol = [flattened_buffer[i][2] for i in sample_ids]
         val = [flattened_buffer[i][3] for i in sample_ids]
+        refl = self._reflect_rows()
+        if refl is not None:
+            # an empty policy is replaced below by the network's output, which already refers to the mirrored input
+            perm = self._host_perm()
+            boards = [b[..., ::-1] if r else b for b, r in zip(boards, refl)]
+            pol = [np.asarray(item)[perm].tolist() if (r and item) else item for item, r in zip(pol, refl)]
         x = torch.from_numpy(np.array(boards)).float().to(self.device)
         p_t, v_t = self.current_net(x)
         pol = [item if item else p_t[i, :].to("cpu").tolist() for i, item in enumerate(pol)]
@@ -295,6 +342,8 @@ class Trainer:
                                  full_search_fraction=self.full_search_fraction)
         if self.forced_playouts is not None:
             engine_kwargs = dict(engine_kwargs, forced_playouts=self.forced_playouts)
+        if self.reflect_evaluations:
+            engine_kwargs = dict(engine_kwargs, reflect_evaluations=True)
         generator = ExampleGenerator(self.current_net, self.name_game, self.device,
                                      n_playouts=self.n_playouts_train, temperature=self.temperature,
                                      dirichlet_ratio=self.dirichlet_ratio, c_puct=self.uct_train, backup=self.backup,

@@ -38,7 +38,9 @@
  *   3 = random start plies, 4 = number of random start plies, 5 = device Dirichlet gammas,
  *   6 = no-resign calibration games (AZ_F_RESIGN: counter(seed,tree,game_seq,0,0,6) % 1000 < disabled_permille),
  *   7 = fast searches (AZ_F_PLAYOUT_CAP: the search at root ply `ply` is fast iff
- *       counter(seed,tree,game_seq,ply,0,7) % 1000 >= full_permille).
+ *       counter(seed,tree,game_seq,ply,0,7) % 1000 >= full_permille),
+ *   8 = reflected evaluations (AZ_F_REFLECT: position (b0, b1, ply) is evaluated reflected iff
+ *       counter(seed,b0,b1,ply & 1,0,8) & 1).
  */
 #ifndef AZ_B200_H
 #define AZ_B200_H
@@ -117,6 +119,19 @@ extern "C" {
                                           ply record's counts (root_n stays the raw visit count); root_q, v_a0c, v_offpolicy,
                                           resignation and tree reuse see the tree as it is.  k: az_set_forced_playouts (0 after
                                           az_create).  Not with AZ_F_MANUAL, AZ_F_UCT or AZ_NOISE_NONE */
+#define AZ_F_REFLECT        (1u << 16) /* left-right reflection of the network evaluations (AlphaGo Zero; an extension: the
+                                          reference evaluates every position as it is).  R(s) mirrors the columns of both
+                                          bitboards (column c <-> cols-1-c; ply unchanged), R(a) is the action map
+                                          (az_reflect_actions: Connect Four a <-> 6-a; Breakthrough the move from (r, c) with
+                                          column step d <-> the move from (r, cols-1-c) with step -d, same capture bit).  A
+                                          position s is evaluated reflected iff m(s) = counter stream 8 & 1 (see above): a
+                                          function of the seed and the position alone.  Then the observation row of its request
+                                          (root or leaf, every obs_format) holds the planes of R(s), the prior of child action a
+                                          is read from evaluator column R(a) and the value is read as it is; AZ_EVAL_HASH
+                                          evaluates R(s) the same way (prior of a = its prior of (R(s), R(a))).  AZ_F_EVAL_CACHE
+                                          stores the priors of s (un-reflected), so it stays exact.  Children, ply records,
+                                          counts, values, az_request_info and az_positions are those of the true position.  Not
+                                          with AZ_F_MANUAL, AZ_F_UCT or AZ_EVAL_ROLLOUT */
 #define AZ_EVAL_CACHE_LOG2_SHIFT 24
 #define AZ_EVAL_CACHE_LOG2(flags) (((flags) >> AZ_EVAL_CACHE_LOG2_SHIFT) & 31u)
 #define AZ_EVAL_CACHE_EXTRA_LOG2 1
@@ -337,6 +352,16 @@ int az_game_replay(int32_t game_id, int32_t rows, int32_t cols, int32_t n, const
  * (int64; NULL = example i).  The trainer's minibatch builder (train.py:108-112). */
 int az_observations(int32_t game_id, int32_t rows, int32_t cols, int32_t n, const uint64_t* bb_dev, const int32_t* ply_dev,
                     const int64_t* idx_dev, void* obs_dev, int32_t obs_format, void* stream);
+
+/* az_observations with a per-row reflection (training minibatches, AZ_F_REFLECT's R): row i holds the planes of R(example
+ * idx_dev[i]) where reflect_dev[i] != 0 (uint8 [n], device).  reflect_dev == NULL gives exactly az_observations. */
+int az_observations_reflected(int32_t game_id, int32_t rows, int32_t cols, int32_t n, const uint64_t* bb_dev,
+                              const int32_t* ply_dev, const int64_t* idx_dev, const uint8_t* reflect_dev, void* obs_dev,
+                              int32_t obs_format, void* stream);
+
+/* AZ_F_REFLECT's action map of a game: perm_host[a] = R(a) for every a < num_distinct_actions (host int32 array); an
+ * involution.  Host only: needs no device. */
+int az_reflect_actions(int32_t game_id, int32_t rows, int32_t cols, int32_t* perm_host);
 
 /* Random playouts entirely on the device from counter stream 3 (seed, i): plays up to max_plies uniformly
  * random legal moves per game and writes the action history (hist_dev [n][max_plies], len_dev [n]).  Used to
