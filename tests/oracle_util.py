@@ -21,7 +21,8 @@ def selfplay_cfg(game_name, n_playouts, c_puct=2.5, dirichlet_ratio=0.25, use_di
 
 
 def selfplay_game(cfg, tree, game_seq=0, max_out=512):
-    """-> (list of ply dicts, returns[2], counters[8])"""
+    """-> (list of ply dicts, returns[2], counters[8]); a ply dict's end is the engine ply record's, 0: the C oracle runs
+    no fast searches"""
     lib = cbind.lib()
     recs = (cbind.OzPlyRecord * max_out)()
     ret = (C.c_double * 2)()
@@ -33,7 +34,7 @@ def selfplay_game(cfg, tree, game_seq=0, max_out=512):
         r = recs[i]
         out.append({"ply": r.ply, "action": r.action, "n_legal": r.n_legal, "bb": (int(r.bb[0]), int(r.bb[1])),
                     "root_q": r.root_q, "root_n": int(r.root_n), "v_a0c": r.v_a0c, "v_offpolicy": r.v_offpolicy,
-                    "counts": list(r.counts[:r.n_legal])})
+                    "counts": list(r.counts[:r.n_legal]), "end": 0})
     return out, [ret[0], ret[1]], list(ctr)
 
 

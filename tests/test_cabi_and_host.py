@@ -124,35 +124,12 @@ def test_remove_illegal_actions_and_policy_target_follow_the_reference_expressio
 
 def test_records_to_games_from_oracle_records():
     """Device record format -> reference example format, checked with records synthesised from the oracle."""
-    from alphazero_openspiel_b200.engine import record_dtype
     from alphazero_openspiel_b200.examplegenerator import records_to_games
-    from tests import oracle_util as ou
+    from tests import oracle_util as ou, selfplay_rule as sr
     game = "connect_four"
     cfg = ou.selfplay_cfg(game, 25, use_dirichlet=2, sample_moves=1, seed=3)
-    dt = record_dtype(7, (72 + 6 * 7 + 7) // 8 * 8)
-    rows = []
-    expect = []
-    for t in range(3):
-        plies, ret, _ = ou.selfplay_game(cfg, t)
-        hist = []
-        for r in plies:
-            rec = np.zeros((), dtype=dt)
-            rec["tree"], rec["game_seq"], rec["ply"], rec["action"] = t, 0, r["ply"], r["action"]
-            rec["n_legal"], rec["kind"], rec["root_n"] = r["n_legal"], 0, r["root_n"]
-            rec["bb"] = r["bb"]
-            rec["root_q"], rec["v_a0c"], rec["v_offpolicy"] = r["root_q"], r["v_a0c"], r["v_offpolicy"]
-            legal = ou.replay(game, hist)["legal"]
-            rec["counts"][:r["n_legal"]] = r["counts"]
-            rec["actions"][:] = -1
-            rec["actions"][:r["n_legal"]] = legal
-            rows.append(rec)
-            hist.append(r["action"])
-        end = np.zeros((), dtype=dt)
-        end["tree"], end["kind"], end["ply"], end["root_q"] = t, 1, len(plies), ret[0]
-        rows.append(end)
-        expect.append((plies, ret))
-    recs = np.array(rows, dtype=dt)
-    recs = recs[np.random.RandomState(0).permutation(len(recs))]  # arrival order is arbitrary
+    expect = [ou.selfplay_game(cfg, t)[:2] for t in range(3)]
+    recs = sr.records(game, [(t, plies, ret, 0) for t, (plies, ret) in enumerate(expect)], shuffle_seed=0)
     for backup in ["on-policy", "soft-Z", "A0C", "off-policy"]:
         games = records_to_games(recs, game, backup)
         assert len(games) == 3

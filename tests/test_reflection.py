@@ -1,83 +1,16 @@
 """Left-right reflection (AZ_F_REFLECT in self-play, Trainer(reflect_minibatches=True) in training): the game symmetry on the
-oracle's games, the training minibatch rule on the host, and on the GPU the engine against a restatement on the reference
-port's search, the evaluator rows, the eval cache, the gather kernel and the Trainer paths."""
+oracle's games, the training minibatch rule on the host, and on the GPU the engine against the restatement of
+tests/selfplay_rule.py, the evaluator rows, the eval cache, the gather kernel and the Trainer paths."""
 import ctypes as C
 
 import numpy as np
 import pytest
 
 from tests import oracle_util as ou
-from tests import test_forced_playouts as fp
-from tests import test_playout_cap as pc
-from tests.test_trainer import _oracle_records
+from tests import selfplay_rule as sr
+from tests.selfplay_rule import BT6, BT8, C4
 
-C4 = "connect_four"
-BT6 = "breakthrough(rows=6,columns=6)"
-BT8 = "breakthrough"
 GAMES = [C4, BT6, BT8]
-
-
-def _mirror(x, rows, cols):
-    """R on a cell mask: column c <-> cols-1-c."""
-    y = 0
-    for r in range(rows):
-        for c in range(cols):
-            if (x >> (r * cols + c)) & 1:
-                y |= 1 << (r * cols + cols - 1 - c)
-    return y
-
-
-def _reflect_action(a, game_id, cols):
-    """R on actions, written out from the games' encodings (include/az_b200.h, AZ_F_REFLECT)."""
-    if game_id == 0:
-        return 6 - a
-    cap, d, cell = a & 1, (a >> 1) % 6, (a >> 1) // 6
-    r, c = divmod(cell, cols)
-    return ((r * cols + cols - 1 - c) * 6 + (2 - d % 3) + 3 * (d // 3)) * 2 + cap
-
-
-def _m(seed, b0, b1, ply):
-    """m(s): position (b0, b1, ply) is evaluated reflected (counter stream 8)."""
-    from oracle import cbind
-    return bool(cbind.lib().oz_counter(seed, b0, b1, ply & 1, 0, 8) & 1)
-
-
-class _ReflectingOracle:
-    """The oracle library with its hash evaluator (oz_synth_eval) answering for R(s) whenever m(s): priors of a = the
-    outputs of oz_synth_eval_bb on the mirrored bitboards at R(a), value as is.  Everything else is the oracle's."""
-
-    def __init__(self, lib):
-        self._lib = lib
-
-    def __getattr__(self, name):
-        return getattr(self._lib, name)
-
-    def oz_synth_eval(self, state_ref, kind, seed, shift, priors, value):
-        st = state_ref._obj
-        bb = (C.c_uint64 * 2)()
-        self._lib.oz_bitboards(C.byref(st), bb)
-        b0, b1 = int(bb[0]), int(bb[1])
-        if not _m(seed, b0, b1, st.ply):
-            return self._lib.oz_synth_eval(state_ref, kind, seed, shift, priors, value)
-        n_actions = len(priors)
-        rbb = np.array([_mirror(b0, st.rows, st.cols), _mirror(b1, st.rows, st.cols)], dtype=np.uint64)
-        ply = np.array([st.ply], dtype=np.int32)
-        pri, val = np.zeros(n_actions, np.float32), np.zeros(1, np.float32)
-        self._lib.oz_synth_eval_bb(n_actions, 1, rbb.ctypes.data, ply.ctypes.data, kind, seed, shift, pri.ctypes.data,
-                                   val.ctypes.data)
-        for a in range(n_actions):
-            priors[a] = float(pri[_reflect_action(a, st.game, st.cols)])
-        value._obj.value = float(val[0])
-
-
-@pytest.fixture
-def reflected_oracle(monkeypatch):
-    """The restatements of tests/test_playout_cap and tests/test_forced_playouts (the C oracle's counter-mode self-play on
-    the reference port's search, with playout cap, forced playouts and resignation) with the reflecting evaluator."""
-    from oracle import cbind
-    wrapped = _ReflectingOracle(cbind.lib())
-    monkeypatch.setattr(cbind, "lib", lambda: wrapped)
-    return wrapped
 
 
 def _random_histories(game, n, seed):
@@ -105,7 +38,7 @@ def test_reflect_actions_is_the_involution_of_the_rule(game):
     perm = reflect_actions(game)
     assert len(perm) == game_shape(game)[1]
     assert np.array_equal(perm[perm], np.arange(len(perm)))
-    assert list(perm) == [_reflect_action(a, gid, cols) for a in range(len(perm))]
+    assert list(perm) == [sr.reflect_action(a, gid, cols) for a in range(len(perm))]
     assert (perm != np.arange(len(perm))).sum() > len(perm) // 2
     lib = L.load()
     out = np.zeros(len(perm), np.int32)
@@ -132,7 +65,7 @@ def test_reflection_is_a_symmetry_of_the_game(game):
             s.apply_action(a)
             rs.apply_action(int(perm[a]))
             b0, b1 = s.bitboards()
-            assert rs.bitboards() == (_mirror(b0, rows, cols), _mirror(b1, rows, cols))
+            assert rs.bitboards() == (sr.mirror(b0, rows, cols), sr.mirror(b1, rows, cols))
         assert sorted(rs.legal_actions()) == sorted(int(perm[a]) for a in s.legal_actions())
         assert rs.is_terminal() == s.is_terminal() and rs.returns() == s.returns()
         n_terminal += s.is_terminal()
@@ -140,7 +73,7 @@ def test_reflection_is_a_symmetry_of_the_game(game):
             t, rt = s.clone(), rs.clone()
             t.apply_action(a)
             rt.apply_action(int(perm[a]))
-            assert rt.bitboards() == tuple(_mirror(x, rows, cols) for x in t.bitboards())
+            assert rt.bitboards() == tuple(sr.mirror(x, rows, cols) for x in t.bitboards())
         board, rboard = ou.replay(game, hist)["board"], ou.replay(game, [int(perm[a]) for a in hist])["board"]
         assert np.array_equal(rboard, board[..., ::-1])
         bb = np.array([s.bitboards(), rs.bitboards()], dtype=np.uint64)
@@ -166,11 +99,12 @@ def test_cabi_reflect_flag_and_entry_points():
         assert b"AZ_F_REFLECT" in lib.az_last_error() and name in lib.az_last_error()
 
 
-def test_restatement_reflects_evaluations(reflected_oracle, monkeypatch):
-    """The reflecting evaluator answers for R(s) on about half of the positions, and the restated games differ from the
+def test_restatement_reflects_evaluations():
+    """The restatement's evaluator answers for R(s) on about half of the positions, and the restated games differ from the
     plain ones."""
-    from oracle import cbind, pyspiel_shim
+    from oracle import pyspiel_shim
     g = pyspiel_shim.load_game(BT6)
+    on, off = sr.Rule(BT6, 1, reflect=True, seed=5), sr.Rule(BT6, 1, seed=5)
     hits = total = 0
     for hist in _random_histories(BT6, 60, 4):
         s = g.new_initial_state()
@@ -178,17 +112,11 @@ def test_restatement_reflects_evaluations(reflected_oracle, monkeypatch):
             s.apply_action(a)
         if s.is_terminal():
             continue
-        pri, v = (C.c_double * 432)(), C.c_double()
-        reflected_oracle.oz_synth_eval(C.byref(s.raw()), 1, 5, 4, pri, C.byref(v))
-        want, wv = (C.c_double * 432)(), C.c_double()
-        reflected_oracle._lib.oz_synth_eval(C.byref(s.raw()), 1, 5, 4, want, C.byref(wv))
-        hits += list(pri) != list(want)
+        hits += sr.evaluate(on, s)[0] != sr.evaluate(off, s)[0]
         total += 1
     assert 0.3 * total < hits < 0.7 * total
-    rule = fp._cfg(C4, 60, seed=5)
-    reflected = [fp._selfplay_game(rule, t)[0] for t in range(4)]
-    monkeypatch.setattr(cbind, "lib", lambda: reflected_oracle._lib)
-    assert reflected != [fp._selfplay_game(rule, t)[0] for t in range(4)]
+    reflected = [sr.selfplay_game(sr.Rule(C4, 60, reflect=True, seed=5), t)[0] for t in range(4)]
+    assert reflected != [sr.selfplay_game(sr.Rule(C4, 60, seed=5), t)[0] for t in range(4)]
 
 
 def _trainer_pair(recs, **kw):
@@ -217,7 +145,7 @@ def test_training_bits_leave_the_global_rng_alone():
     """The sample ids of net_step / net_step_arrays, and the RNG state after the step, are the same with the option on and
     off; the minibatch rows are mirrored exactly where replay.reflect_bits says so."""
     from alphazero_openspiel_b200.replay import reflect_bits
-    recs = _oracle_records(n_games=9)
+    recs = sr.oracle_records(n_games=9)
     boards = {}
     for on in (False, True):
         a, b, merged, batch, first, pol, val = _trainer_pair(recs, reflect_minibatches=on)
@@ -243,7 +171,7 @@ def test_list_and_array_paths_build_the_same_reflected_minibatch():
     """Same seeds, same buffer: the list buffer (net_step) and the array buffer (net_step_arrays) see the same mirrored
     boards, take the same losses and end with the same weights; the reflection changes the losses."""
     import torch
-    recs = _oracle_records(n_games=9)
+    recs = sr.oracle_records(n_games=9)
     losses = {}
     for on in (True, False):
         a, b, merged, batch, first, pol, val = _trainer_pair(recs, reflect_minibatches=on)
@@ -267,29 +195,25 @@ def test_list_and_array_paths_build_the_same_reflected_minibatch():
 @pytest.mark.gpu
 @pytest.mark.parametrize("game,n_trees,n_playouts", [(C4, 64, 100), (BT6, 16, 200), (BT8, 8, 120)])
 @pytest.mark.parametrize("keep", [1, 0])
-def test_selfplay_with_reflection_bit_exact(reflected_oracle, game, n_trees, n_playouts, keep):
+def test_selfplay_with_reflection_bit_exact(game, n_trees, n_playouts, keep):
     """Whole games with the hash evaluator: every ply record and every counter equal the restatement's, whose evaluator
     answers for R(s) whenever m(s)."""
-    from alphazero_openspiel_b200 import _lib as L
-    seed = 1234
-    recs, ctr = fp._engine_selfplay(game, n_trees, n_playouts, seed, keep, None, L.F_REFLECT)
-    rule = fp._cfg(game, n_playouts, keep_tree=keep, seed=seed)
-    fp._check_against_oracle(recs, ctr, rule, n_trees)
+    rule = sr.Rule(game, n_playouts, reflect=True, keep_tree=keep, seed=1234)
+    recs, ctr = sr.engine_selfplay(rule, n_trees)
+    sr.check_against_rule(recs, ctr, rule, n_trees)
     if game == C4 and keep:
-        plain, _ = fp._engine_selfplay(game, n_trees, n_playouts, seed, keep, None)
+        plain, _ = sr.engine_selfplay(sr.Rule(game, n_playouts, keep_tree=keep, seed=1234), n_trees)
         assert not (np.array_equal(plain["counts"], recs["counts"]) and np.array_equal(plain["action"], recs["action"]))
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("game,n_trees,n_playouts", [(C4, 64, 100), (BT6, 16, 200)])
-def test_reflection_with_playout_cap_forced_playouts_and_resignation(reflected_oracle, game, n_trees, n_playouts):
-    from alphazero_openspiel_b200 import _lib as L
-    seed, fast, permille, thr, calib = 4321, n_playouts // 4, 250, 0.0, 300
-    recs, ctr = fp._engine_selfplay(game, n_trees, n_playouts, seed, 1, 2.0, L.F_FORCED_PLAYOUTS | L.F_REFLECT,
-                                    resign=(thr, calib), fast=fast, permille=permille)
-    rule = fp._cfg(game, n_playouts, k=2.0, fast=fast, permille=permille, keep_tree=1, seed=seed)
-    resigned, stats = fp._check_against_oracle(recs, ctr, rule, n_trees, thr, calib)
-    assert resigned > 0 and stats["forced"] > 0 and stats["pruned"] > 0
+def test_reflection_with_playout_cap_forced_playouts_and_resignation(game, n_trees, n_playouts):
+    rule = sr.Rule(game, n_playouts, resign=(0.0, 300), playout_cap=(n_playouts // 4, 250), forced=2.0, reflect=True,
+                   keep_tree=1, seed=4321)
+    recs, ctr = sr.engine_selfplay(rule, n_trees)
+    ends, stats = sr.check_against_rule(recs, ctr, rule, n_trees)
+    assert ends[1] > 0 and stats["forced"] > 0 and stats["pruned"] > 0
     plies = recs[recs["kind"] == 0]
     assert (plies["end"] == 3).any() and (plies["end"] == 0).any()
 
@@ -349,7 +273,7 @@ def test_external_evaluator_rows_are_reflected(game, obs_format, vl):
             bb, ply = info["bb"][req], info["ply"][req]
         if req:
             want = _planes(game, bb, ply, obs_format, dev)
-            flips = torch.tensor([_m(seed, int(b[0]), int(b[1]), int(p)) for b, p in zip(bb, ply)], device=dev)
+            flips = torch.tensor([sr.m(seed, int(b[0]), int(b[1]), int(p)) for b, p in zip(bb, ply)], device=dev)
             want = torch.where(flips.view(-1, 1, 1, 1), want.flip(flip_dim), want)
             assert torch.equal(obs[torch.tensor(req, device=dev) * K], want)
             n_rows += len(req)
@@ -363,7 +287,7 @@ def test_external_evaluator_rows_are_reflected(game, obs_format, vl):
         for t in roots:
             if pos2["ply"][t] != pos["ply"][t] or not np.array_equal(pos2["bb"][t], pos["bb"][t]):
                 continue                                             # the search ended in this step
-            m = _m(seed, int(pos["bb"][t][0]), int(pos["bb"][t][1]), int(pos["ply"][t]))
+            m = sr.m(seed, int(pos["bb"][t][0]), int(pos["bb"][t][1]), int(pos["ply"][t]))
             acts = after["child_action"][t, :after["n_children"][t]]
             cols_ = perm[acts] if m else acts
             assert np.array_equal(after["child_p"][t, :len(acts)], rows[t * K, cols_])
@@ -375,11 +299,11 @@ def test_external_evaluator_rows_are_reflected(game, obs_format, vl):
 @pytest.mark.gpu
 def test_eval_cache_with_reflection_gives_the_same_games():
     """Fused evaluator and the shipped Connect Four checkpoint: the same records with the evaluator cache on and off."""
-    on, c_on = pc._runner_games(C4, 512, True, reflect_evaluations=True)
-    off, c_off = pc._runner_games(C4, 512, False, reflect_evaluations=True)
+    on, c_on = sr.runner_games(C4, 512, True, reflect_evaluations=True)
+    off, c_off = sr.runner_games(C4, 512, False, reflect_evaluations=True)
     assert c_on["overflow"] == 0 and c_off["overflow"] == 0
     assert c_on["cache_hits"] > 0 and c_off["cache_hits"] == 0
-    pc._same_records(on, off)
+    sr.same_records(on, off)
 
 
 @pytest.mark.gpu
@@ -416,7 +340,7 @@ def test_reflected_gather_kernel(game):
                 flip = torch.from_numpy(flags).to(dev).view(-1, 1, 1, 1)
                 assert torch.equal(got, torch.where(flip, want.flip(2 if fmt == L.OBS_BF16_NHWC else 3), want))
     if game == C4:
-        batch = ExampleBatch.from_records(_oracle_records(n_games=6, playouts=15, seed=4), C4)
+        batch = ExampleBatch.from_records(sr.oracle_records(n_games=6, playouts=15, seed=4), C4)
         rb = DeviceReplay(C4, "cuda:0")
         rb.append(batch)
         rng = np.random.RandomState(2)
@@ -436,7 +360,7 @@ def test_reflected_minibatches_take_the_same_steps_on_every_path():
     from alphazero_openspiel_b200.device_replay import DeviceReplay
     from alphazero_openspiel_b200.replay import ExampleBatch
     from alphazero_openspiel_b200.train import Trainer
-    recs = _oracle_records(n_games=12, playouts=15, seed=4)
+    recs = sr.oracle_records(n_games=12, playouts=15, seed=4)
     losses = {}
     for mode in ("array", "device", "graph", "array_plain"):
         torch.manual_seed(3)

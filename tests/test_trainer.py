@@ -9,6 +9,8 @@ import numpy as np
 import pytest
 import torch
 
+from tests import selfplay_rule as sr
+
 
 def _fake_buffer(rng, n=300, n_keys=60, A=7):
     flat = []
@@ -125,44 +127,12 @@ def test_array_buffer_generations_match_the_list_buffer():
         assert all(torch.isfinite(v.float()).all() for v in sd.values())
 
 
-def _oracle_records(n_games=6, game="connect_four", playouts=20, seed=9, start_mod=0):
-    """Device-format training records synthesised from the C oracle's self-play (as in test_cabi_and_host)."""
-    from alphazero_openspiel_b200.engine import record_dtype
-    from tests import oracle_util as ou
-    cfg = ou.selfplay_cfg(game, playouts, use_dirichlet=2, sample_moves=1, seed=seed, start_mod=start_mod)
-    dt = record_dtype(7, (72 + 6 * 7 + 7) // 8 * 8)
-    rows = []
-    for t in range(n_games):
-        plies, ret, _ = ou.selfplay_game(cfg, t % 3)       # trees 0..2 twice: duplicate histories across games
-        hist = []
-        for r in plies:
-            rec = np.zeros((), dtype=dt)
-            rec["tree"], rec["game_seq"], rec["ply"], rec["action"] = t, 0, r["ply"], r["action"]
-            rec["n_legal"], rec["kind"], rec["root_n"] = r["n_legal"], 0, r["root_n"]
-            rec["bb"] = r["bb"]
-            rec["root_q"], rec["v_a0c"], rec["v_offpolicy"] = r["root_q"], r["v_a0c"], r["v_offpolicy"]
-            rec["counts"][:r["n_legal"]] = r["counts"]
-            rec["actions"][:] = -1
-            if start_mod == 0:
-                rec["actions"][:r["n_legal"]] = ou.replay(game, hist)["legal"]
-            else:   # random-start games have no history from the initial position: Connect Four legal = non-full columns
-                occ = int(r["bb"][0]) | int(r["bb"][1])
-                rec["actions"][:r["n_legal"]] = [c for c in range(7) if not (occ >> (35 + c)) & 1]
-            rows.append(rec)
-            hist.append(r["action"])
-        end = np.zeros((), dtype=dt)
-        end["tree"], end["kind"], end["ply"], end["root_q"] = t, 1, plies[-1]["ply"] + 1, ret[0]
-        rows.append(end)
-    recs = np.array(rows, dtype=dt)
-    return recs[np.random.RandomState(1).permutation(len(recs))]
-
-
 def test_example_batch_is_a_lossless_form_of_the_reference_examples():
     """replay.ExampleBatch (SURVEY 8(f) rank 3): from_records + to_games == records_to_games for every value target;
     concat / last_games follow the buffer list semantics."""
     from alphazero_openspiel_b200.examplegenerator import records_to_games
     from alphazero_openspiel_b200.replay import ExampleBatch
-    recs = _oracle_records()
+    recs = sr.oracle_records()
     for backup in ["on-policy", "soft-Z", "A0C", "off-policy"]:
         want = records_to_games(recs, "connect_four", backup)
         b = ExampleBatch.from_records(recs, "connect_four", backup)
@@ -188,7 +158,7 @@ def test_array_remove_duplicates_and_net_step_match_the_list_path():
     seeds and initial weights, the same losses and weights after a few optimisation steps."""
     from alphazero_openspiel_b200.replay import ExampleBatch
     from alphazero_openspiel_b200.train import Trainer
-    recs = _oracle_records(n_games=9)
+    recs = sr.oracle_records(n_games=9)
     batch = ExampleBatch.from_records(recs, "connect_four")
     games = batch.to_games()
     flat = [ex for g in games for ex in g]
@@ -222,7 +192,7 @@ def test_random_start_games_get_signs_from_the_ply_and_keys_from_the_start_posit
     position so that different positions never share a key.  Both example forms agree."""
     from alphazero_openspiel_b200.examplegenerator import records_to_games
     from alphazero_openspiel_b200.replay import ExampleBatch
-    recs = _oracle_records(n_games=12, start_mod=9, seed=3)
+    recs = sr.oracle_records(n_games=12, start_mod=9, seed=3)
     games = records_to_games(recs, "connect_four", "on-policy")
     batch = ExampleBatch.from_records(recs, "connect_four", "on-policy")
     assert len(games) == 12 and batch.n_games == 12
@@ -258,7 +228,7 @@ def test_device_replay_matches_the_array_buffer():
     from alphazero_openspiel_b200.device_replay import DeviceReplay
     from alphazero_openspiel_b200.replay import ExampleBatch
     from alphazero_openspiel_b200.train import Trainer
-    recs = _oracle_records(n_games=12, playouts=15, seed=4)
+    recs = sr.oracle_records(n_games=12, playouts=15, seed=4)
     host = ExampleBatch.concat([ExampleBatch.from_records(recs, "connect_four"), ExampleBatch.from_records(recs, "connect_four")])
     dev = DeviceReplay("connect_four", "cuda:0")
     dev.append(ExampleBatch.from_records(recs, "connect_four"))
@@ -324,7 +294,7 @@ def test_device_replay_key_hash_groups_like_the_reference_keys():
     from alphazero_openspiel_b200.device_replay import key_hash
     from alphazero_openspiel_b200.replay import ExampleBatch
     for start_mod in (0, 9):
-        recs = _oracle_records(n_games=12, start_mod=start_mod, seed=3)
+        recs = sr.oracle_records(n_games=12, start_mod=start_mod, seed=3)
         b = ExampleBatch.concat([ExampleBatch.from_records(recs, "connect_four")] * 2)
         h = key_hash(b)
         keys = [b.key(i) for i in range(len(b))]
